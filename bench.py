@@ -10,13 +10,15 @@ overlapped with the next chunk's kernel.
 
     python bench.py --gpus 1 --steps 20 --warmup 3            # our arm
     python bench.py --impl reference --steps 3 --warmup 1      # CPU oracle port on host cores
+    python bench.py --steps 20 --dump-outputs DIR              # also DIR/log_prob.npy: the last timed step's log-probs
 
 Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for the meaning of every key.
 
 The headline keys describe config 2.  The same line carries `configs`: BASELINE configs 1, 3, 4, 5 (and config 2 under
 strong scaling when N > 1), each measured in this process with its own value / unit / ms / roofline / cpu_baseline /
-e2e, so that every named configuration -- and the second named metric, MNF-LeNet MC predictive samples/s -- is on the
-driver's clock.  `--workload cfg2` prints the headline alone, `--workload cfg4` the MNF-LeNet line alone.
+e2e, so that every named configuration -- and the second named metric, MNF-LeNet MC predictive samples/s -- is
+measured by the same run.  `--steps` is the number of timed steps of every timed loop, headline and configurations.
+`--workload cfg2` prints the headline alone, `--workload cfg4` the MNF-LeNet line alone.
 """
 
 from __future__ import annotations
@@ -43,6 +45,7 @@ MLP_FMA_PER_POINT = 3 * 2 * (16 + 256 + 256 + 16 * 23)  # 5376 fused multiply-ad
 TRAFFIC_FILE = os.path.join(ROOT, "profiles", "ncu_traffic.json")  # written by tools/ncu_traffic.py from an `ncu --set full` capture
 METRIC = "flow log-prob points/s"
 WORKLOAD = "cfg2: [ActNormFlow, Glow, NSF_CL(K=8,B=3,n_h=16)] x3, 2-D points, batch 2^24 per GPU"
+DUMP_MAX_VALUES = 1 << 22  # --dump-outputs: 16 MB of float32 at most, whatever the batch and the number of GPUs
 
 
 def specs():
@@ -103,6 +106,19 @@ def timed_ms(fn, steps, warmup, dev, world=1):
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
         ms = float(tt)
     return ms
+
+
+def dump_sample(values, seed=0):
+    """`values` (1-D, on the device) on the host: all of them up to DUMP_MAX_VALUES, else one value drawn with a fixed
+    seed from each of DUMP_MAX_VALUES equal consecutive blocks.  The indices depend only on the length, so runs with
+    the same arguments sample the same points."""
+    n = values.numel()
+    if n <= DUMP_MAX_VALUES:
+        return values.cpu()
+    stride = n // DUMP_MAX_VALUES
+    g = torch.Generator().manual_seed(seed)
+    idx = torch.arange(DUMP_MAX_VALUES) * stride + torch.randint(stride, (DUMP_MAX_VALUES,), generator=g)
+    return values[idx.to(values.device)].cpu()
 
 
 def peaks():
@@ -354,6 +370,12 @@ def run_ours(args):
         dist.all_gather(sums, mine)
         seen = torch.stack([gathered.view(-1, world, cn)[:, r].double().sum() for r in range(world)])
         gather_ok = bool(torch.allclose(seen, torch.cat(sums), rtol=1e-9, atol=1e-6))
+    if args.dump_outputs and rank == 0:
+        # what the last timed step handed its caller: every rank's log-probs, in rank order (before later legs reuse the buffer)
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "log_prob.npy"), dump_sample(gathered.transpose(0, 1).reshape(-1)).numpy())
     ms_per_step = total_ms / args.steps
     value = world * n / (ms_per_step * 1e-3)
 
@@ -553,11 +575,11 @@ def run_ours(args):
                 prog.run(x, True, out=ys, log_det=lds)
             a_, b_ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a_.record()
-            for _ in range(20):
+            for _ in range(args.steps):
                 prog.run(x, True, out=ys, log_det=lds)
             b_.record()
             torch.cuda.synchronize(dev)
-            sub_ms = a_.elapsed_time(b_) / 20
+            sub_ms = a_.elapsed_time(b_) / args.steps
             out["hbm_bound_substack"] = {
                 "workload": "[ActNormFlow, Glow] x3 (the conditioner-free flows of the headline stack), inverse with z and log_det stored",
                 "bytes_per_point": 20, "ms": sub_ms, "achieved": 20 * n / (sub_ms * 1e-3) / 1e9, "peak": hbm_peak,
@@ -645,7 +667,7 @@ def cfg1(args, dev):
     out_pin = torch.empty(4096).pin_memory()
     x = x_host.to(dev)
     lp = torch.empty(4096, device=dev)
-    K = 200
+    K = args.steps
     sites = kernels_of(lambda: model.log_prob(x, out=lp))
     ms = timed_ms(lambda: model.log_prob(x, out=lp), K, 20, dev)
     ms_fwd = timed_ms(lambda: model.forward(x), K, 20, dev)
@@ -704,7 +726,7 @@ def cfg3(args, dev):
     n = 1 << 20
     x_pin = torch.randn(n, 64, generator=torch.Generator().manual_seed(0)).pin_memory()
     x = x_pin.to(dev)
-    steps = max(3, min(args.steps, 10))
+    steps = args.steps
     res = {}
     rows = []
     for prec in ("auto", "fp32"):
@@ -797,7 +819,7 @@ def cfg4(args, dev, world, rank, total_samples=500, per_gpu_samples=None):
             probs_host.copy_(probs, non_blocking=True)
         return probs
 
-    steps = max(2, min(args.steps, 5))
+    steps = args.steps
     sites = kernels_of(step)
     l0 = _lib.lib().mnf_launch_count()
     ms = timed_ms(step, steps, 3, dev, world)
@@ -882,11 +904,11 @@ def cfg5(args, dev, world, rank):
                 stats_pin.copy_(st / S_tot, non_blocking=True)
         return kl
 
-    steps = max(2, min(args.steps, 3))
+    steps = args.steps
     sites = kernels_of(step)
     ms = timed_ms(step, steps, 2, dev, world)
     fwd_ms = timed_ms(lambda: layer.forward_mc(x64, S, noise=Noise(None, dev, s_lo * 64, seed=5)), steps, 1, dev, world)
-    kl_ms = timed_ms(lambda: layer.kl_div(), 20, 3, dev, world)
+    kl_ms = timed_ms(lambda: layer.kl_div(), steps, 3, dev, world)
     e_ms = timed_ms(lambda: step(True), steps, 1, dev, world)
     if rank != 0:
         return None
@@ -1023,7 +1045,14 @@ def main():
                          "cfg2: the headline alone; cfg4: the MNF-LeNet MC prediction line alone (weak scaling)")
     ap.add_argument("--mc-samples", type=int, default=64, help="--workload cfg4: MC samples per image per GPU per step")
     ap.add_argument("--cfg5-samples", type=int, default=8192, help="cfg5: MC samples (x 64 input rows) in total")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the headline's log-probs of the last step to DIR/log_prob.npy "
+                         "(float32, every rank's points in rank order; above 2^22 values a fixed, seeded sample of them)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "cfg4"):
+        ap.error("--dump-outputs writes the headline (cfg2) outputs: use it with --impl ours and --workload all or cfg2")
     torch.set_grad_enabled(False)  # the workload is density evaluation / prediction, not training
     if args.impl == "reference":
         run_reference(args)
