@@ -15,7 +15,9 @@
 //   flow_pl_kernel<K>      one thread per point, the whole stack in one launch: a conditioner is a branch-free binary
 //                          search over <= 511 sorted breakpoints in shared memory and one FMA per output
 //                          (out = V_i + A_i (c - origin_i)); the spline (flow_math.cuh) then runs on the raw outputs, and only
-//                          the two knot derivatives of the bin the point falls into are ever formed.
+//                          the two knot derivatives of the bin the point falls into are ever formed.  Tables with a fast form
+//                          (written by the builder next to the plain one) are looked up through a bucket index instead, and
+//                          their spline outputs come pre-shifted for the softmax.
 //
 // Per point and conditioner: ~60 instructions instead of 5 376 multiply-adds (or three MMA round trips).  No tensor core
 // and no FMA chain is left to feed: what remains is the spline arithmetic and 12 B/pt of HBM traffic.
@@ -33,9 +35,17 @@ using tc::smem_u32; using tc::mbar_init; using tc::mbar_arrive; using tc::mbar_w
 constexpr int PMAX = 511;       // breakpoints per table
 constexpr int BP_FLOATS = 512;  // sorted breakpoints, padded with +inf (search array)
 constexpr int MAX_GROUPS = 2 * MNF_MAX_OPS;
-constexpr int HDR_INTS = 4;     // per table: breakpoints, overflow flag, 2 spare
+constexpr int HDR_INTS = 4;     // per table: breakpoints, overflow flag, fast form's offset and size (floats; 0 = none)
 constexpr int HDR_FLOATS = MAX_GROUPS * HDR_INTS;
 constexpr int MAX_H = 64;       // hidden width the in-kernel fp32 fallback holds
+// Fast form of a table (see the builder): spline rows shifted so that every exponent is <= FAST_T (log2 units), a bucket
+// index in place of the binary search.  Only for spline bounds up to FAST_B_MAX: the two second-softmax sums of a point,
+// each in [e^-B, K e^B], are then inverted by one reciprocal of their product without leaving the normal fp32 range.
+constexpr double FAST_T = 32.0;
+constexpr float FAST_B_MAX = 32.f;
+constexpr int NB_MIN = 64, NB_MAX = 2048;  // buckets (powers of two)
+constexpr int SMEM_TABLE_FLOATS = 216 * 1024 / 4;  // shared memory the point kernel gives the tables of a program
+constexpr double LOG2E_D = 1.4426950408889634;
 
 __host__ __device__ constexpr int round4i(int n) { return (n + 3) / 4 * 4; }
 // NSF_CL row: K float4 (A_2j, A_2j+1, V_2j, V_2j+1) for the 2K width / height outputs | K - 1 float2 (A, V) of the knot
@@ -55,10 +65,96 @@ struct GroupList {
     signed char group_of[MNF_MAX_OPS][2];
 };
 
+// Bucket of c in the fast form's grid (lo, inv, NB - 1): clamp((c - lo) inv) rounded down, NaN to bucket 0.  Monotone
+// non-decreasing in c, and the builder files every breakpoint with this same function, so the breakpoints below c are
+// those of the buckets before c's plus those of c's own bucket that are < c -- whatever the rounding of the grid.  The
+// float-to-int conversion is an add in round-to-zero mode (FMA pipe) instead of F2I (XU pipe).
+__device__ __forceinline__ int bucket_of(float c, float lo, float inv, float nbm1) {
+    const float t = fminf(fmaxf((c - lo) * inv, 0.f), nbm1);
+    return __float_as_int(__fadd_rz(t, 8388608.f)) & 0x7fffff;
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // builder
 // ---------------------------------------------------------------------------------------------------------
 constexpr int BW = 8;  // warps per builder CTA
+
+// Of the K outputs o0 .. o0 + K - 1 (affine maps A c + B on the piece (lo, hi)), the one that is maximal at the piece's
+// midpoint, or on an unbounded piece the one that is maximal far out (extreme slope, then larger value): a supporting
+// line of the outputs' upper envelope on the piece.
+__device__ int envelope_line(const double *A, const double *B, int o0, int K, double lo, double hi) {
+    int l = o0;
+    if (lo == -INFINITY || hi == INFINITY) {
+        const double sg = lo == -INFINITY ? -1.0 : 1.0;
+        for (int k = o0 + 1; k < o0 + K; ++k)
+            if (sg * A[k] > sg * A[l] || (A[k] == A[l] && B[k] > B[l])) l = k;
+    } else {
+        const double m = 0.5 * lo + 0.5 * hi;
+        for (int k = o0 + 1; k < o0 + K; ++k)
+            if (fma(A[k], m, B[k]) > fma(A[l], m, B[l])) l = k;
+    }
+    return l;
+}
+
+// largest distance at e, over both spline axes, between the envelope of the outputs and the line envelope_line picks on (lo, hi)
+__device__ double envelope_gap(const double *A, const double *B, int K, double lo, double hi, double e) {
+    double g = 0.0;
+    for (int o0 = 0; o0 < 2 * K; o0 += K) {
+        const int l = envelope_line(A, B, o0, K, lo, hi);
+        const double vl = fma(A[l], e, B[l]);
+        for (int k = o0; k < o0 + K; ++k) g = fmax(g, fma(A[k], e, B[k]) - vl);
+    }
+    return g;
+}
+
+// One thread: split points (fp32 values, strictly inside (lo, hi)) that cut the piece into pieces on which the gap of
+// envelope_gap stays <= FAST_T / log2(e) at both ends, hence everywhere (the gap is convex).  An unbounded piece first gets
+// one cut beyond which its extreme line is within the bound, the bounded rest is halved as often as needed.  false: no
+// such cutting within the split budget (the table then gets no fast form).
+__device__ bool split_piece(const double *A, const double *B, int K, double lo, double hi, double *out, int *cnt) {
+    const double TN = FAST_T / LOG2E_D;
+    auto emit = [&](double s) {
+        const int p = atomicAdd(cnt, 1);
+        if (p < PMAX) out[p] = s;
+        return p < PMAX;
+    };
+    double seg[2][2] = {{lo, hi}, {0.0, 0.0}};
+    int nseg = 1;
+    if (lo == -INFINITY && hi == INFINITY) {
+        if (!emit(0.0)) return false;
+        seg[0][1] = 0.0, seg[1][0] = 0.0, seg[1][1] = INFINITY, nseg = 2;
+    }
+    for (int q = 0; q < nseg; ++q) {
+        double a = seg[q][0], b = seg[q][1];
+        const bool left = a == -INFINITY, right = b == INFINITY;
+        if (left || right) {
+            const double e = left ? b : a;
+            if (envelope_gap(A, B, K, a, b, e) <= TN) continue;
+            double w = fmax(1.0, fabs(e)), s;
+            for (;;) {
+                s = (double)(float)(left ? e - w : e + w);
+                if (fabs(s) > 1.0e38) return false;
+                if (envelope_gap(A, B, K, left ? -INFINITY : s, left ? s : INFINITY, s) <= TN) break;
+                w *= 2.0;
+            }
+            if (!emit(s)) return false;
+            a = left ? s : e, b = left ? e : s;
+        }
+        double st[64][2];
+        int sp = 0;
+        st[sp][0] = a, st[sp][1] = b, ++sp;
+        while (sp) {
+            --sp;
+            const double x0 = st[sp][0], x1 = st[sp][1];
+            if (envelope_gap(A, B, K, x0, x1, x0) <= TN && envelope_gap(A, B, K, x0, x1, x1) <= TN) continue;
+            const double s = (double)(float)(0.5 * x0 + 0.5 * x1);
+            if (!(s > x0 && s < x1) || sp + 2 > 64 || !emit(s)) return false;
+            st[sp][0] = s, st[sp][1] = x1, ++sp;
+            st[sp][0] = x0, st[sp][1] = s, ++sp;
+        }
+    }
+    return true;
+}
 
 // a point strictly inside piece i of the n sorted breakpoints (fixes the sign of every pre-activation on the piece)
 __device__ __forceinline__ double piece_point(const double *bp, int n, int i, double &lo, double &hi) {
@@ -107,8 +203,20 @@ __global__ void __launch_bounds__(32 * BW) flow_pl_build_kernel(const __grid_con
                                                                 const float *__restrict__ params, float *__restrict__ image) {
     __shared__ double s_bp[512], s_tmp[512];
     __shared__ double s_va[BW][2][MNF_MAX_HIDDEN], s_vb[BW][2][MNF_MAX_HIDDEN];
-    __shared__ int s_n, s_ncand;
+    __shared__ int s_bidx[PMAX];
+    __shared__ int s_n, s_ncand, s_fail;
     const int g = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, nt = blockDim.x;
+    auto sort_bp = [&](int tot) {  // s_bp[0 .. tot) in ascending order (rank sort, ties by index)
+        for (int e = tid; e < tot; e += nt) {
+            const double v = s_bp[e];
+            int r = 0;
+            for (int u = 0; u < tot; ++u) r += (s_bp[u] < v || (s_bp[u] == v && u < e)) ? 1 : 0;
+            s_tmp[r] = v;
+        }
+        __syncthreads();
+        for (int e = tid; e < tot; e += nt) s_bp[e] = s_tmp[e];
+        __syncthreads();
+    };
     const mnf_flow_op &op = prog.ops[gl.op[g]];
     const bool nsf = op.type == MNF_OP_NSF_CL;
     const int K = op.K, L = op.n_lin, n_out = op.sizes[L];
@@ -153,14 +261,7 @@ __global__ void __launch_bounds__(32 * BW) flow_pl_build_kernel(const __grid_con
         }
         for (int e = tid; e < nc; e += nt) s_bp[n + e] = s_tmp[e];
         __syncthreads();
-        for (int e = tid; e < tot; e += nt) {  // rank sort (ties by index)
-            const double v = s_bp[e];
-            int r = 0;
-            for (int u = 0; u < tot; ++u) r += (s_bp[u] < v || (s_bp[u] == v && u < e)) ? 1 : 0;
-            s_tmp[r] = v;
-        }
-        __syncthreads();
-        for (int e = tid; e < tot; e += nt) s_bp[e] = s_tmp[e];
+        sort_bp(tot);
         if (tid == 0) s_n = tot, s_ncand = 0;
         __syncthreads();
     }
@@ -172,29 +273,107 @@ __global__ void __launch_bounds__(32 * BW) flow_pl_build_kernel(const __grid_con
     for (int e = tid; e < BP_FLOATS; e += nt) region[e] = e < n ? (float)s_bp[e] : INFINITY;
     if (over) return;
     const int stride = 4 * (nsf ? nsf_stride4(K) : AFF_STRIDE4);
-    float *rows = region + BP_FLOATS;
-    for (int i = warp; i <= n; i += BW) {
-        double lo, hi;
-        const double m = piece_point(s_bp, n, i, lo, hi);
-        // origin: the (fp32) breakpoint the piece starts at -- the kernel forms c - origin exactly there
-        const float org = n == 0 ? 0.f : (float)(i == 0 ? s_bp[0] : s_bp[i - 1]);
-        float *row = rows + (size_t)i * stride;
-        for (int e = lane; e < stride; e += 32) row[e] = 0.f;
-        __syncwarp();
-        for (int q = 0; q < n_nets; ++q) {
-            const int cur = net_pre_maps(params + net_off[q], op.sizes, L - 1, m, s_va[warp], s_vb[warp], lane);
-            for (int o = lane; o < n_out; o += 32) {
-                const double A = s_va[warp][cur][o], V = fma(A, (double)org, s_vb[warp][cur][o]);
-                int ia, iv;
-                if (!nsf) ia = net_slot[q], iv = 2 + net_slot[q];
-                else if (o < 2 * K) ia = 4 * (o >> 1) + (o & 1), iv = ia + 2;
-                else ia = nsf_doff(K) + 2 * (o - 2 * K), iv = ia + 1;
-                row[ia] = (float)A, row[iv] = (float)V;
+    // Rows of the nn + 1 pieces of s_bp.  fast: the spline outputs of each axis minus the axis's envelope_line and, like
+    // the knot-derivative outputs, in log2 units (softmax is invariant to the shift; the kernel feeds them to ex2 as they are).
+    auto write_rows = [&](int nn, float *rows, bool fast) {
+        for (int i = warp; i <= nn; i += BW) {
+            double lo, hi;
+            const double m = piece_point(s_bp, nn, i, lo, hi);
+            // origin: the (fp32) breakpoint the piece starts at -- the kernel forms c - origin exactly there
+            const float org = nn == 0 ? 0.f : (float)(i == 0 ? s_bp[0] : s_bp[i - 1]);
+            float *row = rows + (size_t)i * stride;
+            for (int e = lane; e < stride; e += 32) row[e] = 0.f;
+            __syncwarp();
+            for (int q = 0; q < n_nets; ++q) {
+                const int cur = net_pre_maps(params + net_off[q], op.sizes, L - 1, m, s_va[warp], s_vb[warp], lane);
+                const double *va = s_va[warp][cur], *vb = s_vb[warp][cur];
+                for (int o = lane; o < n_out; o += 32) {
+                    double A = va[o], B = vb[o], sc = 1.0;
+                    if (fast && nsf) {
+                        sc = LOG2E_D;
+                        if (o < 2 * K) {
+                            const int l = envelope_line(va, vb, o < K ? 0 : K, K, lo, hi);
+                            A -= va[l], B -= vb[l];
+                        }
+                    }
+                    const double V = fma(A, (double)org, B);
+                    int ia, iv;
+                    if (!nsf) ia = net_slot[q], iv = 2 + net_slot[q];
+                    else if (o < 2 * K) ia = 4 * (o >> 1) + (o & 1), iv = ia + 2;
+                    else ia = nsf_doff(K) + 2 * (o - 2 * K), iv = ia + 1;
+                    row[ia] = (float)(A * sc), row[iv] = (float)(V * sc);
+                }
+                __syncwarp();
             }
+            if (lane == 0) row[nsf ? nsf_org(K) : AFF_ORG] = org;
+        }
+    };
+    write_rows(n, region + BP_FLOATS, false);
+
+    // Fast form, in rows n + 1 .. PMAX of the region (never read otherwise): [lo, inv, NB - 1, offset of the rows]
+    // [NB bucket records (number of breakpoints in the buckets before, the <= 3 breakpoints of the bucket padded with +inf)]
+    // [rows of the fast pieces].  The fast pieces are the pieces cut further (split_piece) where a spline axis's outputs
+    // would reach more than FAST_T above the line they are stored relative to.
+    __syncthreads();  // the rows read s_bp, which becomes the list of fast breakpoints
+    if (tid == 0) s_ncand = 0, s_fail = nsf && !(op.bound <= FAST_B_MAX);
+    __syncthreads();
+    if (nsf && !s_fail) {
+        for (int i = warp; i <= n; i += BW) {
+            double lo, hi;
+            const double m = piece_point(s_bp, n, i, lo, hi);
+            const int cur = net_pre_maps(params + net_off[0], op.sizes, L - 1, m, s_va[warp], s_vb[warp], lane);
+            if (lane == 0 && !split_piece(s_va[warp][cur], s_vb[warp][cur], K, lo, hi, s_tmp, &s_ncand)) s_fail = 1;
             __syncwarp();
         }
-        if (lane == 0) row[nsf ? nsf_org(K) : AFF_ORG] = org;
     }
+    __syncthreads();
+    const int nf = n + s_ncand;
+    if (s_fail || nf > PMAX) return;
+    for (int e = tid; e < nf - n; e += nt) s_bp[n + e] = s_tmp[e];
+    __syncthreads();
+    sort_bp(nf);
+    const int fast_off = BP_FLOATS + (n + 1) * stride, rows_floats = (nf + 1) * stride;
+    // Grid: the fewest buckets NB with <= 3 breakpoints in each, spanning the fast breakpoints from the a-th lowest to the
+    // b-th highest (a, b <= 2: kinks lie dense around the origin with a few far out, which the two clamped end buckets
+    // take).  Bounded so that the fast forms of all tables of the program fit in shared memory together.
+    const int budget = min((PMAX - n) * stride, SMEM_TABLE_FLOATS / gl.n);
+    int nb = NB_MIN;
+    float lo32 = 0.f, inv = 0.f;
+    for (bool found = false; !found; nb *= 2) {
+        if (nb > NB_MAX || 4 + 4 * nb + rows_floats > budget) return;
+        for (int ab = 0; ab < 9 && !found; ++ab) {
+            const int a = ab / 3, b = ab % 3;
+            if (nf && a + b >= nf) continue;
+            lo32 = nf ? (float)s_bp[a] : 0.f;
+            const float hi32 = nf ? (float)s_bp[nf - 1 - b] : 0.f;
+            inv = hi32 > lo32 ? (float)((double)nb / ((double)hi32 - (double)lo32)) : 0.f;
+            for (int e = tid; e < nf; e += nt) s_bidx[e] = bucket_of((float)s_bp[e], lo32, inv, (float)(nb - 1));
+            __syncthreads();
+            int bad = 0;
+            for (int e = tid; e + 3 < nf; e += nt) bad |= s_bidx[e] == s_bidx[e + 3];
+            found = !__syncthreads_or(bad);
+        }
+        if (found) break;
+    }
+    float *fast = region + fast_off;
+    for (int j = tid; j < nb; j += nt) {
+        int a = 0, b = nf;  // first breakpoint of bucket >= j
+        while (a < b) {
+            const int mid = (a + b) >> 1;
+            if (s_bidx[mid] < j) a = mid + 1; else b = mid;
+        }
+        float4 r;
+        r.x = __int_as_float(a);
+        r.y = a < nf && s_bidx[a] == j ? (float)s_bp[a] : INFINITY;
+        r.z = a + 1 < nf && s_bidx[a + 1] == j ? (float)s_bp[a + 1] : INFINITY;
+        r.w = a + 2 < nf && s_bidx[a + 2] == j ? (float)s_bp[a + 2] : INFINITY;
+        reinterpret_cast<float4 *>(fast)[1 + j] = r;
+    }
+    if (tid == 0) {
+        fast[0] = lo32, fast[1] = inv, fast[2] = (float)(nb - 1), fast[3] = __int_as_float(4 + 4 * nb);
+        hdr[2] = fast_off, hdr[3] = 4 + 4 * nb + rows_floats;
+    }
+    write_rows(nf, fast + 4 + 4 * nb, true);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -277,6 +456,21 @@ __device__ __forceinline__ int find_piece(const float *tb, float c) {
     }
 }
 
+enum { KIND_PLAIN = 0, KIND_FAST = 1, KIND_OVER = 2 };  // table evaluated by binary search / by its fast form / layer by layer
+
+// row of the piece of c.  fast: tb is the table's fast form -- one grid load (the same address for the whole warp), one
+// bucket record, three compares; otherwise the binary search over the padded breakpoints.
+template <bool SM>
+__device__ __forceinline__ const float4 *piece_row(const float *tb, bool fast, float c, int stride4) {
+    if (fast) {
+        const float4 gr = *reinterpret_cast<const float4 *>(tb);
+        const float4 bk = reinterpret_cast<const float4 *>(tb)[1 + bucket_of(c, gr.x, gr.y, gr.z)];
+        const int piece = __float_as_int(bk.x) + (c > bk.y) + (c > bk.z) + (c > bk.w);
+        return reinterpret_cast<const float4 *>(tb + __float_as_int(gr.w)) + piece * stride4;
+    }
+    return reinterpret_cast<const float4 *>(tb + BP_FLOATS) + find_piece<SM>(tb, c) * stride4;
+}
+
 __device__ __forceinline__ float ex2_approx(float x) {
     float r;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
@@ -287,50 +481,84 @@ __device__ __forceinline__ float sqrt_approx(float x) {
     asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
     return r;
 }
+__device__ __forceinline__ float lg2_approx(float x) {
+    float r;
+    asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+    return r;
+}
 
-// Knots of one spline axis in units of B: t[0] = -1, t[K] = 1.  The formulas of flow_math.cuh::spline_knots (both
+constexpr float LOG2E = 1.4426950408889634f, LN2 = 0.6931471805599453f;
+
+// Knots of the two spline axes in units of B: t[0] = -1, t[K] = 1.  The formulas of flow_math.cuh::spline_knots (both
 // softmaxes of spline_flow.py:253-255 and :95, floor :96-97, cumsum :99, pinned ends :100-101) with the cumulative sum
 // taken over the second softmax's terms while they are summed: x_{k+1} / B = -1 + 2 (k + 1) min_bin + (2 span / sum f) * (f_0 + .. + f_k),
 // one FFMA per knot.
-template <int K>
-__device__ __forceinline__ void unit_knots(const float *raw, float twoB, float *t) {
-    constexpr float LOG2E = 1.4426950408889634f;
+// FAST: raw holds the outputs of a fast table (log2 units, largest in [0, FAST_T]): no max to subtract, every first-softmax
+// sum lies in [1, K 2^FAST_T] and, with the second softmax's arguments centred on 0, every second-softmax sum in
+// [e^-B, K e^B], so each pair of sums is inverted by one reciprocal of its product.  Otherwise (natural units) the
+// largest output of each axis is subtracted first.
+template <int K, bool FAST>
+__device__ __forceinline__ void unit_knots(const float *raw, float twoB, float *tw, float *th) {
     constexpr float span = 1.f - kMinBin * (float)K;
-    float m = raw[0];
+    float ew[K], eh[K], sw = 0.f, sh = 0.f, scw, sch, offw, offh;
+    if constexpr (FAST) {
 #pragma unroll
-    for (int k = 1; k < K; ++k) m = fmaxf(m, raw[k]);
-    const float mneg = -m * LOG2E;
-    float e[K], sum = 0.f;
+        for (int k = 0; k < K; ++k) {
+            ew[k] = ex2_approx(raw[k]), eh[k] = ex2_approx(raw[K + k]);
+            sw += ew[k], sh += eh[k];
+        }
+        const float r = frcp<true>(sw * sh), s = twoB * LOG2E;  // first softmax scaled by 2B, in log2 units
+        scw = s * (r * sh), sch = s * (r * sw);
+        offw = offh = -0.5f * s;
+    } else {
+        float mw = raw[0], mh = raw[K];
+#pragma unroll
+        for (int k = 1; k < K; ++k) mw = fmaxf(mw, raw[k]), mh = fmaxf(mh, raw[K + k]);
+        const float mwn = -mw * LOG2E, mhn = -mh * LOG2E;
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            ew[k] = ex2_approx(fmaf(raw[k], LOG2E, mwn)), eh[k] = ex2_approx(fmaf(raw[K + k], LOG2E, mhn));
+            sw += ew[k], sh += eh[k];
+        }
+        scw = twoB * frcp<true>(sw) * LOG2E, sch = twoB * frcp<true>(sh) * LOG2E;
+        offw = twoB > 80.f ? -scw : 0.f, offh = twoB > 80.f ? -sch : 0.f;  // arguments of the second softmax lie in [0, 2B]
+    }
+    float pw = 0.f, ph = 0.f;
 #pragma unroll
     for (int k = 0; k < K; ++k) {
-        e[k] = ex2_approx(fmaf(raw[k], LOG2E, mneg));
-        sum += e[k];
+        pw += ex2_approx(fmaf(ew[k], scw, offw)), ph += ex2_approx(fmaf(eh[k], sch, offh));
+        ew[k] = pw, eh[k] = ph;
     }
-    const float sc = twoB * frcp<true>(sum) * LOG2E;  // first softmax scaled by 2B, in log2 units
-    const float off = twoB > 80.f ? -sc : 0.f;        // arguments of the second softmax lie in [0, 2B]
-    float pre = 0.f;
-#pragma unroll
-    for (int k = 0; k < K; ++k) {
-        pre += ex2_approx(fmaf(e[k], sc, off));
-        e[k] = pre;
+    float c1w, c1h;
+    if constexpr (FAST) {
+        const float r = frcp<true>(pw * ph);
+        c1w = 2.f * span * (r * ph), c1h = 2.f * span * (r * pw);
+    } else {
+        c1w = 2.f * span * frcp<true>(pw), c1h = 2.f * span * frcp<true>(ph);
     }
-    const float c1 = 2.f * span * frcp<true>(pre);
-    t[0] = -1.f;
+    tw[0] = th[0] = -1.f;
 #pragma unroll
-    for (int k = 0; k + 1 < K; ++k) t[k + 1] = fmaf(e[k], c1, -1.f + 2.f * (float)(k + 1) * kMinBin);
-    t[K] = 1.f;
+    for (int k = 0; k + 1 < K; ++k) {
+        tw[k + 1] = fmaf(ew[k], c1w, -1.f + 2.f * (float)(k + 1) * kMinBin);
+        th[k + 1] = fmaf(eh[k], c1h, -1.f + 2.f * (float)(k + 1) * kMinBin);
+    }
+    tw[K] = th[K] = 1.f;
+}
+
+// flow_math.cuh::knot_derivative (FAST flavour) of a raw output given in log2 units
+__device__ __forceinline__ float knot_derivative_log2(float r) {
+    return fmaf(LN2, r > 20.f * LOG2E ? r : lg2_approx(2.f + ex2_approx(r)), kMinDeriv);
 }
 
 // The rational-quadratic spline of flow_math.cuh::rq_spline (FAST flavour) for a point already known to lie in [-B, B],
 // evaluated in units of B (the bin ratios, the knot derivatives and the log-det do not depend on the unit).  The raw
 // derivatives of the two knots around the point's bin are fetched through `deriv(j)` once the bin is known -- the
-// conditioner's other K - 3 derivative outputs are never formed.
-template <int K, class DerivFn>
+// conditioner's other K - 3 derivative outputs are never formed.  FAST: raw outputs of a fast table (log2 units).
+template <int K, bool FAST, class DerivFn>
 __device__ __forceinline__ void rq_spline_lazy(const float *raw, float B, float inv_B, float edge_deriv, bool inverse, float &v, float &ld,
                                                DerivFn deriv) {
     float cw[K + 1], ch[K + 1];
-    unit_knots<K>(raw, 2.f * B, cw);
-    unit_knots<K>(raw + K, 2.f * B, ch);
+    unit_knots<K, FAST>(raw, 2.f * B, cw, ch);
     const float u = v * inv_B;
     const float *sk = inverse ? ch : cw;
     // bin = number of interior knots <= u (spline_flow.py:22-24,115-118; u lies inside [t_0, t_K], so the count needs no
@@ -348,25 +576,34 @@ __device__ __forceinline__ void rq_spline_lazy(const float *raw, float B, float 
     // interior knot derivatives (spline_flow.py:256,104), the padded constant at the two ends (:46-49); the loads are
     // unconditional on a clamped index so that lanes in different bins do not diverge
     const float r0 = deriv(max(idx - 1, 0)), r1 = deriv(min(idx, K - 2));
-    const float dk = (idx > 0) ? knot_derivative<true>(r0) : edge_deriv;
-    const float dk1 = (idx < K - 1) ? knot_derivative<true>(r1) : edge_deriv;
-    const float sk_ = __fdividef(hk, wk);  // spline_flow.py:123
-    const float dsum = dk + dk1 - 2.f * sk_;
-    if (inverse) {  // spline_flow.py:133-162
+    float dk, dk1;
+    if constexpr (FAST) {
+        dk = (idx > 0) ? knot_derivative_log2(r0) : edge_deriv;
+        dk1 = (idx < K - 1) ? knot_derivative_log2(r1) : edge_deriv;
+    } else {
+        dk = (idx > 0) ? knot_derivative<true>(r0) : edge_deriv;
+        dk1 = (idx < K - 1) ? knot_derivative<true>(r1) : edge_deriv;
+    }
+    if (inverse) {  // spline_flow.py:133-162 with the quadratic's coefficients and the log-det's terms multiplied by powers of wk,
+                    // which leaves the root and the ratio unchanged and needs no hk / wk
+        const float dkw = dk * wk, dk1w = dk1 * wk;
+        const float dsw = dkw + dk1w - 2.f * hk;  // dsum wk
         const float dy = u - yk;
-        const float a = dy * dsum + hk * (sk_ - dk);
-        const float b = hk * dk - dy * dsum;
-        const float c = -sk_ * dy;
+        const float a = dy * dsw + hk * (hk - dkw);
+        const float b = hk * dkw - dy * dsw;
+        const float c = -hk * dy;
         const float disc = fmaxf(b * b - 4.f * a * c, 0.f);
         const float root = __fdividef(2.f * c, -b - sqrt_approx(disc));
         v = (root * wk + xk) * B;
         const float tt = root * (1.f - root);
-        const float den = sk_ + dsum * tt;
         const float omr = 1.f - root;
-        const float num = (sk_ * sk_) * (dk1 * (root * root) + 2.f * sk_ * tt + dk * (omr * omr));
+        const float den = wk * (hk + dsw * tt);                                                   // den wk^2
+        const float num = (hk * hk) * wk * (dk1w * (root * root) + 2.f * hk * tt + dkw * (omr * omr));  // num wk^4
         const float rd = frcp<true>(den);
         ld -= __logf(num * rd * rd);
     } else {  // spline_flow.py:163-179
+        const float sk_ = __fdividef(hk, wk);  // spline_flow.py:123
+        const float dsum = dk + dk1 - 2.f * sk_;
         const float th = __fdividef(u - xk, wk);
         const float tt = th * (1.f - th);
         const float numer = hk * (sk_ * (th * th) + dk * tt);
@@ -457,13 +694,13 @@ __device__ __forceinline__ void build_exec(const Params &p, Exec *ex, int *n_exe
 // SM: every table of the program sits in shared memory (plain LDS); otherwise a table is read through a generic pointer
 // (shared memory if it fitted, the image in global memory if not).
 template <int K, bool SM>
-__device__ __forceinline__ void run_points(const Params &p, const float *smem, const int *s_off, const int *s_over, const Exec *ex,
-                                           int n_exec) {
+__device__ __forceinline__ void run_points(const Params &p, const float *smem, const int *s_off, const int *s_goff, const int *s_kind,
+                                           const Exec *ex, int n_exec) {
     const bool sum_lp = p.dir_flags & 2;
     auto table = [&](int g) -> const float * {
         if constexpr (SM) return smem + s_off[g];
         const int o = s_off[g];
-        return o >= 0 ? smem + o : p.image + p.gl.region[g];
+        return o >= 0 ? smem + o : p.image + s_goff[g];
     };
     const long long stride = (long long)gridDim.x * blockDim.x;
 #pragma unroll 1
@@ -488,9 +725,8 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
                 const int g = ei.z;
                 float s = 0.f, t = 0.f;
                 if (g < 0) {  // neither net: s = t = 0
-                } else if (!s_over[g]) {
-                    const float *tb = table(g);
-                    const float4 *row = reinterpret_cast<const float4 *>(tb + BP_FLOATS) + find_piece<SM>(tb, c) * AFF_STRIDE4;
+                } else if (s_kind[g] != KIND_OVER) {
+                    const float4 *row = piece_row<SM>(table(g), s_kind[g] == KIND_FAST, c, AFF_STRIDE4);
                     const float4 q = row[0];
                     const float d = c - row[1].x;
                     s = fmaf(q.x, d, q.z), t = fmaf(q.y, d, q.w);
@@ -515,9 +751,9 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
                     const float B = cs.x;
                     if (tr >= -B && tr <= B) {  // identity tails (also NaN), spline_flow.py:40,51-52: the conditioner is not needed
                         const int g = step ? ei.w : ei.z;
-                        if (!s_over[g]) {
-                            const float *tb = table(g);
-                            const float4 *row = reinterpret_cast<const float4 *>(tb + BP_FLOATS) + find_piece<SM>(tb, c) * nsf_stride4(K);
+                        const int kind = s_kind[g];
+                        if (kind != KIND_OVER) {
+                            const float4 *row = piece_row<SM>(table(g), kind == KIND_FAST, c, nsf_stride4(K));
                             const float d = c - row[nsf_org(K) / 4].x;
                             const float2 dd = make_float2(d, d);
                             float raw[2 * K];
@@ -528,10 +764,12 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
                                 raw[2 * j] = o.x, raw[2 * j + 1] = o.y;
                             }
                             const float2 *dv = reinterpret_cast<const float2 *>(row) + nsf_doff(K) / 2;
-                            rq_spline_lazy<K>(raw, B, cs.y, cs.z, (p.dir_flags & 1) != 0, tr, ld, [&](int j) {
+                            const auto deriv = [&](int j) {
                                 const float2 q = dv[j];
                                 return fmaf(q.x, d, q.y);
-                            });
+                            };
+                            if (kind == KIND_FAST) rq_spline_lazy<K, true>(raw, B, cs.y, cs.z, (p.dir_flags & 1) != 0, tr, ld, deriv);
+                            else rq_spline_lazy<K, false>(raw, B, cs.y, cs.z, (p.dir_flags & 1) != 0, tr, ld, deriv);
                         } else {
                             const mnf_flow_op &op = p.prog.ops[ei.y];
                             const float2 o = nsf_fallback<K>(p.params + op.net_off[use_f1 ? 0 : 1], op.n_lin, op.sizes, B, cs.z, c,
@@ -563,7 +801,7 @@ template <int K>
 __global__ void __launch_bounds__(THREADS, 1) flow_pl_kernel(const __grid_constant__ Params p) {
     extern __shared__ __align__(16) float smem[];
     __shared__ __align__(16) Exec s_exec[MNF_MAX_OPS];
-    __shared__ int s_off[MAX_GROUPS], s_over[MAX_GROUPS];
+    __shared__ int s_off[MAX_GROUPS], s_goff[MAX_GROUPS], s_kind[MAX_GROUPS];
     __shared__ int s_allfit, s_nexec;
     __shared__ __align__(8) unsigned long long s_bar;
     const int lane = threadIdx.x & 31, ng = p.gl.n;
@@ -575,17 +813,21 @@ __global__ void __launch_bounds__(THREADS, 1) flow_pl_kernel(const __grid_consta
     __syncthreads();
     if (threadIdx.x >= 32 && threadIdx.x < 64) build_exec(p, s_exec, &s_nexec, lane);
     if (threadIdx.x < 32) {
-        // table sizes from the builder's header -> shared-memory offsets, one bulk copy per table
+        // table sizes from the builder's header -> shared-memory offsets, one bulk copy per table of what its path reads:
+        // the fast form if it has one, else the breakpoints and rows
         const int *hdr = reinterpret_cast<const int *>(p.image);
         int total = 0, fit = 1;
         for (int base = 0; base < ng; base += 32) {
             const int g = base + lane;
-            int sz = 0, ov = 0;
+            int sz = 0, ov = 0, src = 0;
             if (g < ng) {
-                const int2 h = *reinterpret_cast<const int2 *>(hdr + g * HDR_INTS);
+                const int4 h = *reinterpret_cast<const int4 *>(hdr + g * HDR_INTS);
                 const int s4 = p.prog.ops[p.gl.op[g]].type == MNF_OP_NSF_CL ? nsf_stride4(K) : AFF_STRIDE4;
                 ov = h.y;
-                sz = ov ? 0 : BP_FLOATS + (h.x + 1) * 4 * s4;
+                src = p.gl.region[g] + h.z;
+                sz = ov ? 0 : h.z ? h.w : BP_FLOATS + (h.x + 1) * 4 * s4;
+                s_kind[g] = ov ? KIND_OVER : h.z ? KIND_FAST : KIND_PLAIN;
+                s_goff[g] = src;
             }
             int inc = sz;
 #pragma unroll
@@ -597,10 +839,9 @@ __global__ void __launch_bounds__(THREADS, 1) flow_pl_kernel(const __grid_consta
             const bool ok = off + sz <= p.smem_floats;
             if (g < ng) {
                 s_off[g] = (ov || !ok) ? -1 : off;
-                s_over[g] = ov;
                 if (!ov && ok) {
                     asm volatile("mbarrier.expect_tx.relaxed.cta.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"((uint32_t)sz * 4u) : "memory");
-                    bulk_load(smem_u32(smem + off), p.image + p.gl.region[g], (uint32_t)sz * 4u, bar);
+                    bulk_load(smem_u32(smem + off), p.image + src, (uint32_t)sz * 4u, bar);
                 }
             }
             fit &= __all_sync(0xffffffffu, g >= ng || ov || ok) ? 1 : 0;
@@ -614,8 +855,8 @@ __global__ void __launch_bounds__(THREADS, 1) flow_pl_kernel(const __grid_consta
     }
     __syncthreads();
     mbar_wait(bar, 0);
-    if (s_allfit) run_points<K, true>(p, smem, s_off, s_over, s_exec, s_nexec);
-    else run_points<K, false>(p, smem, s_off, s_over, s_exec, s_nexec);
+    if (s_allfit) run_points<K, true>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
+    else run_points<K, false>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
 }
 
 // ---------------------------------------------------------------------------------------------------------
