@@ -12,7 +12,7 @@
 //                          it has at most one zero there), sorts them, and writes per piece the slope and the value at the
 //                          piece's origin of every output.  Exact up to fp64 rounding -- closer to the real-number net than
 //                          an fp32 evaluation of its layers.
-//   flow_pl_kernel<K>      one thread per point, the whole stack in one launch: a conditioner is a branch-free binary
+//   flow_pl_kernel<K, INV> one thread per point, the whole stack in one launch: a conditioner is a branch-free binary
 //                          search over <= 511 sorted breakpoints in shared memory and one FMA per output
 //                          (out = V_i + A_i (c - origin_i)); the spline (flow_math.cuh) then runs on the raw outputs, and only
 //                          the two knot derivatives of the bin the point falls into are ever formed.  Tables with a fast form
@@ -395,6 +395,12 @@ __device__ __forceinline__ float2 f2_fma(float2 a, float2 b, float2 c) {
     asm("fma.rn.f32x2 %0, %1, %2, %3;" : "=l"(rd) : "l"(ra), "l"(rb), "l"(rc));
     return *reinterpret_cast<float2 *>(&rd);
 }
+__device__ __forceinline__ float2 f2_add(float2 a, float2 b) {
+    unsigned long long ra = *reinterpret_cast<unsigned long long *>(&a), rb = *reinterpret_cast<unsigned long long *>(&b), rd;
+    asm("add.rn.f32x2 %0, %1, %2;" : "=l"(rd) : "l"(ra), "l"(rb));
+    return *reinterpret_cast<float2 *>(&rd);
+}
+__device__ __forceinline__ float2 f2_splat(float a) { return make_float2(a, a); }
 
 // exact-fp32 evaluation of a net layer by layer (tables that overflowed): parameter blob, per Linear weight[out][in], bias[out]
 __device__ __noinline__ void mlp_fp32(const float *__restrict__ net, int n_lin, const int *sizes, float c, float *out) {
@@ -489,60 +495,58 @@ __device__ __forceinline__ float lg2_approx(float x) {
 
 constexpr float LOG2E = 1.4426950408889634f, LN2 = 0.6931471805599453f;
 
-// Knots of the two spline axes in units of B: t[0] = -1, t[K] = 1.  The formulas of flow_math.cuh::spline_knots (both
-// softmaxes of spline_flow.py:253-255 and :95, floor :96-97, cumsum :99, pinned ends :100-101) with the cumulative sum
-// taken over the second softmax's terms while they are summed: x_{k+1} / B = -1 + 2 (k + 1) min_bin + (2 span / sum f) * (f_0 + .. + f_k),
-// one FFMA per knot.
+// constant part of knot k in units of B: -1 + 2 k min_bin
+__device__ __forceinline__ float knot_const(float k) { return fmaf(2.f * kMinBin, k, -1.f); }
+
+// The two spline axes of a conditioner in units of B, as prefix sums S[k < K - 1] = (f_0 + .. + f_k) of the second softmax's
+// terms (x = width, y = height axis) and their scales c1 = 2 span / sum f: knot k + 1 is knot_const(k + 1) + c1 S[k], one
+// FMA (t[0] = -1, t[K] = 1 pinned) -- the formulas of flow_math.cuh::spline_knots (both softmaxes of
+// spline_flow.py:253-255 and :95, floor :96-97, cumsum :99, pinned ends :100-101).
 // FAST: raw holds the outputs of a fast table (log2 units, largest in [0, FAST_T]): no max to subtract, every first-softmax
 // sum lies in [1, K 2^FAST_T] and, with the second softmax's arguments centred on 0, every second-softmax sum in
 // [e^-B, K e^B], so each pair of sums is inverted by one reciprocal of its product.  Otherwise (natural units) the
 // largest output of each axis is subtracted first.
 template <int K, bool FAST>
-__device__ __forceinline__ void unit_knots(const float *raw, float twoB, float *tw, float *th) {
+__device__ __forceinline__ void unit_knots(const float *raw, float twoB, float2 *S, float2 &c1) {
     constexpr float span = 1.f - kMinBin * (float)K;
-    float ew[K], eh[K], sw = 0.f, sh = 0.f, scw, sch, offw, offh;
+    float2 e[K], sc, off;
     if constexpr (FAST) {
+        float2 s1;
 #pragma unroll
         for (int k = 0; k < K; ++k) {
-            ew[k] = ex2_approx(raw[k]), eh[k] = ex2_approx(raw[K + k]);
-            sw += ew[k], sh += eh[k];
+            e[k] = make_float2(ex2_approx(raw[k]), ex2_approx(raw[K + k]));
+            s1 = k ? f2_add(s1, e[k]) : e[k];
         }
-        const float r = frcp<true>(sw * sh), s = twoB * LOG2E;  // first softmax scaled by 2B, in log2 units
-        scw = s * (r * sh), sch = s * (r * sw);
-        offw = offh = -0.5f * s;
+        const float r = frcp<true>(s1.x * s1.y), s = twoB * LOG2E;  // first softmax scaled by 2B, in log2 units
+        sc = make_float2(s * (r * s1.y), s * (r * s1.x));
+        off = f2_splat(-0.5f * s);
     } else {
-        float mw = raw[0], mh = raw[K];
+        float mw = raw[0], mh = raw[K], sw = 0.f, sh = 0.f;
 #pragma unroll
         for (int k = 1; k < K; ++k) mw = fmaxf(mw, raw[k]), mh = fmaxf(mh, raw[K + k]);
         const float mwn = -mw * LOG2E, mhn = -mh * LOG2E;
 #pragma unroll
         for (int k = 0; k < K; ++k) {
-            ew[k] = ex2_approx(fmaf(raw[k], LOG2E, mwn)), eh[k] = ex2_approx(fmaf(raw[K + k], LOG2E, mhn));
-            sw += ew[k], sh += eh[k];
+            e[k] = make_float2(ex2_approx(fmaf(raw[k], LOG2E, mwn)), ex2_approx(fmaf(raw[K + k], LOG2E, mhn)));
+            sw += e[k].x, sh += e[k].y;
         }
-        scw = twoB * frcp<true>(sw) * LOG2E, sch = twoB * frcp<true>(sh) * LOG2E;
-        offw = twoB > 80.f ? -scw : 0.f, offh = twoB > 80.f ? -sch : 0.f;  // arguments of the second softmax lie in [0, 2B]
+        sc = make_float2(twoB * frcp<true>(sw) * LOG2E, twoB * frcp<true>(sh) * LOG2E);
+        off = make_float2(twoB > 80.f ? -sc.x : 0.f, twoB > 80.f ? -sc.y : 0.f);  // arguments of the second softmax lie in [0, 2B]
     }
-    float pw = 0.f, ph = 0.f;
+    float2 p;
 #pragma unroll
     for (int k = 0; k < K; ++k) {
-        pw += ex2_approx(fmaf(ew[k], scw, offw)), ph += ex2_approx(fmaf(eh[k], sch, offh));
-        ew[k] = pw, eh[k] = ph;
+        const float2 a = f2_fma(e[k], sc, off);
+        const float2 x = make_float2(ex2_approx(a.x), ex2_approx(a.y));
+        p = k ? f2_add(p, x) : x;
+        if (k + 1 < K) S[k] = p;
     }
-    float c1w, c1h;
     if constexpr (FAST) {
-        const float r = frcp<true>(pw * ph);
-        c1w = 2.f * span * (r * ph), c1h = 2.f * span * (r * pw);
+        const float r = frcp<true>(p.x * p.y);
+        c1 = make_float2(2.f * span * (r * p.y), 2.f * span * (r * p.x));
     } else {
-        c1w = 2.f * span * frcp<true>(pw), c1h = 2.f * span * frcp<true>(ph);
+        c1 = make_float2(2.f * span * frcp<true>(p.x), 2.f * span * frcp<true>(p.y));
     }
-    tw[0] = th[0] = -1.f;
-#pragma unroll
-    for (int k = 0; k + 1 < K; ++k) {
-        tw[k + 1] = fmaf(ew[k], c1w, -1.f + 2.f * (float)(k + 1) * kMinBin);
-        th[k + 1] = fmaf(eh[k], c1h, -1.f + 2.f * (float)(k + 1) * kMinBin);
-    }
-    tw[K] = th[K] = 1.f;
 }
 
 // flow_math.cuh::knot_derivative (FAST flavour) of a raw output given in log2 units
@@ -550,28 +554,51 @@ __device__ __forceinline__ float knot_derivative_log2(float r) {
     return fmaf(LN2, r > 20.f * LOG2E ? r : lg2_approx(2.f + ex2_approx(r)), kMinDeriv);
 }
 
+// Log-det of the spline conditioners of a point as a running product P in [1, 2) times 2^E: one lg2 per point at the end
+// instead of one log per conditioner.  Renormalising multiplies by 2^(127 - exponent field), so 0 and NaN stay what they
+// are.
+__device__ __forceinline__ void ld_mul(float &P, int &E, float q) {
+    P *= q;
+    const int eb = __float_as_int(P) & 0x7f800000;
+    E += (eb >> 23) - 127;
+    P *= __int_as_float(0x7f000000 - eb);
+}
+// ld += (log P + E log 2) negated for INV, and the product reset.  (Also before the calls of the layer-by-layer fallbacks:
+// P and E are then not live across them, which keeps the point loop's state in registers.)
+template <bool INV>
+__device__ __forceinline__ void ld_flush(float &ld, float &P, int &E) {
+    ld = fmaf(INV ? -LN2 : LN2, lg2_approx(P) + (float)E, ld);  // P in [1, 2) (or 0, NaN): no denormal operand
+    P = 1.f, E = 0;
+}
+
 // The rational-quadratic spline of flow_math.cuh::rq_spline (FAST flavour) for a point already known to lie in [-B, B],
 // evaluated in units of B (the bin ratios, the knot derivatives and the log-det do not depend on the unit).  The raw
 // derivatives of the two knots around the point's bin are fetched through `deriv(j)` once the bin is known -- the
-// conditioner's other K - 3 derivative outputs are never formed.  FAST: raw outputs of a fast table (log2 units).
-template <int K, bool FAST, class DerivFn>
-__device__ __forceinline__ void rq_spline_lazy(const float *raw, float B, float inv_B, float edge_deriv, bool inverse, float &v, float &ld,
+// conditioner's other K - 3 derivative outputs are never formed.  FAST: raw outputs of a fast table (log2 units).  The
+// forward spline's derivative at the point goes into the log-det product (P, E) of ld_mul; INV subtracts its log.
+template <int K, bool FAST, bool INV, class DerivFn>
+__device__ __forceinline__ void rq_spline_lazy(const float *raw, float B, float inv_B, float edge_deriv, float &v, float &P, int &E,
                                                DerivFn deriv) {
-    float cw[K + 1], ch[K + 1];
-    unit_knots<K, FAST>(raw, 2.f * B, cw, ch);
+    float2 S[K - 1], c1;
+    unit_knots<K, FAST>(raw, 2.f * B, S, c1);
     const float u = v * inv_B;
-    const float *sk = inverse ? ch : cw;
     // bin = number of interior knots <= u (spline_flow.py:22-24,115-118; u lies inside [t_0, t_K], so the count needs no
-    // clamp); the knots of both axes around it are picked with the same predicates
+    // clamp).  Only the searched axis's knots are formed; the prefix sums at both ends of the bin are picked for both axes
+    // with the same predicates, and the knots made from them afterwards.
     int idx = 0;
-    float xk = cw[0], xk1 = cw[1], yk = ch[0], yk1 = ch[1];
+    float2 lo = f2_splat(0.f), hi = S[0];
 #pragma unroll
     for (int k = 1; k < K; ++k) {
-        const bool ge = u >= sk[k];
+        const bool ge = u >= fmaf(INV ? S[k - 1].y : S[k - 1].x, INV ? c1.y : c1.x, knot_const((float)k));
         idx += ge ? 1 : 0;
-        xk = ge ? cw[k] : xk, xk1 = ge ? cw[k + 1] : xk1;
-        yk = ge ? ch[k] : yk, yk1 = ge ? ch[k + 1] : yk1;
+        lo = ge ? S[k - 1] : lo;
+        if (k + 1 < K) hi = ge ? S[k] : hi;  // (the last bin's upper knots are pinned)
     }
+    const float fidx = __int_as_float(0x4b000000 | idx) - 8388608.f;  // (float)idx without the XU pipe
+    const float k0 = knot_const(fidx), k1 = knot_const(fidx + 1.f);
+    const float xk = fmaf(lo.x, c1.x, k0), yk = fmaf(lo.y, c1.y, k0);
+    const bool last = idx == K - 1;
+    const float xk1 = last ? 1.f : fmaf(hi.x, c1.x, k1), yk1 = last ? 1.f : fmaf(hi.y, c1.y, k1);
     const float wk = xk1 - xk, hk = yk1 - yk;  // spline_flow.py:102,113
     // interior knot derivatives (spline_flow.py:256,104), the padded constant at the two ends (:46-49); the loads are
     // unconditional on a clamped index so that lanes in different bins do not diverge
@@ -584,8 +611,12 @@ __device__ __forceinline__ void rq_spline_lazy(const float *raw, float B, float 
         dk = (idx > 0) ? knot_derivative<true>(r0) : edge_deriv;
         dk1 = (idx < K - 1) ? knot_derivative<true>(r1) : edge_deriv;
     }
-    if (inverse) {  // spline_flow.py:133-162 with the quadratic's coefficients and the log-det's terms multiplied by powers of wk,
-                    // which leaves the root and the ratio unchanged and needs no hk / wk
+    // Reciprocals are rcp.approx.ftz, which differs from __fdividef only where the operand is not a normal number; every
+    // operand below is a product or sum of bin widths and heights (>= 2 min_bin), knot derivatives (>= min_deriv) and
+    // terms in [0, 1], so it is not below the normal range.  (-b - sqrt(disc) is -2 hk dk wk at dy = 0 and grows in
+    // magnitude with dy.)  Above 2^126 (a knot derivative near the fp32 limit) both forms return 0.
+    if constexpr (INV) {  // spline_flow.py:133-162 with the quadratic's coefficients and the log-det's terms multiplied by powers
+                          // of wk, which leaves the root and the ratio unchanged and needs no hk / wk
         const float dkw = dk * wk, dk1w = dk1 * wk;
         const float dsw = dkw + dk1w - 2.f * hk;  // dsum wk
         const float dy = u - yk;
@@ -593,18 +624,19 @@ __device__ __forceinline__ void rq_spline_lazy(const float *raw, float B, float 
         const float b = hk * dkw - dy * dsw;
         const float c = -hk * dy;
         const float disc = fmaxf(b * b - 4.f * a * c, 0.f);
-        const float root = __fdividef(2.f * c, -b - sqrt_approx(disc));
+        const float root = 2.f * c * frcp<true>(-b - sqrt_approx(disc));
         v = (root * wk + xk) * B;
         const float tt = root * (1.f - root);
         const float omr = 1.f - root;
         const float den = wk * (hk + dsw * tt);                                                   // den wk^2
         const float num = (hk * hk) * wk * (dk1w * (root * root) + 2.f * hk * tt + dkw * (omr * omr));  // num wk^4
         const float rd = frcp<true>(den);
-        ld -= __logf(num * rd * rd);
+        ld_mul(P, E, num * rd * rd);
     } else {  // spline_flow.py:163-179
-        const float sk_ = __fdividef(hk, wk);  // spline_flow.py:123
+        const float rw = frcp<true>(wk);
+        const float sk_ = hk * rw;  // spline_flow.py:123
         const float dsum = dk + dk1 - 2.f * sk_;
-        const float th = __fdividef(u - xk, wk);
+        const float th = (u - xk) * rw;
         const float tt = th * (1.f - th);
         const float numer = hk * (sk_ * (th * th) + dk * tt);
         const float den = sk_ + dsum * tt;
@@ -612,7 +644,7 @@ __device__ __forceinline__ void rq_spline_lazy(const float *raw, float B, float 
         const float num = (sk_ * sk_) * (dk1 * (th * th) + 2.f * sk_ * tt + dk * (omt * omt));
         const float rd = frcp<true>(den);
         v = fmaf(numer, rd, yk) * B;
-        ld += __logf(num * rd * rd);
+        ld_mul(P, E, num * rd * rd);
     }
 }
 
@@ -693,7 +725,7 @@ __device__ __forceinline__ void build_exec(const Params &p, Exec *ex, int *n_exe
 
 // SM: every table of the program sits in shared memory (plain LDS); otherwise a table is read through a generic pointer
 // (shared memory if it fitted, the image in global memory if not).
-template <int K, bool SM>
+template <int K, bool SM, bool INV>
 __device__ __forceinline__ void run_points(const Params &p, const float *smem, const int *s_off, const int *s_goff, const int *s_kind,
                                            const Exec *ex, int n_exec) {
     const bool sum_lp = p.dir_flags & 2;
@@ -705,7 +737,8 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
     const long long stride = (long long)gridDim.x * blockDim.x;
 #pragma unroll 1
     for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < p.n_rows; r += stride) {
-        float v0, v1, ld = 0.f;
+        float v0, v1, ld = 0.f, P = 1.f;  // log-det: ld + (log P + E log 2) of the spline conditioners (ld_mul), negated for INV
+        int E = 0;
         {
             const float2 xin = ld_stream2(reinterpret_cast<const float2 *>(p.x) + r);
             v0 = xin.x, v1 = xin.y;
@@ -731,10 +764,11 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
                     const float d = c - row[1].x;
                     s = fmaf(q.x, d, q.z), t = fmaf(q.y, d, q.w);
                 } else {
+                    ld_flush<INV>(ld, P, E);
                     if (op.flags & MNF_FLAG_SCALE) s = mlp_fp32_scalar(p.params + op.net_off[0], op.n_lin, op.sizes, c);
                     if (op.flags & MNF_FLAG_SHIFT) t = mlp_fp32_scalar(p.params + op.net_off[1], op.n_lin, op.sizes, c);
                 }
-                if (p.dir_flags & 1) {  // affine_half_flow.py:54-56
+                if constexpr (INV) {  // affine_half_flow.py:54-56
                     tr = (tr - t) / expf(s), ld -= s;
                 } else {  // affine_half_flow.py:58
                     tr = expf(s) * tr + t, ld += s;
@@ -768,12 +802,13 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
                                 const float2 q = dv[j];
                                 return fmaf(q.x, d, q.y);
                             };
-                            if (kind == KIND_FAST) rq_spline_lazy<K, true>(raw, B, cs.y, cs.z, (p.dir_flags & 1) != 0, tr, ld, deriv);
-                            else rq_spline_lazy<K, false>(raw, B, cs.y, cs.z, (p.dir_flags & 1) != 0, tr, ld, deriv);
+                            if (kind == KIND_FAST) rq_spline_lazy<K, true, INV>(raw, B, cs.y, cs.z, tr, P, E, deriv);
+                            else rq_spline_lazy<K, false, INV>(raw, B, cs.y, cs.z, tr, P, E, deriv);
                         } else {
                             const mnf_flow_op &op = p.prog.ops[ei.y];
+                            ld_flush<INV>(ld, P, E);
                             const float2 o = nsf_fallback<K>(p.params + op.net_off[use_f1 ? 0 : 1], op.n_lin, op.sizes, B, cs.z, c,
-                                                             (p.dir_flags & 1) != 0, tr);
+                                                             INV, tr);
                             tr = o.x, ld += o.y;
                         }
                         if (use_f1) v1 = tr; else v0 = tr;
@@ -782,6 +817,7 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
             }
             if (p.inter) st_stream2(reinterpret_cast<float2 *>(p.inter + ((size_t)kk * p.n_rows + r) * 2), make_float2(v0, v1));
         }
+        ld_flush<INV>(ld, P, E);
         float lp = fmaf(-0.5f, fmaf(v0, v0, v1 * v1), -1.8378770664093453f);  // -(D/2) log(2 pi), D = 2
         if (sum_lp) lp += ld;
         if (p.y) st_stream2(reinterpret_cast<float2 *>(p.y) + r, make_float2(v0, v1));
@@ -797,7 +833,7 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
     }
 }
 
-template <int K>
+template <int K, bool INV>
 __global__ void __launch_bounds__(THREADS, 1) flow_pl_kernel(const __grid_constant__ Params p) {
     extern __shared__ __align__(16) float smem[];
     __shared__ __align__(16) Exec s_exec[MNF_MAX_OPS];
@@ -855,8 +891,8 @@ __global__ void __launch_bounds__(THREADS, 1) flow_pl_kernel(const __grid_consta
     }
     __syncthreads();
     mbar_wait(bar, 0);
-    if (s_allfit) run_points<K, true>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
-    else run_points<K, false>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
+    if (s_allfit) run_points<K, true, INV>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
+    else run_points<K, false, INV>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -920,20 +956,20 @@ static Plan make_plan(const mnf_flow_op *ops, int n_ops, int dim) {
     return pl;
 }
 
-template <int K>
+template <int K, bool INV>
 static int launch_k(const Params &p, const DeviceProps *dp, size_t smem_bytes, cudaStream_t st) {
     static thread_local size_t attr_set[64] = {};  // per device: the attribute belongs to the device's copy of the function
     int dev = 0;
     MNF_CUDA(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64 || attr_set[dev] < smem_bytes) {
-        MNF_CUDA(cudaFuncSetAttribute(flow_pl_kernel<K>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
+        MNF_CUDA(cudaFuncSetAttribute(flow_pl_kernel<K, INV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
         if (dev >= 0 && dev < 64) attr_set[dev] = smem_bytes;
     }
     // small batches are bound by the latency of one point's chain: spread the points over the SMs
     const int threads = p.n_rows <= (long long)dp->sm_count * 64 ? 64 : p.n_rows <= (long long)dp->sm_count * 256 ? 256 : THREADS;
     long long blocks = (p.n_rows + threads - 1) / threads;
     if (blocks > dp->sm_count) blocks = dp->sm_count;
-    flow_pl_kernel<K><<<(unsigned)blocks, threads, smem_bytes, st>>>(p);
+    flow_pl_kernel<K, INV><<<(unsigned)blocks, threads, smem_bytes, st>>>(p);
     return launch_status("flow_pl_kernel");
 }
 
@@ -1000,7 +1036,8 @@ int launch_flow_pl(const mnf_flow_op *ops, int n_ops, const float *params, const
     if (want > cap) want = cap;
     want &= ~(size_t)15;
     p.smem_floats = (int)(want / sizeof(float));
-#define MNF_PL_LAUNCH(KK) if (pl.K == KK) return launch_k<KK>(p, dp, want, stream);
+#define MNF_PL_LAUNCH(KK) \
+    if (pl.K == KK) return (dir_flags & 1) ? launch_k<KK, true>(p, dp, want, stream) : launch_k<KK, false>(p, dp, want, stream);
     MNF_PL_BINS(MNF_PL_LAUNCH)
 #undef MNF_PL_LAUNCH
     return 1;
