@@ -187,6 +187,24 @@ int64_t mnf_flow_stack_workspace(int n_ops, int64_t n_rows, int dim);
  *    5 = eight lanes per point (AffineHalfFlow stacks up to 32768 rows); 3 (round 1's constant-bank variant, removed) runs 2.
  *    A variant the program is not eligible for falls back to the library default. */
 
+/* Draws n_rows points of the flow model (standard-normal base, flows in module order) together with their log-density:
+ *   z[r]        = N(0, I) draw of global row row_offset + r (Noise convention of the MNF layers below: Philox4x32-10
+ *                 keyed by `seed`, stream `noise_stream`, GLOBAL element index (row_offset + r) * dim + c as counter, the
+ *                 same numbers as every other Philox draw of the library -- shards of one draw, each with its
+ *                 row_offset, reproduce the single call bit for bit);
+ *   x[r]        = forward pass of z[r] (NormalizingFlowModel.sample, flows/core.py:51-55);
+ *   log_prob[r] = log N(z[r]) - log|det J|(z[r]) = log q(x[r]), the density of the drawn point, without the inverse pass.
+ * x, log_prob and z are each optional (NULL), at least one must be given.  flags: MNF_RUN_STAGED, MNF_RUN_GENERIC and
+ * MNF_RUN_VARIANT(v) as for mnf_flow_stack_run (forward direction only: MNF_RUN_INVERSE and MNF_RUN_LOGPROB are
+ * MNF_E_ARG).  Programs of the piecewise-linear kernel with a workspace or staged image take ONE launch (after the table
+ * builder when not staged); every other program draws z, runs the forward dispatch of mnf_flow_stack_run and finishes
+ * log_prob: at most three launches, and x or z must be given to hold the draw.  Box-Muller draws u1 >= 2^-23, so every
+ * pair lies within radius 5.65 (a pair of true normals exceeds it with probability 2^-23). */
+int mnf_flow_stack_sample(const mnf_flow_op *ops_host, int n_ops, const float *params, int64_t n_params,
+                          uint64_t seed, uint32_t noise_stream, uint64_t row_offset,
+                          float *x, float *log_prob, float *z, int64_t n_rows, int dim,
+                          int flags, float *workspace, void *stream);
+
 /* Per-parameter-version preparation of a dim-2 stack, done ONCE instead of in every call (call it again whenever a
  * parameter changes): mnf_flow_stack_stage writes into a caller-owned, 16-byte aligned buffer of
  * mnf_flow_stack_stage_size() floats (0 = the program has no such form)

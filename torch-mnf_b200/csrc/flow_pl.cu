@@ -12,12 +12,15 @@
 //                          it has at most one zero there), sorts them, and writes per piece the slope and the value at the
 //                          piece's origin of every output.  Exact up to fp64 rounding -- closer to the real-number net than
 //                          an fp32 evaluation of its layers.
-//   flow_pl_kernel<K, INV> one thread per point, the whole stack in one launch: a conditioner is a branch-free binary
+//   flow_pl_kernel<K, INV[, DRAW]>
+//                          one thread per point, the whole stack in one launch: a conditioner is a branch-free binary
 //                          search over <= 511 sorted breakpoints in shared memory and one FMA per output
 //                          (out = V_i + A_i (c - origin_i)); the spline (flow_math.cuh) then runs on the raw outputs, and only
 //                          the two knot derivatives of the bin the point falls into are ever formed.  Tables with a fast form
 //                          (written by the builder next to the plain one) are looked up through a bucket index instead, and
-//                          their spline outputs come pre-shifted for the softmax.
+//                          their spline outputs come pre-shifted for the softmax.  DRAW (forward direction only): the
+//                          point's z is drawn from Philox in place of being loaded, and log q(x) = log N(z) - log-det
+//                          comes out of the same pass (mnf_flow_stack_sample).
 //
 // Per point and conditioner: ~60 instructions instead of 5 376 multiply-adds (or three MMA round trips).  No tensor core
 // and no FMA chain is left to feed: what remains is the spline arithmetic and 12 B/pt of HBM traffic.
@@ -26,6 +29,7 @@
 // tables live in the caller's workspace (built per call) or in the image of mnf_flow_stack_stage (built per parameter
 // version).
 #include "flow_math.cuh"
+#include "mnf_common.cuh"
 #include "tc_common.cuh"
 
 namespace mnf {
@@ -387,6 +391,10 @@ struct Params {
     long long n_rows;
     int dir_flags, smem_floats;
     mnf_gather_out gather;
+    // DRAW only (after the fields above, so that the other instantiations see the same layout)
+    unsigned long long seed, row_offset;  // Philox key; global index of local row 0
+    float *z;                             // optional output: the drawn base point
+    unsigned noise_stream;
 };
 
 __device__ __forceinline__ float2 f2_fma(float2 a, float2 b, float2 c) {
@@ -725,7 +733,7 @@ __device__ __forceinline__ void build_exec(const Params &p, Exec *ex, int *n_exe
 
 // SM: every table of the program sits in shared memory (plain LDS); otherwise a table is read through a generic pointer
 // (shared memory if it fitted, the image in global memory if not).
-template <int K, bool SM, bool INV>
+template <int K, bool SM, bool INV, bool DRAW>
 __device__ __forceinline__ void run_points(const Params &p, const float *smem, const int *s_off, const int *s_goff, const int *s_kind,
                                            const Exec *ex, int n_exec) {
     const bool sum_lp = p.dir_flags & 2;
@@ -739,7 +747,18 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
     for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < p.n_rows; r += stride) {
         float v0, v1, ld = 0.f, P = 1.f;  // log-det: ld + (log P + E log 2) of the spline conditioners (ld_mul), negated for INV
         int E = 0;
-        {
+        if constexpr (DRAW) {
+            // philox_normal's mapping of global element e = 2 (row_offset + r) + col: counter e >> 2, words (x, y) for even
+            // global rows and (z, w) for odd ones -- the numbers every Philox draw of the library gives for these indices.
+            // The running log-det starts at -log N(z), so that -ld is log q(x) at the end.
+            const unsigned long long gr = p.row_offset + (unsigned long long)r;
+            const uint4 w = Philox(p.seed)(gr >> 1, p.noise_stream);
+            const bool odd = gr & 1ull;
+            const float2 zn = box_muller(odd ? w.z : w.x, odd ? w.w : w.y);
+            v0 = zn.x, v1 = zn.y;
+            if (p.z) st_stream2(reinterpret_cast<float2 *>(p.z) + r, zn);
+            ld = fmaf(0.5f, fmaf(v0, v0, v1 * v1), 1.8378770664093453f);
+        } else {
             const float2 xin = ld_stream2(reinterpret_cast<const float2 *>(p.x) + r);
             v0 = xin.x, v1 = xin.y;
         }
@@ -820,10 +839,12 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
         ld_flush<INV>(ld, P, E);
         float lp = fmaf(-0.5f, fmaf(v0, v0, v1 * v1), -1.8378770664093453f);  // -(D/2) log(2 pi), D = 2
         if (sum_lp) lp += ld;
+        if constexpr (DRAW) lp = -ld;  // log N(z) - log_det
         if (p.y) st_stream2(reinterpret_cast<float2 *>(p.y) + r, make_float2(v0, v1));
         if (p.log_det) p.log_det[r] = ld;
         if (p.base_lp) p.base_lp[r] = lp;
         // fused gather: the result also goes straight to the other ranks over NVLink
+        if constexpr (DRAW) continue;
         if (p.gather.multicast_ptr) {
             asm volatile("multimem.st.relaxed.sys.global.f32 [%0], %1;" ::"l"(p.gather.multicast_ptr + p.gather.row_offset + r), "f"(lp)
                          : "memory");
@@ -833,7 +854,7 @@ __device__ __forceinline__ void run_points(const Params &p, const float *smem, c
     }
 }
 
-template <int K, bool INV>
+template <int K, bool INV, bool DRAW = false>
 __global__ void __launch_bounds__(THREADS, 1) flow_pl_kernel(const __grid_constant__ Params p) {
     extern __shared__ __align__(16) float smem[];
     __shared__ __align__(16) Exec s_exec[MNF_MAX_OPS];
@@ -891,8 +912,8 @@ __global__ void __launch_bounds__(THREADS, 1) flow_pl_kernel(const __grid_consta
     }
     __syncthreads();
     mbar_wait(bar, 0);
-    if (s_allfit) run_points<K, true, INV>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
-    else run_points<K, false, INV>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
+    if (s_allfit) run_points<K, true, INV, DRAW>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
+    else run_points<K, false, INV, DRAW>(p, smem, s_off, s_goff, s_kind, s_exec, s_nexec);
 }
 
 // ---------------------------------------------------------------------------------------------------------
@@ -956,22 +977,27 @@ static Plan make_plan(const mnf_flow_op *ops, int n_ops, int dim) {
     return pl;
 }
 
-template <int K, bool INV>
+template <int K, bool INV, bool DRAW = false>
 static int launch_k(const Params &p, const DeviceProps *dp, size_t smem_bytes, cudaStream_t st) {
     static thread_local size_t attr_set[64] = {};  // per device: the attribute belongs to the device's copy of the function
     int dev = 0;
     MNF_CUDA(cudaGetDevice(&dev));
     if (dev < 0 || dev >= 64 || attr_set[dev] < smem_bytes) {
-        MNF_CUDA(cudaFuncSetAttribute(flow_pl_kernel<K, INV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
+        MNF_CUDA(cudaFuncSetAttribute(flow_pl_kernel<K, INV, DRAW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
         if (dev >= 0 && dev < 64) attr_set[dev] = smem_bytes;
     }
     // small batches are bound by the latency of one point's chain: spread the points over the SMs
     const int threads = p.n_rows <= (long long)dp->sm_count * 64 ? 64 : p.n_rows <= (long long)dp->sm_count * 256 ? 256 : THREADS;
     long long blocks = (p.n_rows + threads - 1) / threads;
     if (blocks > dp->sm_count) blocks = dp->sm_count;
-    flow_pl_kernel<K, INV><<<(unsigned)blocks, threads, smem_bytes, st>>>(p);
+    flow_pl_kernel<K, INV, DRAW><<<(unsigned)blocks, threads, smem_bytes, st>>>(p);
     return launch_status("flow_pl_kernel");
 }
+
+// The part of a point kernel's launch that does not depend on the direction: the tables (built into `workspace` unless
+// it is staged), the program, the row count and the shared memory the kernel asks for (`want` bytes).
+static int setup_params(const Plan &pl, const mnf_flow_op *ops, int n_ops, const float *params, float *workspace, int64_t n_rows,
+                        bool staged, const DeviceProps *dp, cudaStream_t stream, Params &p, size_t &want);
 
 }  // namespace fpl
 
@@ -1000,6 +1026,25 @@ int flow_pl_build(const mnf_flow_op *ops, int n_ops, const float *params, int di
     return launch_status("flow_pl_build_kernel");
 }
 
+int fpl::setup_params(const Plan &pl, const mnf_flow_op *ops, int n_ops, const float *params, float *workspace, int64_t n_rows,
+                      bool staged, const DeviceProps *dp, cudaStream_t stream, Params &p, size_t &want) {
+    if (!staged) {
+        const int rc = flow_pl_build(ops, n_ops, params, 2, workspace, stream);
+        if (rc) return rc;
+    }
+    p.prog.n_ops = n_ops;
+    for (int k = 0; k < n_ops; ++k) p.prog.ops[k] = ops[k];
+    p.gl = pl.gl;
+    p.params = params, p.image = workspace, p.n_rows = n_rows;
+    // shared memory: every table at its largest, capped by what a CTA can have
+    want = (size_t)(pl.image_floats - HDR_FLOATS) * sizeof(float);
+    const size_t cap = (size_t)dp->smem_optin - 4096;  // static shared memory of the kernel: execution list, offsets, barrier
+    if (want > cap) want = cap;
+    want &= ~(size_t)15;
+    p.smem_floats = (int)(want / sizeof(float));
+    return 0;
+}
+
 // returns 1 if the program is not eligible (caller falls back to the other dim-2 kernels).  dir_flags: bit0 inverse,
 // bit1 log-det summed into base_lp, bit2 `workspace` already holds the image of flow_pl_build for these parameters.
 int launch_flow_pl(const mnf_flow_op *ops, int n_ops, const float *params, const float *x, float *y, float *log_det,
@@ -1016,28 +1061,45 @@ int launch_flow_pl(const mnf_flow_op *ops, int n_ops, const float *params, const
     MNF_REQUIRE(((uintptr_t)x % 8) == 0 && (!y || ((uintptr_t)y % 8) == 0) && (!inter || ((uintptr_t)inter % 8) == 0), MNF_E_ALIGN,
                 "x, y and intermediates must be 8-byte aligned");
     MNF_REQUIRE(n_rows > 0, MNF_E_ARG, "bad row count");
-    if (!(dir_flags & 4)) {
-        const int rc = flow_pl_build(ops, n_ops, params, dim, workspace, stream);
-        if (rc) return rc;
-    }
     Params p{};
-    p.prog.n_ops = n_ops;
-    for (int k = 0; k < n_ops; ++k) p.prog.ops[k] = ops[k];
-    p.gl = pl.gl;
-    p.params = params, p.x = x, p.image = workspace, p.y = y, p.log_det = log_det, p.base_lp = base_lp, p.inter = inter;
-    p.n_rows = n_rows, p.dir_flags = dir_flags & 3;
+    size_t want = 0;
+    int rc = setup_params(pl, ops, n_ops, params, workspace, n_rows, (dir_flags & 4) != 0, dp, stream, p, want);
+    if (rc) return rc;
+    p.x = x, p.y = y, p.log_det = log_det, p.base_lp = base_lp, p.inter = inter;
+    p.dir_flags = dir_flags & 3;
     if (gather) {
         MNF_REQUIRE(gather->n_peers >= 0 && gather->n_peers <= MNF_MAX_PEERS, MNF_E_ARG, "bad n_peers");
         p.gather = *gather;
     }
-    // shared memory: every table at its largest, capped by what a CTA can have
-    size_t want = (size_t)(pl.image_floats - HDR_FLOATS) * sizeof(float);
-    const size_t cap = (size_t)dp->smem_optin - 4096;  // static shared memory of the kernel: execution list, offsets, barrier
-    if (want > cap) want = cap;
-    want &= ~(size_t)15;
-    p.smem_floats = (int)(want / sizeof(float));
 #define MNF_PL_LAUNCH(KK) \
     if (pl.K == KK) return (dir_flags & 1) ? launch_k<KK, true>(p, dp, want, stream) : launch_k<KK, false>(p, dp, want, stream);
+    MNF_PL_BINS(MNF_PL_LAUNCH)
+#undef MNF_PL_LAUNCH
+    return 1;
+}
+
+// Forward pass of base points drawn in the kernel (flow_pl_kernel<K, false, true>): x [n_rows, 2], log q(x) and the drawn
+// z, each optional.  Returns 1 if the program is not eligible or no workspace was given (the caller takes the
+// draw-then-forward path).  staged: `workspace` already holds the image of flow_pl_build for these parameters.
+int launch_flow_pl_sample(const mnf_flow_op *ops, int n_ops, const float *params, uint64_t seed, uint32_t noise_stream,
+                          uint64_t row_offset, float *x, float *log_prob, float *z, int64_t n_rows, int dim, bool staged,
+                          float *workspace, cudaStream_t stream) {
+    using namespace fpl;
+    const Plan pl = make_plan(ops, n_ops, dim);
+    if (!pl.ok || !workspace) return 1;
+    const DeviceProps *dp = device_props();
+    MNF_REQUIRE(dp != nullptr, MNF_E_DEVICE, "no CUDA device");
+    MNF_REQUIRE(((uintptr_t)workspace % 16) == 0, MNF_E_ALIGN, "workspace must be 16-byte aligned");
+    MNF_REQUIRE((!x || ((uintptr_t)x % 8) == 0) && (!z || ((uintptr_t)z % 8) == 0), MNF_E_ALIGN, "x and z must be 8-byte aligned");
+    MNF_REQUIRE(n_rows > 0, MNF_E_ARG, "bad row count");
+    Params p{};
+    size_t want = 0;
+    int rc = setup_params(pl, ops, n_ops, params, workspace, n_rows, staged, dp, stream, p, want);
+    if (rc) return rc;
+    p.y = x, p.base_lp = log_prob, p.z = z;
+    p.seed = seed, p.row_offset = row_offset, p.noise_stream = noise_stream;
+#define MNF_PL_LAUNCH(KK) \
+    if (pl.K == KK) return launch_k<KK, false, true>(p, dp, want, stream);
     MNF_PL_BINS(MNF_PL_LAUNCH)
 #undef MNF_PL_LAUNCH
     return 1;

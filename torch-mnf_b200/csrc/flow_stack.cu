@@ -5,6 +5,7 @@
 #include <new>
 
 #include "common.cuh"
+#include "mnf_common.cuh"
 
 namespace mnf {
 int validate_program(const mnf_flow_op *ops, int n_ops, int dim, int64_t n_params);
@@ -22,6 +23,43 @@ int flow_stage_image(const mnf_flow_op *ops, int n_ops, const float *params, int
 int launch_made_fast(const mnf_flow_op *ops, int n_ops, const float *params, const float *x, float *y, float *log_det,
                      float *base_lp, float *inter, int64_t n_rows, int dim, int dir_flags, float *scratch,
                      cudaStream_t stream, bool plan_only);
+int launch_flow_pl_sample(const mnf_flow_op *ops, int n_ops, const float *params, uint64_t seed, uint32_t noise_stream,
+                          uint64_t row_offset, float *x, float *log_prob, float *z, int64_t n_rows, int dim, bool staged,
+                          float *workspace, cudaStream_t stream);
+
+// ---- base draws of mnf_flow_stack_sample for the programs the table kernel does not run ----
+// One thread per row: z[r, c] = philox_normal(element (row_offset + r) dim + c).  finish = 0 stores z; finish = 1 draws the
+// same numbers again and turns the log-det the forward pass left in log_prob into log N(z) - log_det (re-drawing costs
+// a few hundred instructions per row and needs no [n_rows] buffer between the launches, while the forward pass may have
+// overwritten z with x in place).
+__global__ void flow_base_draw_kernel(uint64_t seed, uint32_t noise_stream, uint64_t row_offset, float *__restrict__ z,
+                                      float *__restrict__ log_prob, long long n_rows, int dim, int finish) {
+    const Philox g(seed);
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long r = (long long)blockIdx.x * blockDim.x + threadIdx.x; r < n_rows; r += stride) {
+        const uint64_t e0 = (row_offset + (uint64_t)r) * (uint64_t)dim;
+        float sq = 0.f;
+        for (int c = 0; c < dim; ++c) {
+            const float v = philox_normal(g, e0 + c, noise_stream);
+            if (finish) sq = fmaf(v, v, sq);
+            else z[r * dim + c] = v;
+        }
+        if (finish) log_prob[r] = fmaf(-0.5f, sq, -0.9189385332046727f * (float)dim) - log_prob[r];  // log N(z) - log_det
+    }
+}
+
+static int launch_base_draw(uint64_t seed, uint32_t noise_stream, uint64_t row_offset, float *z, float *log_prob,
+                            int64_t n_rows, int dim, int finish, cudaStream_t stream) {
+    const DeviceProps *dp = device_props();
+    MNF_REQUIRE(dp != nullptr, MNF_E_DEVICE, "no CUDA device");
+    const int threads = 256;
+    long long blocks = (n_rows + threads - 1) / threads;
+    const long long cap = (long long)dp->sm_count * 8;
+    if (blocks > cap) blocks = cap;
+    flow_base_draw_kernel<<<(unsigned)blocks, threads, 0, stream>>>(seed, noise_stream, row_offset, z, log_prob, n_rows, dim,
+                                                                    finish);
+    return launch_status("flow_base_draw_kernel");
+}
 
 // ---- Glow: W = P (tril(L,-1)+I) (triu(U,1)+diag S), W^-1 = Um^-1 Lm^-1 P^T (glow.py:20-24,35) ----
 // one thread per column; fp64 internally, rounded once to fp32.
@@ -145,6 +183,51 @@ int mnf_flow_stack_run(const mnf_flow_op *ops_host, int n_ops, const float *para
                 "peer-memory gather output needs the piecewise-linear or the tensor-core dim-2 kernel (AffineHalfFlow / NSF_CL stack in log-prob mode, with a workspace)");
     return launch_flow_generic(ops_host, n_ops, params, n_params, x, y, log_det, base_log_prob, intermediates,
                                n_rows, dim, inverse & 3, st);
+}
+
+int mnf_flow_stack_sample(const mnf_flow_op *ops_host, int n_ops, const float *params, int64_t n_params, uint64_t seed,
+                          uint32_t noise_stream, uint64_t row_offset, float *x, float *log_prob, float *z, int64_t n_rows,
+                          int dim, int flags, float *workspace, void *stream) {
+    int rc = validate_program(ops_host, n_ops, dim, n_params);
+    if (rc) return rc;
+    MNF_REQUIRE(n_rows >= 0, MNF_E_ARG, "n_rows=%lld is negative", (long long)n_rows);
+    MNF_REQUIRE((flags & ~(MNF_RUN_GENERIC | MNF_RUN_STAGED | MNF_RUN_VARIANT_MASK)) == 0, MNF_E_ARG,
+                "flags=0x%x: sampling takes MNF_RUN_GENERIC, MNF_RUN_STAGED and MNF_RUN_VARIANT(v) only", flags);
+    if (n_rows == 0) return 0;
+    MNF_REQUIRE(x || log_prob || z, MNF_E_ARG, "no output requested");
+    MNF_REQUIRE(params || n_params == 0, MNF_E_ARG, "params is NULL");
+    cudaStream_t st = (cudaStream_t)stream;
+    const bool staged = (flags & MNF_RUN_STAGED) && workspace && dim == 2;
+    const int variant = ((flags & MNF_RUN_VARIANT_MASK) >> 4) - 1;
+    // whole call in the table kernel: the draw, the stack and log N(z) - log_det in one pass
+    if (!(flags & MNF_RUN_GENERIC) && (variant < 0 || variant == 6 || staged) && n_ops > 0 && (x || log_prob)) {
+        rc = launch_flow_pl_sample(ops_host, n_ops, params, seed, noise_stream, row_offset, x, log_prob, z, n_rows, dim, staged,
+                                   workspace, st);
+        if (rc != 1) return rc;
+    }
+    // otherwise: draw z (into x when the caller does not want z, the forward pass then runs in place), run the forward
+    // dispatch of mnf_flow_stack_run with its log-det in log_prob, and finish log_prob with the re-drawn log N(z)
+    float *zb = z ? z : x;
+    MNF_REQUIRE(zb != nullptr, MNF_E_ARG,
+                "this program is not run by the table kernel (or no workspace was given): pass x or z to hold the drawn points");
+    rc = launch_base_draw(seed, noise_stream, row_offset, zb, nullptr, n_rows, dim, 0, st);
+    if (rc || !(x || log_prob)) return rc;
+    if (n_ops == 0) {
+        if (x && x != zb) MNF_CUDA(cudaMemcpyAsync(x, zb, sizeof(float) * n_rows * dim, cudaMemcpyDeviceToDevice, st));
+        if (log_prob) MNF_CUDA(cudaMemsetAsync(log_prob, 0, sizeof(float) * n_rows, st));
+    } else {
+        const int dir = staged ? 4 : 0;  // forward; a staged image is passed on as such
+        rc = 1;
+        if (!(flags & MNF_RUN_GENERIC))
+            rc = launch_made_fast(ops_host, n_ops, params, zb, x, log_prob, nullptr, nullptr, n_rows, dim, dir, workspace, st, false);
+        if (rc == 1 && !(flags & MNF_RUN_GENERIC))
+            rc = launch_flow_fast(ops_host, n_ops, params, n_params, zb, x, log_prob, nullptr, nullptr, n_rows, dim, dir, variant,
+                                  workspace, nullptr, st, false);
+        if (rc == 1)
+            rc = launch_flow_generic(ops_host, n_ops, params, n_params, zb, x, log_prob, nullptr, nullptr, n_rows, dim, 0, st);
+        if (rc) return rc;
+    }
+    return log_prob ? launch_base_draw(seed, noise_stream, row_offset, nullptr, log_prob, n_rows, dim, 1, st) : 0;
 }
 
 struct mnf_flow_handle {

@@ -70,6 +70,11 @@ _SIGS = {
         [C.POINTER(FlowOp), C.c_int, _f32p, C.c_int64, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p,
          C.c_int64, C.c_int, C.c_int, C.c_void_p],
     ),
+    "mnf_flow_stack_sample": (
+        C.c_int,
+        [C.POINTER(FlowOp), C.c_int, _f32p, C.c_int64, C.c_uint64, C.c_uint32, C.c_uint64, _f32p, _f32p, _f32p,
+         C.c_int64, C.c_int, C.c_int, _f32p, C.c_void_p],
+    ),
     "mnf_flow_stack_stage_size": (C.c_int64, [C.POINTER(FlowOp), C.c_int, C.c_int, C.c_int64]),
     "mnf_flow_stack_stage_max_rows": (C.c_int64, [C.POINTER(FlowOp), C.c_int, C.c_int, C.c_int64]),
     "mnf_flow_stack_stage": (C.c_int, [C.POINTER(FlowOp), C.c_int, _f32p, C.c_int64, C.c_int, _f32p, C.c_void_p]),

@@ -342,6 +342,38 @@ class FlowProgram:
         return _FlowStackFn.apply(self, inverse, x, blob)
 
     @torch.no_grad()
+    def sample(self, n_rows: int, dim: int, device, seed: int, row_offset: int = 0, want_x: bool = True,
+               want_log_prob: bool = True, want_z: bool = False, kernel=None):
+        """(x, log_prob, z) of ``n_rows`` standard-normal base draws pushed through the flows (mnf_flow_stack_sample):
+        z of global row row_offset + r from Philox(seed, stream 0), x its forward pass, log_prob = log N(z) - log_det.
+        Outputs not asked for are None.  kernel as for ``run``.  Single-chunk programs only."""
+        self._build(device)
+        if not 0 < self._n_ops <= _lib.MAX_OPS:
+            raise NotImplementedError(f"sampling through {self._n_ops} flows: between 1 and {_lib.MAX_OPS} supported")
+        lib = _lib.lib()
+        dev = self._blob.device
+        x = torch.empty(n_rows, dim, device=dev, dtype=torch.float32) if want_x else None
+        lp = torch.empty(n_rows, device=dev, dtype=torch.float32) if want_log_prob else None
+        z = torch.empty(n_rows, dim, device=dev, dtype=torch.float32) if want_z else None
+        flags = 0
+        if kernel == "generic":
+            flags |= _lib.RUN_GENERIC
+        elif kernel is not None:
+            flags |= ((int(kernel) + 1) << 4) & 0x70
+        ws = self._staged_image(lib, n_rows, dim, kernel)
+        if ws is not None:
+            flags |= _lib.RUN_STAGED
+        else:
+            ws = self._workspace(lib, self._n_ops, n_rows, dim, dev, have_y=want_x, kernel=kernel)
+        with _lib.on_device(dev):
+            rc = lib.mnf_flow_stack_sample(self._ops, self._n_ops, self._blob.data_ptr(), self._blob.numel(),
+                                           int(seed) & (2**64 - 1), 0, int(row_offset), _lib.ptr(x), _lib.ptr(lp),
+                                           _lib.ptr(z), n_rows, dim, flags, _lib.ptr(ws), _lib.stream_ptr(dev))
+        _lib.check(rc, "mnf_flow_stack_sample")
+        _lib.launch_count += 1
+        return x, lp, z
+
+    @torch.no_grad()
     def run(self, x, inverse: bool, want_inter: bool = False, want_base_lp: bool = False, out=None,
             log_det=None, kernel=None, log_prob_only=False, log_prob_out=None, gather=None):
         """kernel: None = library default, "generic" = interpreter, 0/1/2 = dim-2 kernel variant.

@@ -219,9 +219,73 @@ class NormalizingFlowModel(NormalizingFlow):
             raise RuntimeError("run the data-dependent initialisation (one forward / inverse call) before binding the model")
         return BoundLogProb(self._program(), p.device, dim, max_rows)
 
-    def sample(self, *num_samples: int) -> Tensor:
+    def sample_and_log_prob(self, *num_samples: int, seed: int | None = None, row_offset: int = 0) -> tuple[Tensor, Tensor]:
+        """``(x [*n, dim], log_prob [*n])``: draws from the model together with their log-density log q(x) =
+        log N(z) - log_det(forward), without the inverse pass ``log_prob(x)`` would take.  Additive API.
+
+        With a standard-normal base, z of global row ``row_offset + r`` comes from Philox4x32-10 keyed by ``seed``
+        (``seed=None``: a seed drawn from torch's generator, so ``torch.manual_seed`` fixes it), the same numbers as
+        every Philox draw of the library for those indices; dim-2 stacks of the table kernel draw, transform and score
+        in one launch.  A batch sharded over ranks reproduces the single call bit for bit when every rank passes the
+        same seed and its slice as offset::
+
+            lo, hi = torch_mnf.distributed.shard_range(n, world, rank)
+            x, lp = model.sample_and_log_prob(hi - lo, seed=seed, row_offset=lo)
+
+        With grad enabled and trainable parameters, x and log_prob carry reparameterisation gradients (the same z, no
+        gradient of its own; backward through mnf_flow_stack_backward), e.g. for reverse-KL fitting.  Under CUDA-graph
+        capture with ``seed=None`` z is drawn by torch's graph-safe generator, so that every replay draws anew.  Any
+        other base is sampled by torch.distributions (``seed`` is then a ValueError)."""
+        return self._sample(num_samples, seed, row_offset, want_log_prob=True)
+
+    def _sample(self, num_samples, seed, row_offset, want_log_prob):
+        n = tuple(num_samples[0]) if len(num_samples) == 1 and not isinstance(num_samples[0], int) else tuple(num_samples)
+        rows = math.prod(n)
+        dim = int(self.base.event_shape[0]) if len(self.base.event_shape) == 1 else None
+        p = next(self.parameters(), None)
+        std = p is not None and p.is_cuda and dim is not None and self._base_is_std(dim)
+        if any(getattr(f, "data_dep_init_done", True) is False for f in self.flows):
+            raise RuntimeError("run the data-dependent initialisation (one forward / inverse call) before binding the model")
+        if not std:
+            if seed is not None:
+                raise ValueError("seed= draws a standard-normal base with Philox; this model's base is sampled by "
+                                 "torch.distributions")
+            z = self.base.sample(n)
+            if p is not None and z.device != p.device:
+                z = z.to(p.device)
+            z = z.float().reshape(-1, z.size(-1))
+            xs, ld = self.forward(z)
+            loc = getattr(self.base, "loc", None)
+            lp = self.base.log_prob(z if loc is None or loc.device == z.device else z.to(loc.device)).to(z.device) - ld
+            return xs[-1].reshape(*n, -1), lp.reshape(n)
+        if not 0 < len(self.flows) <= _lib.MAX_OPS:
+            raise NotImplementedError(f"sampling through {len(self.flows)} flows: between 1 and {_lib.MAX_OPS} supported")
+        prog = self._program()
+        capturing = seed is None and torch.cuda.is_current_stream_capturing()
+        if seed is None and not capturing:
+            seed = int(torch.randint(0, 2**62, (1,)).item())  # follows torch.manual_seed, as _mnf_ops.Noise
+        grad = prog.needs_grad(p.detach())
+        if capturing or grad:
+            if capturing:  # a seed passed by value would be frozen into the graph: torch's generator advances per replay
+                z = torch.randn(rows, dim, device=p.device, dtype=torch.float32)
+            else:
+                _, _, z = prog.sample(rows, dim, p.device, seed, row_offset, want_x=False, want_log_prob=False, want_z=True)
+            if grad:  # reparameterisation gradients through mnf_flow_stack_backward
+                ld, inter = prog.run_autograd(z, inverse=False)
+                x = inter[-1]
+            else:
+                x, ld, _, _ = prog.run(z, inverse=False)
+            lp = -0.5 * z.square().sum(1) - 0.5 * dim * math.log(2 * math.pi) - ld
+        else:
+            x, lp, _ = prog.sample(rows, dim, p.device, seed, row_offset, want_log_prob=want_log_prob)
+        return x.reshape(*n, dim), (lp.reshape(n) if lp is not None else None)
+
+    def sample(self, *num_samples: int, seed: int | None = None) -> Tensor:
         """core.py:51-55.  A standard-normal base is drawn directly on the flows' device (no host round trip);
-        any other base is sampled by torch.distributions and moved over."""
+        any other base is sampled by torch.distributions and moved over.  ``seed`` (additive): the Philox draw of
+        ``sample_and_log_prob(..., seed=seed)``, whose x this returns (without computing log-densities)."""
+        if seed is not None:
+            return self._sample(num_samples, seed, 0, want_log_prob=False)[0]
         p = next(self.parameters(), None)
         n = tuple(num_samples[0]) if len(num_samples) == 1 and not isinstance(num_samples[0], int) else num_samples
         dim = int(self.base.event_shape[0]) if len(self.base.event_shape) == 1 else None
