@@ -113,8 +113,8 @@ typedef struct mnf_flow_op {
  * log-probability straight into the gather buffers of the other ranks (peer-mapped device pointers, e.g. from
  * torch.distributed._symmetric_memory) at element row_offset + i -- or, when multicast_ptr is set, with ONE
  * multimem.st per element that the switch replicates to every rank.  The data transfer overlaps the kernel's
- * arithmetic; the only collective left after the launch is a barrier.  Supported by the piecewise-linear and the
- * tensor-core dim-2 kernels in MNF_RUN_LOGPROB mode. */
+ * arithmetic; the only collective left after the launch is a barrier.  Supported by the piecewise-linear dim-2 kernel
+ * in MNF_RUN_LOGPROB mode. */
 #define MNF_MAX_PEERS 8
 typedef struct mnf_gather_out {
     int32_t n_peers;                 /* entries of peer_ptrs in use (0 with multicast)       */
@@ -132,12 +132,12 @@ int mnf_flow_stack_run(const mnf_flow_op *ops_host, int n_ops, const float *para
 
 /* A flow program bound once, for call sites that evaluate the same model over and over (BASELINE config 1: 4096
  * points per call, where a call is latency-bound): the handle keeps a host copy of the descriptors and the device
- * pointers of the packed parameters and of the pre-staged net image, so that a log-probability call is five arguments
- * and no validation.  The caller owns every device buffer and must keep them alive and UNCHANGED while the handle is in
- * use (re-create it after a parameter update); the handle itself is a small host allocation freed by
+ * pointers of the packed parameters and of the staged conditioner tables, so that a log-probability call is five
+ * arguments and no validation.  The caller owns every device buffer and must keep them alive and UNCHANGED while the
+ * handle is in use (re-create it after a parameter update); the handle itself is a small host allocation freed by
  * mnf_flow_handle_destroy.  staged: mnf_flow_stack_stage output for these parameters or NULL; workspace:
- * mnf_flow_stack_workspace(n_ops, max_rows, dim) floats or NULL if that is 0 (with `staged`, programs of the
- * piecewise-linear kernel need none at any batch size, others none below 65536 rows).
+ * mnf_flow_stack_workspace(n_ops, max_rows, dim) floats or NULL if that is 0 (with `staged`, none is needed at any
+ * batch size).
  *   mnf_flow_handle_log_prob: log_prob[r] = log|det J|(x_r) + standard-normal log-density of the result, i.e.
  *   NormalizingFlowModel.log_prob (flows/core.py:46-49 over :27-35) for an N(0, I) base, one fused pass. */
 typedef struct mnf_flow_handle mnf_flow_handle;
@@ -166,10 +166,9 @@ int mnf_flow_stack_backward(const mnf_flow_op *ops_host, int n_ops, const float 
                             float *grad_x, int64_t n_rows, int dim, int flags, void *stream);
 
 /* Floats of scratch `workspace` must provide for a run of this shape (0 = none needed; NULL is then
- * accepted).  dim 2: room for the conditioner tables of the piecewise-linear kernel (built per call when no staged image
- * is passed) or the weight image of the tensor-core kernel, whichever is larger (the library keeps no device state of
- * its own: per-call staging lives here; without a workspace a dim-2 run takes the shared-memory kernels, which need
- * none); dim 64: a log-prob-only MADE run parks the points between flows. */
+ * accepted).  dim 2: room for the conditioner tables of the piecewise-linear kernel, built per call when no staged image
+ * is passed (the library keeps no device state of its own: per-call staging lives here; without a workspace a dim-2 run
+ * takes the shared-memory kernels, which need none); dim 64: a log-prob-only MADE run parks the points between flows. */
 int64_t mnf_flow_stack_workspace(int n_ops, int64_t n_rows, int dim);
 
 #define MNF_RUN_INVERSE 1
@@ -181,10 +180,10 @@ int64_t mnf_flow_stack_workspace(int n_ops, int64_t n_rows, int dim);
 /* v: 6 = every conditioner as a piecewise-linear table of its scalar input (csrc/flow_pl.cu) -- the library default for
  *        dim-2 stacks of AffineConstantFlow / ActNormFlow / Glow / AffineHalfFlow / NSF_CL(K in {4, 5, 6, 8, 10, 12, 16}) whose conditioners
  *        have 1..5 hidden layers of width <= 64, any batch size;
- *    0, 1, 2 = shared-memory weight variants of the register-resident dim-2 kernel (2 = default of the remaining shapes of
- *        its (hidden, bins) grid, and of calls without a workspace);
- *    4 = conditioner MLPs on the tensor cores (NSF_CL(K=8, n_h=16) stacks);
- *    5 = eight lanes per point (AffineHalfFlow stacks up to 32768 rows); 3 (round 1's constant-bank variant, removed) runs 2.
+ *    2 = register-resident dim-2 kernel with the nets in shared memory (default of the remaining shapes of its
+ *        (hidden, bins) grid, and of calls without a workspace);
+ *    5 = eight lanes per point (AffineHalfFlow stacks up to 32768 rows).
+ *    0, 1 and 3 (removed shared-memory variants) run 2; 4 (the removed tensor-core kernel) runs the library default.
  *    A variant the program is not eligible for falls back to the library default. */
 
 /* Draws n_rows points of the flow model (standard-normal base, flows in module order) together with their log-density:
@@ -207,21 +206,18 @@ int mnf_flow_stack_sample(const mnf_flow_op *ops_host, int n_ops, const float *p
 
 /* Per-parameter-version preparation of a dim-2 stack, done ONCE instead of in every call (call it again whenever a
  * parameter changes): mnf_flow_stack_stage writes into a caller-owned, 16-byte aligned buffer of
- * mnf_flow_stack_stage_size() floats (0 = the program has no such form)
- *   - the conditioner TABLES of the piecewise-linear kernel (sorted breakpoints and per-piece slopes / values of every
- *     conditioner, found in fp64) for the programs that kernel runs -- any batch size; a run with MNF_RUN_STAGED and that
- *     buffer as `workspace` is then ONE launch, always of that kernel (a variant request is ignored);
- *   - otherwise the shared-memory layout of the nets for the register-resident kernel (variant 2), for runs of fewer
- *     than 65 536 rows: the kernel then starts with a plain vector copy. */
+ * mnf_flow_stack_stage_size() floats (0 = the program has no such form) the conditioner TABLES of the piecewise-linear
+ * kernel (sorted breakpoints and per-piece slopes / values of every conditioner, found in fp64), for the programs that
+ * kernel runs.  A run with MNF_RUN_STAGED and that buffer as `workspace` is then ONE launch of that kernel at any batch
+ * size (a variant request is ignored). */
 int64_t mnf_flow_stack_stage_size(const mnf_flow_op *ops_host, int n_ops, int dim, int64_t n_params);
-/* Largest batch a MNF_RUN_STAGED run of this program accepts: INT64_MAX when the staged image holds the conditioner
- * tables (any batch), 65535 when it is the shared-memory layout of the register-resident kernel, 0 without a staged form. */
+/* Largest batch a MNF_RUN_STAGED run of this program accepts: INT64_MAX when it has a staged form, else 0. */
 int64_t mnf_flow_stack_stage_max_rows(const mnf_flow_op *ops_host, int n_ops, int dim, int64_t n_params);
 int mnf_flow_stack_stage(const mnf_flow_op *ops_host, int n_ops, const float *params, int64_t n_params, int dim,
                          float *staged, void *stream);
 
 /* Which kernel mnf_flow_stack_run would pick: 0 = generic interpreter, 1 = specialised
- * D=2 kernels (tensor cores / register-resident / lane-split by shape and batch), 2 = the exact-fp32 MADE kernels
+ * D=2 kernels (table / register-resident / lane-split by shape and batch), 2 = the exact-fp32 MADE kernels
  * (all-MAF/IAF stacks of an instantiated (dim, hidden) shape with three hidden layers).  Host-only, no launch. */
 int mnf_flow_stack_plan(const mnf_flow_op *ops_host, int n_ops, int dim, int64_t n_params);
 

@@ -89,7 +89,7 @@ def test_stack_vs_golden(name, kernel):
 
 
 @pytest.mark.parametrize("name", ["rnvp9_moons", "nsfcl3_stack"])
-@pytest.mark.parametrize("variant", [0, 1, 2, 5, 6])
+@pytest.mark.parametrize("variant", [0, 1, 2, 3, 4, 5, 6])
 def test_dim2_kernel_variants(name, variant):
     g = load_golden(name)
     sd, specs = golden_sd(g), golden_spec(g)
@@ -360,7 +360,7 @@ def test_conditioner_free_stack_streaming_kernel():
 @pytest.mark.parametrize("name,n_rows", [("cfg1_shape", 4096), ("cfg2_shape", 777), ("cfg2_shape", 70001), ("nsf_wide_d6", 501)])
 def test_bound_log_prob_equals_module_call(name, n_rows):
     """NormalizingFlowModel.log_prob_fn (mnf_flow_handle_*: the program bound once) returns exactly what log_prob
-    returns, for the staged small-batch kernel, the large-batch kernel and the interpreter."""
+    returns, for the table kernel on staged tables at small and large batches, and for the interpreter."""
     specs = ORACLE_CASES[name]
     model = load_flow_model(specs, random_flow_sd(specs, seed=2, scale=0.4), return_intermediates=False)
     dim = specs[0]["dim"]
@@ -378,7 +378,7 @@ def test_bound_log_prob_equals_module_call(name, n_rows):
 
 def test_two_programs_on_two_streams_do_not_share_state():
     """SURVEY 8b: entry points are re-entrant, the library keeps no device state.  Two different models of the benchmark
-    shape, launched interleaved on two streams (tensor-core kernel: >= 65536 rows, and the small-batch kernels), must give
+    shape, launched interleaved on two streams (the table kernel on each model's staged tables, at a large and a small batch), must give
     bit-identical results to running them one after the other."""
     specs = ORACLE_CASES["cfg2_shape"]
     models = [load_flow_model(specs, random_flow_sd(specs, seed=s, scale=0.5), return_intermediates=False) for s in (1, 2)]

@@ -9,7 +9,7 @@ from tests.helpers import load_flow_model, random_flow_sd
 from tests.test_flows_gpu import ORACLE_CASES
 
 name = os.environ.get("CASE", "cfg2_shape")
-variant = os.environ.get("VARIANT", "3")
+variant = os.environ.get("VARIANT", "6")
 variant = variant if variant == "generic" else int(variant)
 n = int(os.environ.get("N", 1 << 24))
 specs = ORACLE_CASES[name]

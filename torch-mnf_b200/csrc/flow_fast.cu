@@ -8,21 +8,13 @@ namespace mnf {
 // (hidden width, spline bins) instantiations, one translation unit each (flow_fast_h*k*.cu): the BASELINE shapes
 // (16, 8), (24, 8) and the reference's defaults (8, 5), plus neighbours so that common variations stay off the interpreter
 #define MNF_FLOW_FAST_SHAPES(X) X(16, 8) X(24, 8) X(8, 5) X(8, 8) X(16, 5) X(32, 8)
-#define MNF_DECLARE_SHAPE(HH, KK)                \
-    int launch_fast_##HH##_##KK(MNF_FLOW_FAST_ARGS); \
-    int stage_image_##HH##_##KK(const FlowProgram &, const FastLayout &, const float *, float *, cudaStream_t);
+#define MNF_DECLARE_SHAPE(HH, KK) int launch_fast_##HH##_##KK(MNF_FLOW_FAST_ARGS);
 MNF_FLOW_FAST_SHAPES(MNF_DECLARE_SHAPE)
 #undef MNF_DECLARE_SHAPE
-
-int launch_flow_tc(const mnf_flow_op *ops, int n_ops, const float *params, const float *x, float *y, float *log_det,
-                   float *base_lp, float *inter, int64_t n_rows, int dim, int dir_flags, float *workspace,
-                   const mnf_gather_out *gather, cudaStream_t stream, bool plan_only);
 
 int launch_flow_pl(const mnf_flow_op *ops, int n_ops, const float *params, const float *x, float *y, float *log_det,
                    float *base_lp, float *inter, int64_t n_rows, int dim, int dir_flags, float *workspace,
                    const mnf_gather_out *gather, cudaStream_t stream, bool plan_only);
-int64_t flow_pl_image_floats(const mnf_flow_op *ops, int n_ops, int dim);
-int flow_pl_build(const mnf_flow_op *ops, int n_ops, const float *params, int dim, float *image, cudaStream_t stream);
 
 int launch_flow_lanes(const mnf_flow_op *ops, int n_ops, const float *params, const float *x, float *y, float *log_det,
                       float *base_lp, float *inter, int64_t n_rows, int dim, int dir_flags, cudaStream_t stream, bool plan_only,
@@ -36,7 +28,7 @@ struct FastPlan {
     FastLayout lay;
 };
 
-static FastPlan plan_fast(const mnf_flow_op *ops, int n_ops, int dim, int variant) {
+static FastPlan plan_fast(const mnf_flow_op *ops, int n_ops, int dim) {
     FastPlan p;
     if (dim != 2 || n_ops < 1) return p;
     int H = 0, K = 0, slots = 0;
@@ -59,7 +51,7 @@ static FastPlan plan_fast(const mnf_flow_op *ops, int n_ops, int dim, int varian
             n_out = 3 * K - 1;
         }
         if (op.sizes[4] != n_out) return p;
-        const int per_net = fast_net_slots(h, n_out, variant);
+        const int per_net = fast_net_slots(h, n_out);
         for (int which = 0; which < 2; ++which) {
             p.lay.net_slot[k][which] = slots;
             slots += per_net;
@@ -83,11 +75,6 @@ static FastPlan plan_fast(const mnf_flow_op *ops, int n_ops, int dim, int varian
     p.ok = true;
     return p;
 }
-
-// rows from which the large-batch kernel (tensor-core conditioners, flow_tc.cu) is considered
-constexpr long long kCbankMinRows = 1 << 16;
-constexpr int kNumVariants = 3;  // 0, 1, 2 (variant 3, round 1's constant-bank kernel, was removed: a request for it runs 2)
-constexpr bool kTcDefault = true;  // measured (profiles/r02_flow_tc.md): 3.85 vs 4.12 ms per 2^24 points at unchanged parity, one launch, 12 B/pt of DRAM traffic
 
 // ---------------------------------------------------------------------------------------------------
 // Conditioner-free stacks (AffineConstantFlow / ActNormFlow / Glow only, dim 2): the whole stack is ONE
@@ -173,63 +160,23 @@ static int launch_affine_stream(const FlowProgram &prog, const float *params, co
     return launch_status("affine_stream_kernel");
 }
 
-// Pre-staged shared-memory image of a program's conditioner nets (variant-2 layout): floats needed, 0 if the program
-// has no such form.  Small-batch calls spend most of their kernel time re-laying the nets out in every CTA; with the
-// image (built once per parameter change) the prologue is a plain vector copy.
-int64_t flow_stage_size(const mnf_flow_op *ops, int n_ops, int dim) {
-    // programs with a piecewise-linear form (flow_pl.cu) stage their conditioner TABLES; the image below is for the rest
-    if (const int64_t pl = flow_pl_image_floats(ops, n_ops, dim)) return pl;
-    FastPlan p = plan_fast(ops, n_ops, dim, 2);
-    bool has_net = false;
-    for (int k = 0; k < n_ops; ++k) has_net |= ops[k].type == MNF_OP_NSF_CL || ops[k].type == MNF_OP_AFFINE_HALF;
-    if (!p.ok || !has_net || (size_t)p.lay.total_slots * sizeof(float) > 227 * 1024) return 0;
-    return p.lay.total_slots;
-}
-
-int flow_stage_image(const mnf_flow_op *ops, int n_ops, const float *params, int dim, float *image, cudaStream_t stream) {
-    if (flow_pl_image_floats(ops, n_ops, dim) > 0) return flow_pl_build(ops, n_ops, params, dim, image, stream);
-    FastPlan p = plan_fast(ops, n_ops, dim, 2);
-    MNF_REQUIRE(p.ok && flow_stage_size(ops, n_ops, dim) > 0, MNF_E_SHAPE, "program has no staged form");
-    MNF_REQUIRE(params && image && ((uintptr_t)image % 16) == 0, MNF_E_ARG, "NULL or misaligned pointer");
-    FlowProgram prog;
-    prog.n_ops = n_ops;
-    for (int k = 0; k < n_ops; ++k) prog.ops[k] = ops[k];
-#define MNF_STAGE_SHAPE(HH, KK) \
-    if (p.H == HH && p.K == KK) return stage_image_##HH##_##KK(prog, p.lay, params, image, stream);
-    MNF_FLOW_FAST_SHAPES(MNF_STAGE_SHAPE)
-#undef MNF_STAGE_SHAPE
-    return fail(MNF_E_SHAPE, "no instantiation for hidden width %d, %d bins", p.H, p.K);
-}
-
 // returns 1 if the program is not eligible (caller falls back to the generic kernel)
 int launch_flow_fast(const mnf_flow_op *ops, int n_ops, const float *params, int64_t n_params, const float *x,
                      float *y, float *log_det, float *base_lp, float *inter, int64_t n_rows, int dim, int inverse,
                      int variant, float *workspace, const mnf_gather_out *gather, cudaStream_t stream,
                      bool plan_only) {
-    bool has_spline = false, has_net = false;
-    for (int k = 0; k < n_ops; ++k) {
-        has_spline |= ops[k].type == MNF_OP_NSF_CL;
-        has_net |= ops[k].type == MNF_OP_NSF_CL || ops[k].type == MNF_OP_AFFINE_HALF;
-    }
+    bool has_net = false;
+    for (int k = 0; k < n_ops; ++k) has_net |= ops[k].type == MNF_OP_NSF_CL || ops[k].type == MNF_OP_AFFINE_HALF;
     const bool want_gather = gather && (gather->n_peers > 0 || gather->multicast_ptr);
     // variant 6 (default wherever it applies): every conditioner as a piecewise-linear table of its scalar input
     // (flow_pl.cu), one launch for the whole stack after the table builder; any hidden widths up to 64, K in {4, 5, 6, 8, 10, 12, 16}.
-    // A staged image (bit 2) of such a program IS its tables, so a staged call always lands here.
+    // A staged image (bit 2) holds such tables (mnf_flow_stack_stage stages nothing else), so a staged call always lands here.
     if ((variant == 6 || variant < 0 || (inverse & 4)) && (!want_gather || (inverse & 2)) && (workspace || plan_only)) {
         const int rc = launch_flow_pl(ops, n_ops, params, x, y, log_det, base_lp, inter, n_rows, dim, inverse & 7, workspace, gather,
                                       stream, plan_only);
         if (rc != 1) return rc;
     }
     if (variant == 6) variant = -1;
-    // variant 4: conditioners on the tensor cores (flow_tc.cu), one launch for the whole stack, weights in the caller's
-    // workspace.  Spline stacks of its shape class take it by default from kCbankMinRows rows up.
-    if (!(inverse & 4) && (variant == 4 || (variant < 0 && kTcDefault && has_spline && (plan_only || n_rows >= kCbankMinRows))) &&
-        (!want_gather || (inverse & 2))) {
-        const int rc = launch_flow_tc(ops, n_ops, params, x, y, log_det, base_lp, inter, n_rows, dim, inverse & 3, workspace,
-                                      gather, stream, plan_only);
-        if (rc != 1) return rc;
-    }
-    if (variant == 4) variant = -1;  // not of the tensor-core kernel's shape class: library default
     // variant 5: eight lanes per point (flow_lanes.cu) -- small batches of AffineHalfFlow stacks, where a call is bound by
     // the latency of one point's chain.  Default for its class up to 2048 rows (a staged image, bit 2, is simply not needed by it).
     if (!want_gather && (variant == 5 || (variant < 0 && !plan_only))) {
@@ -238,11 +185,10 @@ int launch_flow_fast(const mnf_flow_op *ops, int n_ops, const float *params, int
         if (rc != 1) return rc;
     }
     if (variant == 5) variant = -1;
-    // every remaining variant keeps its weights in shared memory and needs no workspace; 2 (output-packed FFMA2) is the default
-    int mode = (variant >= 0 && variant < kNumVariants) ? variant : 2;
-    if (want_gather) return 1;  // the fused peer-memory gather lives in the tensor-core kernel only: caller reports the restriction
-    if (mode != 2) inverse &= ~4;  // a staged image (bit 2) is in the variant-2 layout
-    FastPlan p = plan_fast(ops, n_ops, dim, mode);
+    // variant 2, also run for requests of 0, 1 and 3 (variants removed earlier): the shared-memory FFMA2 kernel, which
+    // needs no workspace
+    if (want_gather) return 1;  // the fused peer-memory gather lives in the table kernel only: caller reports the restriction
+    FastPlan p = plan_fast(ops, n_ops, dim);
     if (!p.ok) return 1;
     const DeviceProps *dp = plan_only ? nullptr : device_props();
     const size_t smem_bytes = (size_t)p.lay.total_slots * sizeof(float);
@@ -263,8 +209,8 @@ int launch_flow_fast(const mnf_flow_op *ops, int n_ops, const float *params, int
         return launch_affine_stream(prog, params, x, y, log_det, base_lp, n_rows, inverse, workspace, dp, stream);
 #define MNF_LAUNCH_SHAPE(HH, KK)                                                                                           \
     if (p.H == HH && p.K == KK)                                                                                            \
-        return launch_fast_##HH##_##KK(mode, prog, p.lay, smem_bytes, params, x, y, log_det, base_lp, inter, n_rows, inverse, \
-                                       workspace, gather, dp, stream);
+        return launch_fast_##HH##_##KK(prog, p.lay, smem_bytes, params, x, y, log_det, base_lp, inter, n_rows, inverse, dp, \
+                                       stream);
     MNF_FLOW_FAST_SHAPES(MNF_LAUNCH_SHAPE)
 #undef MNF_LAUNCH_SHAPE
     return 1;

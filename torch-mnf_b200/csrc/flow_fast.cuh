@@ -11,15 +11,8 @@
 // Supported ops (all with dim == 2): AffineConstantFlow/ActNormFlow, Glow, AffineHalfFlow with
 // h_sizes (H,H,H), NSF_CL with n_h = H and K bins.  Anything else -> flow_generic.cu.
 //
-// VARIANT selects how the MLP is mapped onto the packed FMA:
-//   0: point-packed, scalar FFMA (two per weight)           -- reference variant
-//   1: point-packed FFMA2, (w,w) operand built with a MOV per weight
-//   2: output-packed FFMA2: weights stored transposed ([in][out]) so one LDS.128 delivers two
-//      ready (w_j, w_j+1) operands; the activation is duplicated once per input instead
-//   (3: round 1's constant-bank variant -- weights as uniform-register operands, the stack cut into one launch per
-//      conditioner.  Removed in round 2: it kept the nets in __constant__ / __device__ arrays of the library behind a
-//      mutex (global state the ABI excludes), and the tensor-core kernel of flow_tc.cu replaced it as the large-batch
-//      path; a request for variant 3 runs variant 2.)
+// The MLP is mapped onto the packed FMA by output (variant 2 of MNF_RUN_VARIANT): weights stored transposed ([in][out])
+// so one LDS.128 delivers two ready (w_j, w_j+1) operands; the activation is duplicated once per input.
 #pragma once
 #include "flow_math.cuh"
 
@@ -37,7 +30,7 @@ struct FastLayout {
 
 constexpr int round4(int n) { return (n + 3) / 4 * 4; }
 
-// Variant 2 does not evaluate layers 0 and 1 of a conditioner as layers: its input is ONE scalar c, so
+// The kernel does not evaluate layers 0 and 1 of a conditioner as layers: its input is ONE scalar c, so
 // W1 leaky(w0 c + b0) + b1 is a piecewise-linear function of c with the H breakpoints -b0_j / w0_j; on each of the H + 1
 // intervals it is A_i c + B_i.  The staged net holds the sorted breakpoints and the (A_i | B_i) rows: a point finds its
 // interval with H compares and forms the layer-1 pre-activations with H FMAs instead of H + H^2 (RNVP, H = 24: 648 instead
@@ -47,9 +40,8 @@ constexpr int pl_stride(int H) { return 2 * H + 4; }  // padded off the 32-bank 
 constexpr int pl_hidden_slots(int H) { return H + (H + 1) * pl_stride(H) + H * H + H; }
 
 // floats one staged net occupies in shared memory
-constexpr int fast_net_slots(int H, int n_out, int variant) {
-    if (variant >= 2) return pl_hidden_slots(H) + (n_out == 1 ? H + 4 : H * round4(n_out) + round4(n_out));
-    return 2 * H + 2 * (H * H + H) + n_out * H + round4(n_out);
+constexpr int fast_net_slots(int H, int n_out) {
+    return pl_hidden_slots(H) + (n_out == 1 ? H + 4 : H * round4(n_out) + round4(n_out));
 }
 
 __device__ __forceinline__ float2 fma2_packed(float2 a, float2 b, float2 c) {
@@ -68,100 +60,25 @@ __device__ __forceinline__ float2 mul2_packed(float2 a, float2 b) {
     return *reinterpret_cast<float2 *>(&rd);
 }
 
-template <int VARIANT>
-__device__ __forceinline__ float2 fma2(float2 w, float2 x, float2 c) {
-    if constexpr (VARIANT == 0)
-        return make_float2(fmaf(w.x, x.x, c.x), fmaf(w.y, x.y, c.y));
-    else
-        return fma2_packed(w, x, c);
-}
-
 __device__ __forceinline__ float2 leaky2(float2 v) {
     const float2 s = mul2_packed(v, make_float2(0.2f, 0.2f));
     return make_float2(fmaxf(v.x, s.x), fmaxf(v.y, s.y));
 }
 
-__device__ __forceinline__ float4 lds4(const float *base, int i) {  // i: compile-time multiple of 4
-    return reinterpret_cast<const float4 *>(base)[i >> 2];
-}
-
-// weight accessors: offsets are in floats from the start of the staged net
+// weight accessor: offsets are in floats from the start of the staged net
 struct WShared {
     const float *p;
     __device__ __forceinline__ float4 ld4(int i) const { return reinterpret_cast<const float4 *>(p)[i >> 2]; }
     __device__ __forceinline__ float ld1(int i) const { return p[i]; }
 };
-// =====================================================================================
-// point-packed engine (variants 0, 1): float2 = (value for point A, value for point B)
-// smem net layout = blob layout: per Linear weight[out][in], bias[out]
-// =====================================================================================
-template <int H, int VARIANT>
-__device__ __forceinline__ void pp_hidden(const float *W, float2 x, float2 (&h)[H]) {
-    static_assert(H % 4 == 0, "hidden width must be a multiple of 4");
-    float2 g[H];
-#pragma unroll
-    for (int j = 0; j < H; j += 4) {  // layer 0: weight[H][1], bias[H]
-        const float4 w = lds4(W, j), b = lds4(W, H + j);
-        g[j + 0] = leaky2(fma2<VARIANT>(make_float2(w.x, w.x), x, make_float2(b.x, b.x)));
-        g[j + 1] = leaky2(fma2<VARIANT>(make_float2(w.y, w.y), x, make_float2(b.y, b.y)));
-        g[j + 2] = leaky2(fma2<VARIANT>(make_float2(w.z, w.z), x, make_float2(b.z, b.z)));
-        g[j + 3] = leaky2(fma2<VARIANT>(make_float2(w.w, w.w), x, make_float2(b.w, b.w)));
-    }
-#pragma unroll
-    for (int layer = 0; layer < 2; ++layer) {  // layers 1, 2: weight[H][H], bias[H]
-        const int wo = 2 * H + layer * (H * H + H);
-        float2(&src)[H] = layer == 0 ? g : h;
-        float2(&dst)[H] = layer == 0 ? h : g;
-#pragma unroll
-        for (int j = 0; j < H; j += 4) {
-            const float4 b = lds4(W, wo + H * H + j);
-            float2 acc[4] = {make_float2(b.x, b.x), make_float2(b.y, b.y), make_float2(b.z, b.z),
-                             make_float2(b.w, b.w)};
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-#pragma unroll
-                for (int i = 0; i < H; i += 4) {
-                    const float4 w = lds4(W, wo + (j + u) * H + i);
-                    acc[u] = fma2<VARIANT>(make_float2(w.x, w.x), src[i + 0], acc[u]);
-                    acc[u] = fma2<VARIANT>(make_float2(w.y, w.y), src[i + 1], acc[u]);
-                    acc[u] = fma2<VARIANT>(make_float2(w.z, w.z), src[i + 2], acc[u]);
-                    acc[u] = fma2<VARIANT>(make_float2(w.w, w.w), src[i + 3], acc[u]);
-                }
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) dst[j + u] = leaky2(acc[u]);
-        }
-    }
-#pragma unroll
-    for (int j = 0; j < H; ++j) h[j] = g[j];
-}
-
-template <int H, int NO, int VARIANT>
-__device__ __forceinline__ void pp_last(const float *W, const float2 (&h)[H], float2 (&out)[NO]) {
-    const int wo = 2 * H + 2 * (H * H + H);
-#pragma unroll
-    for (int j = 0; j < NO; ++j) {
-        const float b = W[wo + NO * H + j];
-        float2 acc = make_float2(b, b);
-#pragma unroll
-        for (int i = 0; i < H; i += 4) {
-            const float4 w = lds4(W, wo + j * H + i);
-            acc = fma2<VARIANT>(make_float2(w.x, w.x), h[i + 0], acc);
-            acc = fma2<VARIANT>(make_float2(w.y, w.y), h[i + 1], acc);
-            acc = fma2<VARIANT>(make_float2(w.z, w.z), h[i + 2], acc);
-            acc = fma2<VARIANT>(make_float2(w.w, w.w), h[i + 3], acc);
-        }
-        out[j] = acc;
-    }
-}
 
 // =====================================================================================
-// output-packed engine (variant 2): float2 = (unit j, unit j+1) of ONE point; two points A, B
+// output-packed engine: float2 = (unit j, unit j+1) of ONE point; two points A, B
 // smem net layout: w0[H] b0[H] | Wt1[in][out] b1[H] | Wt2[in][out] b2[H] | Wt3[in][NOP] b3[NOP]
 // (n_out == 1: w3[H] b3[4])
 // =====================================================================================
-template <int H, int NOUT2, class WT>
-__device__ __forceinline__ void op_dense(const WT W, int wt_off, int bias_off, const float2 (&inA)[H / 2],
+template <int H, int NOUT2>
+__device__ __forceinline__ void op_dense(const WShared W, int wt_off, int bias_off, const float2 (&inA)[H / 2],
                                          const float2 (&inB)[H / 2], float2 (&outA)[NOUT2],
                                          float2 (&outB)[NOUT2]) {
     // out[j] = bias[j] + sum_i Wt[i][j] * in[i]; NOUT2 pairs of outputs, row stride 2*NOUT2
@@ -189,8 +106,8 @@ __device__ __forceinline__ void op_dense(const WT W, int wt_off, int bias_off, c
     }
 }
 
-template <int H, class WT>
-__device__ __forceinline__ void op_hidden(const WT W, float xA, float xB, float2 (&hA)[H / 2],
+template <int H>
+__device__ __forceinline__ void op_hidden(const WShared W, float xA, float xB, float2 (&hA)[H / 2],
                                           float2 (&hB)[H / 2]) {
     static_assert(H % 4 == 0, "hidden width must be a multiple of 4");
     constexpr int TS = pl_stride(H), TBL = H, L2 = H + (H + 1) * TS;
@@ -223,8 +140,8 @@ __device__ __forceinline__ void op_hidden(const WT W, float xA, float xB, float2
 }
 
 // single output (AffineHalfFlow s / t): dot product packed over input pairs
-template <int H, class WT>
-__device__ __forceinline__ void op_last1(const WT W, const float2 (&hA)[H / 2], const float2 (&hB)[H / 2],
+template <int H>
+__device__ __forceinline__ void op_last1(const WShared W, const float2 (&hA)[H / 2], const float2 (&hB)[H / 2],
                                          float &oA, float &oB) {
     const int wo = pl_hidden_slots(H);
     float2 accA = make_float2(0.f, 0.f), accB = make_float2(0.f, 0.f);
@@ -244,82 +161,48 @@ __device__ __forceinline__ void op_last1(const WT W, const float2 (&hA)[H / 2], 
 // =====================================================================================
 // conditioner -> spline for both points
 // =====================================================================================
-template <int VARIANT>
-struct WSel {
-    using type = WShared;
-    static __device__ __forceinline__ WShared make(const float *smem, int slot) { return WShared{smem + slot}; }
-};
-
-template <int H, int K, int VARIANT, bool ONE = false>
+template <int H, int K, bool ONE = false>
 __device__ __forceinline__ void spline_half(const float *smem, int slot, const mnf_flow_op &op, float2 cond,
                                             float2 &trans, bool rqs_inverse, float2 &ld) {
     constexpr int NB = 3 * K - 1;
     constexpr bool FAST = MNF_SPLINE_FAST != 0;
-    const float *W = smem + slot;
-    if constexpr (VARIANT >= 2) {
-        constexpr int NP2 = round4(NB) / 2;
-        float2 rA[NP2], rB[NP2];
-        {
-            const auto Wa = WSel<VARIANT>::make(smem, slot);
-            float2 hA[H / 2], hB[H / 2];
-            op_hidden<H>(Wa, cond.x, cond.y, hA, hB);
-            const int wo = pl_hidden_slots(H);
-            op_dense<H, NP2>(Wa, wo, wo + H * 2 * NP2, hA, hB, rA, rB);
-        }
+    constexpr int NP2 = round4(NB) / 2;
+    float2 rA[NP2], rB[NP2];
+    {
+        const WShared W{smem + slot};
+        float2 hA[H / 2], hB[H / 2];
+        op_hidden<H>(W, cond.x, cond.y, hA, hB);
+        const int wo = pl_hidden_slots(H);
+        op_dense<H, NP2>(W, wo, wo + H * 2 * NP2, hA, hB, rA, rB);
+    }
 #pragma unroll 1
-        for (int pt = 0; pt < (ONE ? 1 : 2); ++pt) {
-            float raw[NB];
+    for (int pt = 0; pt < (ONE ? 1 : 2); ++pt) {
+        float raw[NB];
 #pragma unroll
-            for (int o = 0; o < NB; ++o) {
-                const float2 q = pt ? rB[o >> 1] : rA[o >> 1];
-                raw[o] = (o & 1) ? q.y : q.x;
-            }
-            float v = pt ? trans.y : trans.x;
-            float l = 0.f;
-            rq_spline<K, FAST>(raw, K, op.bound, op.edge_deriv, rqs_inverse, v, l);
-            if (pt) { trans.y = v; ld.y += l; } else { trans.x = v; ld.x += l; }
+        for (int o = 0; o < NB; ++o) {
+            const float2 q = pt ? rB[o >> 1] : rA[o >> 1];
+            raw[o] = (o & 1) ? q.y : q.x;
         }
-    } else {
-        float2 raw2[NB];
-        {
-            float2 h[H];
-            pp_hidden<H, VARIANT>(W, cond, h);
-            pp_last<H, NB, VARIANT>(W, h, raw2);
-        }
-#pragma unroll 1
-        for (int pt = 0; pt < 2; ++pt) {
-            float raw[NB];
-#pragma unroll
-            for (int o = 0; o < NB; ++o) raw[o] = pt ? raw2[o].y : raw2[o].x;
-            float v = pt ? trans.y : trans.x;
-            float l = 0.f;
-            rq_spline<K, FAST>(raw, K, op.bound, op.edge_deriv, rqs_inverse, v, l);
-            if (pt) { trans.y = v; ld.y += l; } else { trans.x = v; ld.x += l; }
-        }
+        float v = pt ? trans.y : trans.x;
+        float l = 0.f;
+        rq_spline<K, FAST>(raw, K, op.bound, op.edge_deriv, rqs_inverse, v, l);
+        if (pt) { trans.y = v; ld.y += l; } else { trans.x = v; ld.x += l; }
     }
 }
 
 // scalar-output conditioner (s or t of AffineHalfFlow) for both points
-template <int H, int VARIANT>
+template <int H>
 __device__ __forceinline__ float2 affine_net(const float *smem, int slot, float2 cond) {
-    const float *W = smem + slot;
-    if constexpr (VARIANT >= 2) {
-        const auto Wa = WSel<VARIANT>::make(smem, slot);
-        float2 hA[H / 2], hB[H / 2];
-        op_hidden<H>(Wa, cond.x, cond.y, hA, hB);
-        float2 o;
-        op_last1<H>(Wa, hA, hB, o.x, o.y);
-        return o;
-    } else {
-        float2 h[H], o[1];
-        pp_hidden<H, VARIANT>(W, cond, h);
-        pp_last<H, 1, VARIANT>(W, h, o);
-        return o[0];
-    }
+    const WShared W{smem + slot};
+    float2 hA[H / 2], hB[H / 2];
+    op_hidden<H>(W, cond.x, cond.y, hA, hB);
+    float2 o;
+    op_last1<H>(W, hA, hB, o.x, o.y);
+    return o;
 }
 
-// variant 2: piecewise-linear table of layers 0 + 1, transposed layer 2, last layer (see pl_hidden_slots).  Called by every
-// thread of the CTA (block barriers inside); dst may be shared or global memory.
+// stage one net from the parameter blob into shared memory: piecewise-linear table of layers 0 + 1, transposed layer 2,
+// last layer (see pl_hidden_slots).  Called by every thread of the CTA (block barriers inside).
 template <int H>
 __device__ __forceinline__ void stage_net_pl(const float *__restrict__ src, float *dst, int n_out) {
     constexpr int TS = pl_stride(H), TBL = H, L2 = H + (H + 1) * TS, B2 = L2 + H * H, LAST = B2 + H;
@@ -372,60 +255,27 @@ __device__ __forceinline__ void stage_net_pl(const float *__restrict__ src, floa
     __syncthreads();
 }
 
-// stage one net from the parameter blob into shared memory in the variant's layout (variants 0, 1: the blob's own layout)
-template <int H, int VARIANT>
-__device__ __forceinline__ void stage_net(const float *__restrict__ src, float *dst, int n_out) {
-    if constexpr (VARIANT >= 2) {
-        stage_net_pl<H>(src, dst, n_out);
-        return;
-    }
-    const int hidden = 2 * H + 2 * (H * H + H);
-    const int n = hidden + n_out * H + n_out;
-    // eight independent loads in flight per thread: with one load per trip the copy runs at one L2 latency per
-    // element and thread (measured: ~45 us to stage the 18 nets of BASELINE config 1, most of a small-batch call)
-    for (int e0 = threadIdx.x; e0 < n; e0 += 8 * blockDim.x) {
-        float w8[8];
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-            const int e = e0 + u * blockDim.x;
-            w8[u] = e < n ? src[e] : 0.f;
-        }
-#pragma unroll
-        for (int u = 0; u < 8; ++u) {
-            const int e = e0 + u * blockDim.x;
-            if (e < n) dst[e] = w8[u];
-        }
-    }
-}
-
-// all nets of a program into an image laid out by `lay` (shared memory in the kernel, global memory when pre-staging)
-template <int H, int VARIANT>
+// all nets of a program into shared memory, laid out by `lay`
+template <int H>
 __device__ __forceinline__ void stage_program(const FlowProgram &prog, const FastLayout &lay,
                                               const float *__restrict__ params, float *image) {
-    if constexpr (VARIANT == 2) {  // padding lanes of the last layers must read zeros
-        for (int e = threadIdx.x; e < lay.total_slots; e += blockDim.x) image[e] = 0.f;
-        __syncthreads();
-    }
+    // padding lanes of the last layers must read zeros
+    for (int e = threadIdx.x; e < lay.total_slots; e += blockDim.x) image[e] = 0.f;
+    __syncthreads();
     for (int k = 0; k < prog.n_ops; ++k) {
         const mnf_flow_op &op = prog.ops[k];
         if (op.type != MNF_OP_AFFINE_HALF && op.type != MNF_OP_NSF_CL) continue;
         for (int which = 0; which < 2; ++which) {
             if (op.type == MNF_OP_AFFINE_HALF && !(op.flags & (which ? MNF_FLAG_SHIFT : MNF_FLAG_SCALE))) continue;
-            stage_net<H, VARIANT>(params + op.net_off[which], image + lay.net_slot[k][which], op.sizes[op.n_lin]);
+            stage_net_pl<H>(params + op.net_off[which], image + lay.net_slot[k][which], op.sizes[op.n_lin]);
         }
     }
-}
-
-template <int H>
-__global__ void flow_stage_image_kernel(const __grid_constant__ FlowProgram prog, const __grid_constant__ FastLayout lay,
-                                        const float *__restrict__ params, float *__restrict__ image) {
-    stage_program<H, 2>(prog, lay, params, image);
 }
 
 // everything that happens to one pair of points: load, all flows, store.
 // ONE: small-batch mode -- `pair` is a POINT index, the B lane of every float2 is a dead copy that the compiler removes
 // (nothing is stored from it), so a thread walks half the dependent FFMA2 chain and twice as many warps share the work.
-template <int H, int K, int VARIANT, bool ONE = false>
+template <int H, int K, bool ONE = false>
 __device__ __forceinline__ void process_pair(const FlowProgram &prog, const FastLayout &lay,
                                              const float *__restrict__ params, const float *smem,
                                              const float *__restrict__ x, float *__restrict__ y,
@@ -484,7 +334,7 @@ __device__ __forceinline__ void process_pair(const FlowProgram &prog, const Fast
 #pragma unroll 1
             for (int which = 0; which < 2; ++which) {
                 if (!(op.flags & (which ? MNF_FLAG_SHIFT : MNF_FLAG_SCALE))) continue;
-                const float2 o = affine_net<H, VARIANT>(smem, lay.net_slot[k][which], cond);
+                const float2 o = affine_net<H>(smem, lay.net_slot[k][which], cond);
                 if (which) st[1] = o; else st[0] = o;
             }
             const float2 s = st[0], t = st[1];
@@ -507,7 +357,7 @@ __device__ __forceinline__ void process_pair(const FlowProgram &prog, const Fast
                 const bool use_f1 = (step == 0) != (inverse != 0);
                 const float2 cond = use_f1 ? v0 : v1;
                 float2 tr = use_f1 ? v1 : v0;
-                spline_half<H, K, VARIANT, ONE>(smem, lay.net_slot[k][use_f1 ? 0 : 1], op, cond, tr, inverse != 0, ld);
+                spline_half<H, K, ONE>(smem, lay.net_slot[k][use_f1 ? 0 : 1], op, cond, tr, inverse != 0, ld);
                 if (use_f1) v1 = tr; else v0 = tr;
             }
         }
@@ -536,56 +386,39 @@ __device__ __forceinline__ void process_pair(const FlowProgram &prog, const Fast
     }
 }
 
-template <int H, int K, int VARIANT, bool ONE = false>
+template <int H, int K, bool ONE = false>
 __global__ void __launch_bounds__(128, 4)
 flow_fast_kernel(const __grid_constant__ FlowProgram prog, const __grid_constant__ FastLayout lay,
                  const float *__restrict__ params, const float *__restrict__ x, float *__restrict__ y,
                  float *__restrict__ log_det, float *__restrict__ base_lp, float *__restrict__ inter,
-                 long long n_rows, int dir_flags, const float *__restrict__ staged) {
+                 long long n_rows, int dir_flags) {
     extern __shared__ __align__(16) float smem[];
     const int inverse = dir_flags & 1;
     const bool sum_lp = dir_flags & 2;
-    if (staged != nullptr) {
-        // the shared-memory image was laid out once by flow_stage_image_kernel (mnf_flow_stack_stage): plain 16-byte
-        // copy, eight loads in flight per thread (total_slots is a multiple of 4)
-        const float4 *src = reinterpret_cast<const float4 *>(staged);
-        float4 *dst = reinterpret_cast<float4 *>(smem);
-        const int n4 = lay.total_slots >> 2;
-        for (int i0 = threadIdx.x; i0 < n4; i0 += 8 * blockDim.x) {
-            float4 v[8];
-#pragma unroll
-            for (int u = 0; u < 8; ++u)
-                if (i0 + u * blockDim.x < n4) v[u] = src[i0 + u * blockDim.x];
-#pragma unroll
-            for (int u = 0; u < 8; ++u)
-                if (i0 + u * blockDim.x < n4) dst[i0 + u * blockDim.x] = v[u];
-        }
-    } else {
-        stage_program<H, VARIANT>(prog, lay, params, smem);
-    }
+    stage_program<H>(prog, lay, params, smem);
     __syncthreads();
 
     const long long n_pairs = ONE ? n_rows : (n_rows + 1) >> 1;
     const long long first = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     // persistent grid-stride loop: the nets are staged once per CTA
     for (long long pair = first; pair < n_pairs; pair += (long long)gridDim.x * blockDim.x)
-        process_pair<H, K, VARIANT, ONE>(prog, lay, params, smem, x, y, log_det, base_lp, inter, n_rows, inverse, sum_lp,
-                                         pair, true);
+        process_pair<H, K, ONE>(prog, lay, params, smem, x, y, log_det, base_lp, inter, n_rows, inverse, sum_lp, pair,
+                                true);
 }
 
-// batches below this many points take the one-point-per-thread form of variant 2 (latency, not throughput, matters)
+// batches below this many points take the one-point-per-thread form (latency, not throughput, matters)
 constexpr long long kOnePointMaxRows = 148LL * 128;
 
-template <int H, int K, int VARIANT, bool ONE = false>
+template <int H, int K, bool ONE = false>
 int launch_inst(const FlowProgram &prog, const FastLayout &lay, size_t smem_bytes, const float *params,
                 const float *x, float *y, float *log_det, float *base_lp, float *inter, int64_t n_rows,
-                int inverse, const DeviceProps *dp, cudaStream_t stream, const float *staged = nullptr) {
-    if constexpr (VARIANT == 2 && !ONE) {
+                int inverse, const DeviceProps *dp, cudaStream_t stream) {
+    if constexpr (!ONE) {
         if (n_rows <= kOnePointMaxRows)
-            return launch_inst<H, K, 2, true>(prog, lay, smem_bytes, params, x, y, log_det, base_lp, inter, n_rows, inverse, dp,
-                                              stream, staged);
+            return launch_inst<H, K, true>(prog, lay, smem_bytes, params, x, y, log_det, base_lp, inter, n_rows, inverse, dp,
+                                           stream);
     }
-    auto kern = flow_fast_kernel<H, K, VARIANT, ONE>;
+    auto kern = flow_fast_kernel<H, K, ONE>;
     static thread_local int occ_cache = -1;
     static thread_local size_t occ_smem = 0;
     if (occ_cache < 0 || occ_smem != smem_bytes) {
@@ -605,31 +438,19 @@ int launch_inst(const FlowProgram &prog, const FastLayout &lay, size_t smem_byte
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
     kern<<<(unsigned)blocks, threads, smem_bytes, stream>>>(prog, lay, params, x, y, log_det, base_lp, inter, n_rows,
-                                                            inverse & 3, VARIANT == 2 ? staged : nullptr);
+                                                            inverse & 3);
     return launch_status("flow_fast_kernel");
 }
 
+#define MNF_FLOW_FAST_ARGS                                                                                            \
+    const FlowProgram &prog, const FastLayout &lay, size_t smem_bytes, const float *params, const float *x, float *y, \
+        float *log_det, float *base_lp, float *inter, int64_t n_rows, int inverse, const DeviceProps *dp,             \
+        cudaStream_t stream
 
-#define MNF_FLOW_FAST_ARGS                                                                                    \
-    int variant, const FlowProgram &prog, const FastLayout &lay, size_t smem_bytes, const float *params,      \
-        const float *x, float *y, float *log_det, float *base_lp, float *inter, int64_t n_rows, int inverse,  \
-        float *workspace, const mnf_gather_out *gather, const DeviceProps *dp, cudaStream_t stream
-
-#define MNF_FLOW_FAST_DEFINE(HH, KK)                                                                            \
-    int launch_fast_##HH##_##KK(MNF_FLOW_FAST_ARGS) {                                                           \
-        if (variant == 0)                                                                                       \
-            return launch_inst<HH, KK, 0>(prog, lay, smem_bytes, params, x, y, log_det, base_lp, inter, n_rows, \
-                                          inverse, dp, stream);                                                 \
-        if (variant == 1)                                                                                       \
-            return launch_inst<HH, KK, 1>(prog, lay, smem_bytes, params, x, y, log_det, base_lp, inter, n_rows, \
-                                          inverse, dp, stream);                                                 \
-        return launch_inst<HH, KK, 2>(prog, lay, smem_bytes, params, x, y, log_det, base_lp, inter, n_rows,     \
-                                      inverse, dp, stream, (inverse & 4) ? workspace : nullptr);                \
-    }                                                                                                           \
-    int stage_image_##HH##_##KK(const FlowProgram &prog, const FastLayout &lay, const float *params,            \
-                                float *image, cudaStream_t stream) {                                            \
-        flow_stage_image_kernel<HH><<<1, 256, 0, stream>>>(prog, lay, params, image);                           \
-        return launch_status("flow_stage_image_kernel");                                                        \
+#define MNF_FLOW_FAST_DEFINE(HH, KK)                                                                                  \
+    int launch_fast_##HH##_##KK(MNF_FLOW_FAST_ARGS) {                                                                 \
+        return launch_inst<HH, KK>(prog, lay, smem_bytes, params, x, y, log_det, base_lp, inter, n_rows, inverse, dp, \
+                                   stream);                                                                           \
     }
 
 }  // namespace mnf

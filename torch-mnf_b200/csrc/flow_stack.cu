@@ -15,17 +15,22 @@ int launch_flow_generic(const mnf_flow_op *ops, int n_ops, const float *params, 
 int launch_flow_fast(const mnf_flow_op *ops, int n_ops, const float *params, int64_t n_params, const float *x,
                      float *y, float *log_det, float *base_lp, float *inter, int64_t n_rows, int dim, int inverse,
                      int mode, float *workspace, const mnf_gather_out *gather, cudaStream_t stream, bool plan_only);
-int64_t flow_stage_size(const mnf_flow_op *ops, int n_ops, int dim);
-int64_t flow_tc_workspace_floats();
 int64_t flow_pl_workspace_floats(int n_ops);
 int64_t flow_pl_image_floats(const mnf_flow_op *ops, int n_ops, int dim);
-int flow_stage_image(const mnf_flow_op *ops, int n_ops, const float *params, int dim, float *image, cudaStream_t stream);
+int flow_pl_build(const mnf_flow_op *ops, int n_ops, const float *params, int dim, float *image, cudaStream_t stream);
 int launch_made_fast(const mnf_flow_op *ops, int n_ops, const float *params, const float *x, float *y, float *log_det,
                      float *base_lp, float *inter, int64_t n_rows, int dim, int dir_flags, float *scratch,
                      cudaStream_t stream, bool plan_only);
 int launch_flow_pl_sample(const mnf_flow_op *ops, int n_ops, const float *params, uint64_t seed, uint32_t noise_stream,
                           uint64_t row_offset, float *x, float *log_prob, float *z, int64_t n_rows, int dim, bool staged,
                           float *workspace, cudaStream_t stream);
+
+// MNF_RUN_VARIANT(v) of a call, -1 = library default.  Variant 4 named a kernel the table kernel replaced: its requests run
+// the library default.
+static int requested_variant(int flags) {
+    const int v = ((flags & MNF_RUN_VARIANT_MASK) >> 4) - 1;
+    return v == 4 ? -1 : v;
+}
 
 // ---- base draws of mnf_flow_stack_sample for the programs the table kernel does not run ----
 // One thread per row: z[r, c] = philox_normal(element (row_offset + r) dim + c).  finish = 0 stores z; finish = 1 draws the
@@ -160,10 +165,10 @@ int mnf_flow_stack_run(const mnf_flow_op *ops_host, int n_ops, const float *para
     MNF_REQUIRE(n_rows >= 0, MNF_E_ARG, "n_rows=%lld is negative", (long long)n_rows);
     MNF_REQUIRE((flags & ~(MNF_RUN_INVERSE | MNF_RUN_GENERIC | MNF_RUN_LOGPROB | MNF_RUN_STAGED | MNF_RUN_VARIANT_MASK)) == 0, MNF_E_ARG,
                 "unknown bits in flags=0x%x", flags);
-    // bit1: sum into base_lp; bit2: workspace holds the pre-staged image (dim-2 shared-memory kernel only)
+    // bit1: sum into base_lp; bit2: workspace holds the staged tables of the dim-2 table kernel
     const int inverse = (flags & MNF_RUN_INVERSE) | ((flags & MNF_RUN_LOGPROB) ? 2 : 0) |
                         ((flags & MNF_RUN_STAGED) && workspace && dim == 2 ? 4 : 0);
-    const int variant = ((flags & MNF_RUN_VARIANT_MASK) >> 4) - 1;  // -1 = library default
+    const int variant = requested_variant(flags);
     if (n_rows == 0) return 0;
     MNF_REQUIRE(x != nullptr, MNF_E_ARG, "x is NULL");
     MNF_REQUIRE(y || log_det || base_log_prob, MNF_E_ARG, "no output requested");
@@ -180,7 +185,7 @@ int mnf_flow_stack_run(const mnf_flow_op *ops_host, int n_ops, const float *para
         if (rc != 1) return rc;
     }
     MNF_REQUIRE(!gather || (gather->n_peers == 0 && !gather->multicast_ptr), MNF_E_SHAPE,
-                "peer-memory gather output needs the piecewise-linear or the tensor-core dim-2 kernel (AffineHalfFlow / NSF_CL stack in log-prob mode, with a workspace)");
+                "peer-memory gather output needs the piecewise-linear dim-2 kernel (AffineHalfFlow / NSF_CL stack in log-prob mode, with a workspace)");
     return launch_flow_generic(ops_host, n_ops, params, n_params, x, y, log_det, base_log_prob, intermediates,
                                n_rows, dim, inverse & 3, st);
 }
@@ -198,7 +203,7 @@ int mnf_flow_stack_sample(const mnf_flow_op *ops_host, int n_ops, const float *p
     MNF_REQUIRE(params || n_params == 0, MNF_E_ARG, "params is NULL");
     cudaStream_t st = (cudaStream_t)stream;
     const bool staged = (flags & MNF_RUN_STAGED) && workspace && dim == 2;
-    const int variant = ((flags & MNF_RUN_VARIANT_MASK) >> 4) - 1;
+    const int variant = requested_variant(flags);
     // whole call in the table kernel: the draw, the stack and log N(z) - log_det in one pass
     if (!(flags & MNF_RUN_GENERIC) && (variant < 0 || variant == 6 || staged) && n_ops > 0 && (x || log_prob)) {
         rc = launch_flow_pl_sample(ops_host, n_ops, params, seed, noise_stream, row_offset, x, log_prob, z, n_rows, dim, staged,
@@ -269,8 +274,7 @@ int mnf_flow_handle_log_prob(const mnf_flow_handle *h, const float *x, float *lo
         rc = launch_made_fast(h->ops, h->n_ops, h->params, x, nullptr, nullptr, log_prob, nullptr, n_rows, h->dim, base,
                               n_rows <= h->workspace_rows ? h->workspace : nullptr, st, false);
         if (rc != 1) return rc;
-    } else if (h->staged && (n_rows < (1 << 16) || flow_pl_image_floats(h->ops, h->n_ops, h->dim) > 0)) {
-        // the staged conditioner tables (any batch), or for programs without them the pre-staged shared-memory image (small batches)
+    } else if (h->staged) {  // the staged conditioner tables: the table kernel, any batch
         rc = launch_flow_fast(h->ops, h->n_ops, h->params, h->n_params, x, nullptr, nullptr, log_prob, nullptr, n_rows, 2,
                               base | 4, -1, const_cast<float *>(h->staged), nullptr, st, false);
         if (rc != 1) return rc;
@@ -288,30 +292,27 @@ int mnf_flow_handle_log_prob(const mnf_flow_handle *h, const float *x, float *lo
 
 int64_t mnf_flow_stack_stage_size(const mnf_flow_op *ops_host, int n_ops, int dim, int64_t n_params) {
     if (validate_program(ops_host, n_ops, dim, n_params)) return 0;
-    return flow_stage_size(ops_host, n_ops, dim);
+    return flow_pl_image_floats(ops_host, n_ops, dim);
 }
 
 int64_t mnf_flow_stack_stage_max_rows(const mnf_flow_op *ops_host, int n_ops, int dim, int64_t n_params) {
     if (validate_program(ops_host, n_ops, dim, n_params)) return 0;
-    if (flow_pl_image_floats(ops_host, n_ops, dim) > 0) return INT64_MAX;
-    return flow_stage_size(ops_host, n_ops, dim) > 0 ? (1 << 16) - 1 : 0;
+    return flow_pl_image_floats(ops_host, n_ops, dim) > 0 ? INT64_MAX : 0;
 }
 
 int mnf_flow_stack_stage(const mnf_flow_op *ops_host, int n_ops, const float *params, int64_t n_params, int dim,
                          float *staged, void *stream) {
     int rc = validate_program(ops_host, n_ops, dim, n_params);
     if (rc) return rc;
-    return flow_stage_image(ops_host, n_ops, params, dim, staged, (cudaStream_t)stream);
+    return flow_pl_build(ops_host, n_ops, params, dim, staged, (cudaStream_t)stream);
 }
 
 int64_t mnf_flow_stack_workspace(int n_ops, int64_t n_rows, int dim) {
     if (dim == 64) return n_rows * 64;  // MADE density stack in log-prob mode parks z here between flows
-    // dim 2: the conditioner tables of the piecewise-linear kernel or the weight image of the tensor-core kernel, whichever
-    // is larger (every other dim-2 kernel needs none)
+    // dim 2: the conditioner tables of the piecewise-linear kernel (the constants of affine_stream_kernel fit in less;
+    // every other dim-2 kernel needs none)
     (void)n_rows;
-    if (dim != 2) return 0;
-    const int64_t tc = flow_tc_workspace_floats(), pl = flow_pl_workspace_floats(n_ops);
-    return tc > pl ? tc : pl;
+    return dim == 2 ? flow_pl_workspace_floats(n_ops) : 0;
 }
 
 int mnf_glow_assemble(const float *P, const float *L, const float *U, const float *S, float *out, int dim,

@@ -216,8 +216,8 @@ class BoundLogProb:
         self.device, self.dim, self.max_rows = prog._blob.device, dim, int(max_rows)
         self._blob = prog._blob
         self._staged = prog._staged_image(lib, 1, dim, None)
-        # dim 2: the kernels a bound call can reach need at most the weight image of the tensor-core kernel, whatever the
-        # batch; other dims (MADE density in log-prob mode) park max_rows points in the workspace
+        # dim 2: the kernels a bound call can reach need at most room for the conditioner tables, whatever the batch; other
+        # dims (MADE density in log-prob mode) park max_rows points in the workspace
         need = lib.mnf_flow_stack_workspace(prog._n_ops, 0 if dim == 2 else self.max_rows, dim)
         self._ws = torch.empty(need, device=self.device, dtype=torch.float32) if need > 0 else None
         ws_rows = (1 << 62) if dim == 2 else self.max_rows
@@ -275,19 +275,18 @@ class FlowProgram:
         self._ops = (_lib.FlowOp * max(len(ops), 1))(*ops)
         self._n_ops = len(ops)
         self._blob = blob
-        self._staged = {}  # dim -> pre-staged shared-memory image of the nets (or False), rebuilt with the blob
+        self._staged = {}  # dim -> staged conditioner tables (or False), rebuilt with the blob
         self._key = key
 
     def _staged_image(self, lib, n_rows, dim, kernel):
         """Per-parameter-version image of a dim-2 program (mnf_flow_stack_stage), cached until a parameter changes: the
-        conditioner tables of the piecewise-linear kernel (any batch size) or, for the shapes without them, the
-        shared-memory layout of the nets (batches below 65536 rows)."""
+        conditioner tables of the piecewise-linear kernel.  They serve a call of any batch size, so ``n_rows`` does not
+        decide whether the image is used."""
         if dim != 2 or kernel is not None or not 0 < self._n_ops <= _lib.MAX_OPS:
             return None
         img = self._staged.get(dim)
         if img is None:
             size = lib.mnf_flow_stack_stage_size(self._ops, self._n_ops, dim, self._blob.numel())
-            self._staged["max_rows"] = lib.mnf_flow_stack_stage_max_rows(self._ops, self._n_ops, dim, self._blob.numel())
             img = False
             if size > 0:
                 img = torch.empty(size, device=self._blob.device, dtype=torch.float32)
@@ -296,7 +295,7 @@ class FlowProgram:
                                                   img.data_ptr(), _lib.stream_ptr(self._blob.device))
                 _lib.check(rc, "mnf_flow_stack_stage")
             self._staged[dim] = img
-        return img if img is not False and n_rows <= self._staged["max_rows"] else None
+        return img if img is not False else None
 
     @staticmethod
     def _workspace(lib, n_ops, n_rows, dim, dev, have_y=False, kernel=None):
@@ -376,7 +375,8 @@ class FlowProgram:
     @torch.no_grad()
     def run(self, x, inverse: bool, want_inter: bool = False, want_base_lp: bool = False, out=None,
             log_det=None, kernel=None, log_prob_only=False, log_prob_out=None, gather=None):
-        """kernel: None = library default, "generic" = interpreter, 0/1/2 = dim-2 kernel variant.
+        """kernel: None = library default, "generic" = interpreter, an int = dim-2 kernel variant (MNF_RUN_VARIANT:
+        2 = shared-memory FFMA2 kernel, 5 = lane-split kernel, 6 = table kernel with the tables built inside the call).
         log_prob_only: return (None, None, None, log_det + standard-normal log-density) without
         storing the transformed points (single-chunk programs only).
         gather: optional _lib.GatherOut -- also store the log-probs into peer ranks' buffers (fused gather)."""
