@@ -280,6 +280,16 @@ int mnf_linear_forward(const float *x, int64_t x_rows, const float *z, const flo
                        const float *W_log_var, const float *b_mean, const float *b_log_var,
                        const float *eps, uint64_t seed, uint32_t noise_stream, uint64_t row_offset,
                        float *out, int64_t n_rows, int n_in, int n_out, int relu, void *stream);
+/* mnf_linear_forward followed, after the noise and the ReLU, by the per-column affine map
+ *   out[r, n] = col_scale[n] * out[r, n] + col_shift[n]
+ * -- an eval-mode BatchNorm1d folded to its inference coefficients, col_scale = weight / sqrt(running_var + eps),
+ * col_shift = bias - running_mean * col_scale (MNFFeedForward's hidden blocks).  col_scale and col_shift are both
+ * [n_out] or both NULL (MNF_E_ARG otherwise); with NULL the output is bit for bit mnf_linear_forward's. */
+int mnf_linear_forward_affine(const float *x, int64_t x_rows, const float *z, const float *W_mean,
+                              const float *W_log_var, const float *b_mean, const float *b_log_var,
+                              const float *eps, uint64_t seed, uint32_t noise_stream, uint64_t row_offset,
+                              float *out, int64_t n_rows, int n_in, int n_out, int relu,
+                              const float *col_scale, const float *col_shift, void *stream);
 
 /* Tensor-core (tcgen05, TF32 inputs, fp32 accumulation in TMEM, TMA-fed) variant of mnf_linear_forward
  * for n_in % 4 == 0 and 16-byte aligned operands; results agree with the fp32 path to the 2e-3 relative
@@ -291,6 +301,22 @@ int mnf_linear_forward_tc(const float *x, int64_t x_rows, const float *z, const 
                           const float *eps, uint64_t seed, uint32_t noise_stream, uint64_t row_offset,
                           float *out, int64_t n_rows, int n_in, int n_out, int relu, float *workspace,
                           void *stream);
+/* mnf_linear_forward_tc with the per-column affine map of mnf_linear_forward_affine applied in the mean GEMM's
+ * epilogue; col_scale and col_shift must also be 16-byte aligned (MNF_E_ALIGN). */
+int mnf_linear_forward_tc_affine(const float *x, int64_t x_rows, const float *z, const float *W_mean,
+                                 const float *W_log_var, const float *b_mean, const float *b_log_var,
+                                 const float *eps, uint64_t seed, uint32_t noise_stream, uint64_t row_offset,
+                                 float *out, int64_t n_rows, int n_in, int n_out, int relu,
+                                 const float *col_scale, const float *col_shift, float *workspace, void *stream);
+/* Monte-Carlo moments of a sample-major batch y [n_samples * n_unique, n_cols] (row s * n_unique + b is sample s of
+ * input b, as MNFFeedForward.forward_mc lays them out):
+ *   sums[0, b, n] += sum_s f(y[s * n_unique + b])[n],   sums[1, b, n] += sum_s f(y[s * n_unique + b])[n]^2
+ * sums: fp64 [2, n_unique, n_cols], owned by the caller.  f is the identity, or with softmax = 1 a softmax over the
+ * row (mean class probabilities and their spread).  The sums are formed in fp64 from zero, in sample order, and added
+ * to the buffer once per call: no atomics, no dependence on the launch geometry, and sums of consecutive chunks added
+ * in order give the bits of one call over all samples. */
+int mnf_mc_moments(const float *y, int64_t n_unique, int64_t n_samples, int n_cols, int softmax, double *sums,
+                   void *stream);
 /* mnf_rnvp_forward on the tensor cores (single-Linear conditioners of width <= 64, dim % 16 == 0).
  * Optionally leaves xz_out = tf32(x[m % x_rows] * z_final), the A operand of mnf_linear_forward_tc's mean
  * GEMM (pass z = NULL there and put xz_out at the start of its workspace).  workspace:

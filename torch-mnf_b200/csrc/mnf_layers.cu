@@ -138,6 +138,9 @@ struct MnfLinearProb {
     float *out;
     NoiseSrc eps;
     int relu;
+    // optional per-column affine map after the noise and ReLU, out = col_scale[n] * v + col_shift[n]: an eval-mode
+    // BatchNorm1d folded to its inference coefficients (MNFFeedForward's hidden blocks); NULL = none
+    const float *col_scale, *col_shift;
     static constexpr bool kRowReduce = false;
     struct RowCtx {
         size_t xo, zo;
@@ -154,6 +157,7 @@ struct MnfLinearProb {
     }
     __device__ void epilogue4(int m0, int n, const float (&acc)[2][4], float (&)[4]) const {
         const float b0 = bm[n], b1 = expf(blv[n]);
+        const float sc = col_scale ? col_scale[n] : 1.f, sh = col_scale ? col_shift[n] : 0.f;
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
             const int m = m0 + i;
@@ -161,7 +165,8 @@ struct MnfLinearProb {
             const long long e = (long long)m * N + n;
             const float mean = acc[0][i] + b0, var = acc[1][i] + b1;
             const float v = mean + sqrtf(var) * noise_normal(eps, e, (long long)eps.row_offset * N + e);
-            out[e] = relu ? fmaxf(v, 0.f) : v;
+            const float a = relu ? fmaxf(v, 0.f) : v;
+            out[e] = col_scale ? fmaf(sc, a, sh) : a;
         }
     }
     __device__ void row_out(int, float) const {}
@@ -698,11 +703,22 @@ int mnf_linear_forward(const float *x, int64_t x_rows, const float *z, const flo
                        const float *b_mean, const float *b_log_var, const float *eps, uint64_t seed,
                        uint32_t noise_stream, uint64_t row_offset, float *out, int64_t n_rows, int n_in, int n_out,
                        int relu, void *stream) {
+    return mnf_linear_forward_affine(x, x_rows, z, W_mean, W_log_var, b_mean, b_log_var, eps, seed, noise_stream,
+                                     row_offset, out, n_rows, n_in, n_out, relu, nullptr, nullptr, stream);
+}
+
+int mnf_linear_forward_affine(const float *x, int64_t x_rows, const float *z, const float *W_mean,
+                              const float *W_log_var, const float *b_mean, const float *b_log_var, const float *eps,
+                              uint64_t seed, uint32_t noise_stream, uint64_t row_offset, float *out, int64_t n_rows,
+                              int n_in, int n_out, int relu, const float *col_scale, const float *col_shift,
+                              void *stream) {
     MNF_REQUIRE(x && z && W_mean && W_log_var && b_mean && b_log_var && out, MNF_E_ARG, "NULL pointer");
+    MNF_REQUIRE((col_scale == nullptr) == (col_shift == nullptr), MNF_E_ARG,
+                "col_scale and col_shift must both be given or both be NULL");
     MNF_REQUIRE(n_rows >= 0 && n_in >= 1 && n_out >= 1 && x_rows >= 1, MNF_E_ARG, "bad shape");
     MNF_REQUIRE(n_rows <= 0x7fffffff / 64, MNF_E_SHAPE, "too many rows for one call (%lld)", (long long)n_rows);
     MnfLinearProb p{(int)n_rows, n_out, n_in, x, (int)x_rows, z, W_mean, W_log_var, b_mean, b_log_var, out,
-                    NoiseSrc{eps, seed, noise_stream, row_offset}, relu};
+                    NoiseSrc{eps, seed, noise_stream, row_offset}, relu, col_scale, col_shift};
     return launch_simt_gemm<MnfLinearProb, 2>(p, (cudaStream_t)stream, "mnf_linear_forward");
 }
 

@@ -54,6 +54,9 @@ struct Epilogue {
     uint32_t noise_stream;
     uint64_t row_offset;
     int relu;
+    // mode 1: optional per-column affine map after the noise and ReLU, v = col_scale[n] * v + col_shift[n] (an eval-mode
+    // BatchNorm1d folded to its inference coefficients); NULL = none.  16-byte aligned.
+    const float *col_scale, *col_shift;
     float *out;  // [M, N]  (mode 3: [M, N/2])
     // mode 0 extras
     int round_out;  // store rn_tf32(value): the output feeds another TF32 GEMM
@@ -311,6 +314,17 @@ tf32_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
                             }
                             v[u] = a;
                         }
+                        // per-column affine, 4 columns at a time: the 32-wide staging arrays above are at the register
+                        // limit, so the two pointers are re-read from the parameter bank here (volatile) instead of being
+                        // held in registers across the chunk -- holding them added spill stores to the BN = 32 kernel
+                        const float *cs = *reinterpret_cast<const float *const volatile *>(&ep.col_scale);
+                        if (cs) {
+                            const float *ch = *reinterpret_cast<const float *const volatile *>(&ep.col_shift);
+                            const float4 sc = __ldg(reinterpret_cast<const float4 *>(cs + n0 + j));
+                            const float4 sh = __ldg(reinterpret_cast<const float4 *>(ch + n0 + j));
+                            v[0] = fmaf(sc.x, v[0], sh.x), v[1] = fmaf(sc.y, v[1], sh.y);
+                            v[2] = fmaf(sc.z, v[2], sh.z), v[3] = fmaf(sc.w, v[3], sh.w);
+                        }
                         *reinterpret_cast<float4 *>(orow + j) = make_float4(v[0], v[1], v[2], v[3]);
                     }
                 } else if (m < M && n0 < N) {
@@ -333,6 +347,7 @@ tf32_gemm_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
                                 a = fmaf(sdrow[n], z, a);
                             }
                             if (ep.relu) a = fmaxf(a, 0.f);
+                            if (ep.col_scale) a = fmaf(ep.col_scale[n], a, ep.col_shift[n]);
                             if (ep.round_out) a = rn_tf32(a);
                         }
                         orow[n] = a;
@@ -826,7 +841,21 @@ int mnf_linear_forward_tc(const float *x, int64_t x_rows, const float *z, const 
                           const float *b_mean, const float *b_log_var, const float *eps, uint64_t seed,
                           uint32_t noise_stream, uint64_t row_offset, float *out, int64_t n_rows, int n_in, int n_out,
                           int relu, float *workspace, void *stream) {
+    return mnf_linear_forward_tc_affine(x, x_rows, z, W_mean, W_log_var, b_mean, b_log_var, eps, seed, noise_stream,
+                                        row_offset, out, n_rows, n_in, n_out, relu, nullptr, nullptr, workspace, stream);
+}
+
+// ... and out = col_scale[n] * out + col_shift[n] after the ReLU (both NULL: the plain layer, bit for bit)
+int mnf_linear_forward_tc_affine(const float *x, int64_t x_rows, const float *z, const float *W_mean,
+                                 const float *W_log_var, const float *b_mean, const float *b_log_var, const float *eps,
+                                 uint64_t seed, uint32_t noise_stream, uint64_t row_offset, float *out, int64_t n_rows,
+                                 int n_in, int n_out, int relu, const float *col_scale, const float *col_shift,
+                                 float *workspace, void *stream) {
     MNF_REQUIRE(x && W_mean && W_log_var && b_mean && b_log_var && out && workspace, MNF_E_ARG, "NULL pointer");
+    MNF_REQUIRE((col_scale == nullptr) == (col_shift == nullptr), MNF_E_ARG,
+                "col_scale and col_shift must both be given or both be NULL");
+    MNF_REQUIRE(((uintptr_t)col_scale % 16) == 0 && ((uintptr_t)col_shift % 16) == 0, MNF_E_ALIGN,
+                "col_scale and col_shift must be 16-byte aligned");
     MNF_REQUIRE(n_rows >= 0 && n_rows <= 0x7fffffff - 256 && x_rows >= 1 && x_rows <= n_rows + (n_rows == 0), MNF_E_ARG,
                 "bad row counts");
     MNF_REQUIRE(n_in % 4 == 0, MNF_E_SHAPE, "tensor-core path needs n_in %% 4 == 0 (got %d)", n_in);
@@ -850,6 +879,7 @@ int mnf_linear_forward_tc(const float *x, int64_t x_rows, const float *z, const 
     tc::Epilogue em{};
     em.mode = 1, em.bias = b_mean, em.sd = sd, em.sd_rows = (int)x_rows, em.eps = eps, em.seed = seed;
     em.noise_stream = noise_stream, em.row_offset = row_offset, em.relu = relu, em.out = out;
+    em.col_scale = col_scale, em.col_shift = col_shift;
     return tc::launch(xz, wm, (int)n_rows, n_out, n_in, em, st);
 }
 

@@ -137,7 +137,7 @@ _data_ptr_of = __import__("operator").methodcaller("data_ptr")
 
 #: per-module caches that hold ctypes descriptors / device blobs: never copied or pickled with the module
 CACHE_KEYS = ("_prog", "_single_prog", "_tc_plan", "_fused_plan", "_rnvp_struct_cache", "_std_base", "_last_kl_terms",
-              "_kl_plan")
+              "_kl_plan", "_bn_fold")
 
 
 def state_without_caches(module):

@@ -60,12 +60,17 @@ _lib.register({
                                 _i64, _int, _vp, _vp, _vp]),
     "mnf_linear_forward": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int,
                                   _int, _int, _vp]),
+    "mnf_linear_forward_affine": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int,
+                                         _int, _int, _vp, _vp, _vp]),
     "mnf_conv2d_forward": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int, _int,
                                   _int, _int, _int, _int, _vp]),
     "mnf_kl_div": (_int, [C.POINTER(KlArgs), _vp]),
     "mnf_linear_tc_workspace": (_i64, [_i64, _i64, _int, _int]),
     "mnf_linear_forward_tc": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int,
                                      _int, _int, _vp, _vp]),
+    "mnf_linear_forward_tc_affine": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int,
+                                            _int, _int, _vp, _vp, _vp, _vp]),
+    "mnf_mc_moments": (_int, [_vp, _i64, _i64, _int, _int, _vp, _vp]),
     "mnf_rnvp_tc_workspace": (_i64, [_int, _i64, _int]),
     "mnf_rnvp_forward_tc": (_int, [C.POINTER(RnvpFlow), _int, _vp, _vp, C.POINTER(C.c_void_p), _u64, _u32, _u64, _i64,
                                    _int, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _u32, _int, _vp]),
@@ -301,9 +306,12 @@ def use_tensor_cores(layer, n_rows, precision):
 
 
 @torch.no_grad()
-def linear_forward(layer, x, z, noise: Noise, x_rows=None, relu=False, precision="auto", staged_ws=None, n_rows=None):
-    """staged_ws: tensor-core workspace whose first n_rows*n_in floats already hold tf32(x*z) (z is then None)."""
+def linear_forward(layer, x, z, noise: Noise, x_rows=None, relu=False, precision="auto", staged_ws=None, n_rows=None,
+                   affine=None):
+    """staged_ws: tensor-core workspace whose first n_rows*n_in floats already hold tf32(x*z) (z is then None).
+    affine: optional (col_scale, col_shift) [n_out] applied after the noise and ReLU (a folded eval-mode BatchNorm1d)."""
     dev = x.device
+    scale, shift = affine if affine is not None else (None, None)
     R = z.size(0) if z is not None else n_rows
     n_in, n_out = layer.W_mean.shape[1], layer.W_mean.shape[0]
     eps, sid = noise.normal((R, n_out))
@@ -315,19 +323,40 @@ def linear_forward(layer, x, z, noise: Noise, x_rows=None, relu=False, precision
         ws = staged_ws if staged_ws is not None else torch.empty(
             _lib.lib().mnf_linear_tc_workspace(xr, R, n_in, n_out), device=dev, dtype=torch.float32)
         with torch.cuda.device(dev):
-            rc = _lib.lib().mnf_linear_forward_tc(x.data_ptr(), xr, _p(z), *(a.data_ptr() for a in args), _p(eps),
-                                                  noise.seed, sid, noise.row_offset, out.data_ptr(), R, n_in, n_out,
-                                                  int(relu), ws.data_ptr(), _lib.stream_ptr(dev))
+            rc = _lib.lib().mnf_linear_forward_tc_affine(x.data_ptr(), xr, _p(z), *(a.data_ptr() for a in args),
+                                                         _p(eps), noise.seed, sid, noise.row_offset, out.data_ptr(), R,
+                                                         n_in, n_out, int(relu), _p(scale), _p(shift), ws.data_ptr(),
+                                                         _lib.stream_ptr(dev))
         _lib.check(rc, "mnf_linear_forward_tc")
         _lib.launch_count += 5
         return out
     with torch.cuda.device(dev):
-        rc = _lib.lib().mnf_linear_forward(x.data_ptr(), x_rows or x.size(0), z.data_ptr(), *(a.data_ptr() for a in args),
-                                           _p(eps), noise.seed, sid, noise.row_offset, out.data_ptr(), R, n_in, n_out,
-                                           int(relu), _lib.stream_ptr(dev))
+        rc = _lib.lib().mnf_linear_forward_affine(x.data_ptr(), x_rows or x.size(0), z.data_ptr(),
+                                                  *(a.data_ptr() for a in args), _p(eps), noise.seed, sid, noise.row_offset,
+                                                  out.data_ptr(), R, n_in, n_out, int(relu), _p(scale), _p(shift),
+                                                  _lib.stream_ptr(dev))
     _lib.check(rc, "mnf_linear_forward")
     _lib.launch_count += 1
     return out
+
+
+def mc_moments(y, n_unique, n_samples, sums, softmax=False):
+    """sums [2, n_unique, n_cols] fp64 += (sum_s f(y), sum_s f(y)^2) over the samples of the sample-major y
+    [n_samples * n_unique, n_cols]; f = identity or a per-row softmax (mnf_mc_moments)."""
+    dev = y.device
+    n_cols = y.size(1)
+    if y.shape != (n_samples * n_unique, n_cols) or sums.shape != (2, n_unique, n_cols):
+        raise ValueError(f"mc_moments: y {tuple(y.shape)} / sums {tuple(sums.shape)} do not match "
+                         f"{n_samples} samples of {n_unique} rows")
+    if sums.dtype != torch.float64 or not sums.is_contiguous() or sums.device != dev:
+        raise ValueError("mc_moments: sums must be a contiguous float64 tensor on the device of y")
+    y = _lib.require_cuda_f32(y, "y")
+    with _lib.on_device(dev):
+        rc = _lib.lib().mnf_mc_moments(y.data_ptr(), n_unique, n_samples, n_cols, int(softmax), sums.data_ptr(),
+                                       _lib.stream_ptr(dev))
+    _lib.check(rc, "mnf_mc_moments")
+    _lib.launch_count += 1
+    return sums
 
 
 @torch.no_grad()

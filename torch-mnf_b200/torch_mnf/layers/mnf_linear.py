@@ -57,8 +57,9 @@ class MNFLinear(nn.Module):
         ld, _ = ops.rnvp_stack_inplace(list(self.flow_q.flows), z, noise)
         return z, ld.squeeze()
 
-    def _forward_rows(self, x, n_rows, noise, relu, precision=None):
-        """forward over n_rows output rows, row r reading x[r % len(x)]."""
+    def _forward_rows(self, x, n_rows, noise, relu, precision=None, affine=None):
+        """forward over n_rows output rows, row r reading x[r % len(x)].  affine: optional (col_scale, col_shift)
+        [n_out] applied after the ReLU in the kernel epilogue (a folded eval-mode BatchNorm1d)."""
         precision = precision or self.precision
         flows_q = list(self.flow_q.flows)
         if ops.use_tensor_cores(self, n_rows, precision) and ops.rnvp_tc_ok(flows_q, self.n_in):
@@ -72,9 +73,10 @@ class MNFLinear(nn.Module):
             else:
                 z = ops.sample_z0(self.q0_mean, self.q0_log_var, n_rows, noise)
                 ops.rnvp_stack_tc(flows_q, z, noise, x=x, x_rows=x.size(0), xz_out=ws, z_is_scratch=True)
-            return ops.linear_forward(self, x, None, noise, x_rows=x.size(0), relu=relu, staged_ws=ws, n_rows=n_rows)
+            return ops.linear_forward(self, x, None, noise, x_rows=x.size(0), relu=relu, staged_ws=ws, n_rows=n_rows,
+                                      affine=affine)
         z, _ = self.sample_z(n_rows, noise)
-        return ops.linear_forward(self, x, z, noise, x_rows=x.size(0), relu=relu, precision=precision)
+        return ops.linear_forward(self, x, z, noise, x_rows=x.size(0), relu=relu, precision=precision, affine=affine)
 
     def forward(self, x, noise=None, row_offset=0, relu=False, precision=None):
         if _train.needs_grad(self, x):  # training: differentiable exact-fp32 path (layers/_train.py)
