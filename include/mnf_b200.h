@@ -104,8 +104,8 @@ typedef struct mnf_flow_op {
  *                  execution order (core.py:20-25 returns them as a list).
  *   workspace    : mnf_flow_stack_workspace() floats of scratch (caller-owned), or NULL if that is 0.
  *   flags        : MNF_RUN_INVERSE = inverse direction (flows[n-1] first), else forward;
- *                  MNF_RUN_GENERIC forces the generic interpreter; MNF_RUN_VARIANT(v) picks a
- *                  code variant of the dim-2 kernel (tests / tuning; 0 = library default);
+ *                  MNF_RUN_GENERIC forces the generic interpreter; MNF_RUN_VARIANT(v) is accepted
+ *                  and runs the library default (see below);
  *                  MNF_RUN_LOGPROB makes base_log_prob receive log_det + base log-density, i.e.
  *                  log p(x) of tests/test_flows.py:22-24 in one pass.
  * Replaces NormalizingFlow.forward/inverse (flows/core.py:17-35). */
@@ -113,8 +113,8 @@ typedef struct mnf_flow_op {
  * log-probability straight into the gather buffers of the other ranks (peer-mapped device pointers, e.g. from
  * torch.distributed._symmetric_memory) at element row_offset + i -- or, when multicast_ptr is set, with ONE
  * multimem.st per element that the switch replicates to every rank.  The data transfer overlaps the kernel's
- * arithmetic; the only collective left after the launch is a barrier.  Supported by the piecewise-linear dim-2 kernel
- * in MNF_RUN_LOGPROB mode. */
+ * arithmetic; the only collective left after the launch is a barrier.  Supported by the dim-2 table kernel for the
+ * programs it runs, in MNF_RUN_LOGPROB mode. */
 #define MNF_MAX_PEERS 8
 typedef struct mnf_gather_out {
     int32_t n_peers;                 /* entries of peer_ptrs in use (0 with multicast)       */
@@ -166,9 +166,10 @@ int mnf_flow_stack_backward(const mnf_flow_op *ops_host, int n_ops, const float 
                             float *grad_x, int64_t n_rows, int dim, int flags, void *stream);
 
 /* Floats of scratch `workspace` must provide for a run of this shape (0 = none needed; NULL is then
- * accepted).  dim 2: room for the conditioner tables of the piecewise-linear kernel, built per call when no staged image
- * is passed (the library keeps no device state of its own: per-call staging lives here; without a workspace a dim-2 run
- * takes the shared-memory kernels, which need none); dim 64: a log-prob-only MADE run parks the points between flows. */
+ * accepted).  dim 2: room for the conditioner tables of the table kernel, built per call when no staged image is passed
+ * (the library keeps no device state of its own: per-call staging lives here).  Required for dim-2 programs with
+ * conditioner nets (AffineHalfFlow / NSF_CL): without it or a staged image such a run returns MNF_E_ARG.  dim 64: a
+ * log-prob-only MADE run parks the points between flows. */
 int64_t mnf_flow_stack_workspace(int n_ops, int64_t n_rows, int dim);
 
 #define MNF_RUN_INVERSE 1
@@ -177,14 +178,14 @@ int64_t mnf_flow_stack_workspace(int n_ops, int64_t n_rows, int dim);
 #define MNF_RUN_STAGED 8  /* `workspace` holds the image written by mnf_flow_stack_stage for these params (below) */
 #define MNF_RUN_VARIANT_MASK 0x70
 #define MNF_RUN_VARIANT(v) ((((v) + 1) << 4) & MNF_RUN_VARIANT_MASK)
-/* v: 6 = every conditioner as a piecewise-linear table of its scalar input (csrc/flow_pl.cu) -- the library default for
- *        dim-2 stacks of AffineConstantFlow / ActNormFlow / Glow / AffineHalfFlow / NSF_CL(K in {4, 5, 6, 8, 10, 12, 16}) whose conditioners
- *        have 1..5 hidden layers of width <= 64, any batch size;
- *    2 = register-resident dim-2 kernel with the nets in shared memory (default of the remaining shapes of its
- *        (hidden, bins) grid, and of calls without a workspace);
- *    5 = eight lanes per point (AffineHalfFlow stacks up to 32768 rows).
- *    0, 1 and 3 (removed shared-memory variants) run 2; 4 (the removed tensor-core kernel) runs the library default.
- *    A variant the program is not eligible for falls back to the library default. */
+/* Dim-2 stacks of AffineConstantFlow / ActNormFlow / Glow / AffineHalfFlow / NSF_CL (K in {4, 5, 6, 8, 10, 12, 16}) whose
+ * conditioners have 1..5 hidden layers of width <= 64 run in one kernel at any batch size: every conditioner as a
+ * piecewise-linear table of its scalar input (csrc/flow_pl.cu).  A stack without conditioner nets has no tables; when the
+ * call has a workspace, an even row count, no intermediates and 16-byte aligned points it is one streaming affine map
+ * instead.  Other programs run the generic interpreter.
+ * v of MNF_RUN_VARIANT(v) once chose among several dim-2 kernels; the others were removed once the table kernel ran every
+ * program they ran, and every v now runs the library default.  6 names the table kernel with its tables built inside the
+ * call, which is what a run without MNF_RUN_STAGED does. */
 
 /* Draws n_rows points of the flow model (standard-normal base, flows in module order) together with their log-density:
  *   z[r]        = N(0, I) draw of global row row_offset + r (Noise convention of the MNF layers below: Philox4x32-10
@@ -195,8 +196,8 @@ int64_t mnf_flow_stack_workspace(int n_ops, int64_t n_rows, int dim);
  *   log_prob[r] = log N(z[r]) - log|det J|(z[r]) = log q(x[r]), the density of the drawn point, without the inverse pass.
  * x, log_prob and z are each optional (NULL), at least one must be given.  flags: MNF_RUN_STAGED, MNF_RUN_GENERIC and
  * MNF_RUN_VARIANT(v) as for mnf_flow_stack_run (forward direction only: MNF_RUN_INVERSE and MNF_RUN_LOGPROB are
- * MNF_E_ARG).  Programs of the piecewise-linear kernel with a workspace or staged image take ONE launch (after the table
- * builder when not staged); every other program draws z, runs the forward dispatch of mnf_flow_stack_run and finishes
+ * MNF_E_ARG).  Programs of the table kernel that have conditioner nets take ONE launch with a workspace or staged image
+ * (after the table builder when not staged); every other program draws z, runs the forward dispatch of mnf_flow_stack_run and finishes
  * log_prob: at most three launches, and x or z must be given to hold the draw.  Box-Muller draws u1 >= 2^-23, so every
  * pair lies within radius 5.65 (a pair of true normals exceeds it with probability 2^-23). */
 int mnf_flow_stack_sample(const mnf_flow_op *ops_host, int n_ops, const float *params, int64_t n_params,
@@ -209,16 +210,16 @@ int mnf_flow_stack_sample(const mnf_flow_op *ops_host, int n_ops, const float *p
  * mnf_flow_stack_stage_size() floats (0 = the program has no such form) the conditioner TABLES of the piecewise-linear
  * kernel (sorted breakpoints and per-piece slopes / values of every conditioner, found in fp64), for the programs that
  * kernel runs.  A run with MNF_RUN_STAGED and that buffer as `workspace` is then ONE launch of that kernel at any batch
- * size (a variant request is ignored). */
+ * size. */
 int64_t mnf_flow_stack_stage_size(const mnf_flow_op *ops_host, int n_ops, int dim, int64_t n_params);
 /* Largest batch a MNF_RUN_STAGED run of this program accepts: INT64_MAX when it has a staged form, else 0. */
 int64_t mnf_flow_stack_stage_max_rows(const mnf_flow_op *ops_host, int n_ops, int dim, int64_t n_params);
 int mnf_flow_stack_stage(const mnf_flow_op *ops_host, int n_ops, const float *params, int64_t n_params, int dim,
                          float *staged, void *stream);
 
-/* Which kernel mnf_flow_stack_run would pick: 0 = generic interpreter, 1 = specialised
- * D=2 kernels (table / register-resident / lane-split by shape and batch), 2 = the exact-fp32 MADE kernels
- * (all-MAF/IAF stacks of an instantiated (dim, hidden) shape with three hidden layers).  Host-only, no launch. */
+/* Which kernel mnf_flow_stack_run would pick: 0 = generic interpreter, 1 = the dim-2 kernels (the table kernel, or
+ * the streaming affine map for a stack without conditioner nets), 2 = the exact-fp32 MADE kernels (all-MAF/IAF stacks
+ * of an instantiated (dim, hidden) shape with three hidden layers).  Host-only, no launch. */
 int mnf_flow_stack_plan(const mnf_flow_op *ops_host, int n_ops, int dim, int64_t n_params);
 
 /* Glow._assemble_W + torch.inverse (glow.py:20-24, 34-35):  W = P (tril(L,-1)+I)(triu(U,1)+diag S),

@@ -1,5 +1,5 @@
-"""Timing + error statistics of the piecewise-linear table kernel (variant 6, flow_pl.cu) next to the shared-memory FFMA2
-kernel (variant 2) on BASELINE config 2, and of the config-1 bound call.
+"""Timing + error statistics of the piecewise-linear table kernel (variant 6, flow_pl.cu: tables built in the call) on
+BASELINE config 2, and of the config-1 bound call.
 Run on a GPU box:  python tests/measure/flow_pl_timing.py [log2_rows]"""
 import json
 import os
@@ -22,7 +22,7 @@ x = 1.5 * torch.randn(n, 2, device="cuda", generator=torch.Generator(device="cud
 out = {"rows": n}
 lp_out = torch.empty(n, device="cuda")
 lps = {}
-for kernel in (2, 6):
+for kernel in (6,):
     for _ in range(3):
         prog.run(x, True, log_prob_only=True, kernel=kernel, log_prob_out=lp_out)
     torch.cuda.synchronize()
@@ -37,7 +37,7 @@ for kernel in (2, 6):
     out[f"k{kernel}_gpts"] = n / ms / 1e6
     lps[kernel] = lp_out[: 1 << 16].clone()
 _, _, _, lpg = prog.run(x[: 1 << 16].contiguous(), True, log_prob_only=True, kernel="generic")
-for k in (2, 6):
+for k in (6,):
     d = (lps[k] - lpg).abs()
     out[f"k{k}_vs_generic_max"] = float(d.max())
     out[f"k{k}_vs_generic_mean"] = float(d.mean())

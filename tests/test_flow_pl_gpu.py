@@ -72,7 +72,7 @@ def test_pl_vs_oracle_seeded(name, scale):
 
 
 SHAPES = {
-    # conditioner shapes outside the (hidden, bins) grid of the register-resident kernels: any depth 2..6, any widths <= 64
+    # conditioner shapes outside the (hidden, bins) grid of the earlier dim-2 kernels: any depth 2..6, any widths <= 64
     "affine_32_16": [{"type": "AffineHalfFlow", "dim": 2, "parity": bool(i % 2), "scale": True, "shift": True, "h_sizes": [32, 16]} for i in range(4)],
     "affine_one_hidden": [{"type": "AffineHalfFlow", "dim": 2, "parity": bool(i % 2), "scale": True, "shift": True, "h_sizes": [40]} for i in range(3)],
     "affine_scale_only": [{"type": "AffineHalfFlow", "dim": 2, "parity": False, "scale": True, "shift": False, "h_sizes": [24, 24, 24]},

@@ -89,19 +89,25 @@ def test_stack_vs_golden(name, kernel):
 
 
 @pytest.mark.parametrize("name", ["rnvp9_moons", "nsfcl3_stack"])
-@pytest.mark.parametrize("variant", [0, 1, 2, 3, 4, 5, 6])
+@pytest.mark.parametrize("variant", [None, 0, 1, 2, 3, 4, 5, 6])
 def test_dim2_kernel_variants(name, variant):
+    """The library default (staged tables) and every MNF_RUN_VARIANT(v) request (tables built in the call; 6 names that
+    kernel, the others name kernels that were removed and run it too): all the table kernel."""
+    from tests.test_flow_pl_gpu import _launched
+
     g = load_golden(name)
     sd, specs = golden_sd(g), golden_spec(g)
     model = load_flow_model(specs, sd)
     prog = model._program()
-    assert prog.plan(torch.device("cuda"), 2) == 1, "BASELINE dim-2 stacks must take the register-resident kernel"
+    assert prog.plan(torch.device("cuda"), 2) == 1, "BASELINE dim-2 stacks must take the table kernel"
     x = t(g, "inv/x").cuda()
+    if variant is not None:
+        assert _launched(lambda: prog.run(x, inverse=True, kernel=variant)) == {"flow_pl_build_kernel": 1, "flow_pl_kernel": 1}
     y, ld, _, _ = prog.run(x, inverse=True, kernel=variant)
     close(y, t(g, "inv/z"), "z", atol_scale=2e-5)
     close(ld, t(g, "inv/ld"), "log_det", atol_scale=4e-5)
     close_vs_oracle((y, ld), sd, specs, t(g, "inv/x"), True, f"{name} variant {variant}")
-    # odd row count exercises the half-filled last pair
+    # odd row count
     y, ld, _, _ = prog.run(x[:101].contiguous(), inverse=True, kernel=variant)
     close(y, t(g, "inv/z")[:101], "z odd", atol_scale=2e-5)
     close(ld, t(g, "inv/ld")[:101], "log_det odd", atol_scale=4e-5)
@@ -340,19 +346,33 @@ def test_full_size_properties_cfg2():
 
 def test_conditioner_free_stack_streaming_kernel():
     """[ActNorm, Glow] x 3 in 2-D is a single affine map: the composed streaming kernel (HBM-bound path) must agree
-    with the oracle and with the op-by-op kernel."""
+    with the oracle, and so must the op-by-op table kernel without tables that takes the calls the streaming kernel
+    cannot (intermediates requested, an odd row count)."""
+    from tests.test_flow_pl_gpu import _launched
+
     specs = [{"type": "ActNormFlow", "dim": 2, "scale": True, "shift": True}, {"type": "Glow", "dim": 2}] * 3
     sd = random_flow_sd(specs, seed=5, scale=0.4)
     model = load_flow_model(specs, sd, return_intermediates=False)
+    prog = model._program()
+    assert prog.plan(torch.device("cuda"), 2) == 1  # also packs the parameters (Glow assembly) before launches are counted
     g = torch.Generator().manual_seed(2)
     x = 2.0 * torch.randn(40000, 2, generator=g)
+    xo = x[:39999]
     for inverse in (True, False):
         ref, ref_ld = flows_cpu.stack(sd, specs, x, inverse=inverse)
-        y, ld, _, _ = model._program().run(x.cuda(), inverse)             # composed streaming path
-        y2, ld2, _, _ = model._program().run(x.cuda(), inverse, kernel=2)  # op-by-op register-resident kernel
-        for a, b in ((y, ld), (y2, ld2)):
-            torch.testing.assert_close(a.cpu(), ref[-1], rtol=1e-5, atol=2e-5)
-            torch.testing.assert_close(b.cpu(), ref_ld, rtol=1e-5, atol=1e-5)
+        stream = lambda: prog.run(x.cuda(), inverse)                       # composed streaming path
+        op_by_op = lambda: prog.run(x.cuda(), inverse, want_inter=True)    # table kernel, every flow's output
+        odd = lambda: prog.run(xo.cuda(), inverse)                         # table kernel, odd row count
+        assert _launched(stream) == {"affine_compose_kernel": 1, "affine_stream_kernel": 1}
+        assert _launched(op_by_op) == {"flow_pl_kernel": 1}
+        assert _launched(odd) == {"flow_pl_kernel": 1}
+        y, ld, _, _ = stream()
+        y2, ld2, inter, _ = op_by_op()
+        y3, ld3, _, _ = odd()
+        for a, b, n in ((y, ld, 40000), (y2, ld2, 40000), (y3, ld3, 39999)):
+            torch.testing.assert_close(a.cpu(), ref[-1][:n], rtol=1e-5, atol=2e-5)
+            torch.testing.assert_close(b.cpu(), ref_ld[:n], rtol=1e-5, atol=1e-5)
+        torch.testing.assert_close(inter.cpu(), torch.stack(ref[1:]), rtol=1e-5, atol=2e-5)
     lp = model.log_prob(x.cuda())
     torch.testing.assert_close(lp.cpu(), flows_cpu.log_prob(sd, specs, x), rtol=1e-5, atol=5e-5)
 
@@ -399,9 +419,9 @@ def test_two_programs_on_two_streams_do_not_share_state():
 
 
 @pytest.mark.parametrize("n_rows", [1, 15, 16, 17, 4096, 20001])
-def test_lane_split_kernel_matches_oracle(n_rows):
-    """Variant 5 (eight lanes per point, csrc/flow_lanes.cu) on AffineHalfFlow stacks: both directions, every output,
-    ragged sizes around the 16-point CTA, against the oracle and the interpreter; h = 24 and h = 8."""
+def test_table_kernel_small_ragged_batches_match_oracle(n_rows):
+    """The table kernel (the default path) on AffineHalfFlow stacks at small and ragged batch sizes: both directions,
+    every output, against the oracle and the interpreter; h = 24 and h = 8."""
     for h in (24, 8):
         specs = [{"type": "ActNormFlow", "dim": 2, "scale": True, "shift": True}] + [
             {"type": "AffineHalfFlow", "dim": 2, "parity": bool(i % 2), "scale": i != 1, "shift": i != 2, "h_sizes": [h, h, h]}
@@ -410,14 +430,14 @@ def test_lane_split_kernel_matches_oracle(n_rows):
         prog = load_flow_model(specs, sd)._program()
         x = 1.2 * torch.randn(n_rows, 2, generator=torch.Generator().manual_seed(n_rows + h))
         for inverse in (True, False):
-            y, ld, inter, lp = prog.run(x.cuda(), inverse, want_inter=True, want_base_lp=True, kernel=5)
+            y, ld, inter, lp = prog.run(x.cuda(), inverse, want_inter=True, want_base_lp=True)
             yg, ldg, interg, lpg = prog.run(x.cuda(), inverse, want_inter=True, want_base_lp=True, kernel="generic")
             torch.testing.assert_close(y, yg, rtol=1e-5, atol=1e-5)
             torch.testing.assert_close(inter, interg, rtol=1e-5, atol=1e-5)
             torch.testing.assert_close(ld, ldg, rtol=1e-5, atol=2e-5)
             torch.testing.assert_close(lp, lpg, rtol=1e-5, atol=2e-5)
             if n_rows >= 16:
-                close_vs_oracle((y, ld), sd, specs, x, inverse, f"lanes h={h} inverse={inverse}")
+                close_vs_oracle((y, ld), sd, specs, x, inverse, f"table kernel h={h} inverse={inverse}")
 
 
 @pytest.mark.parametrize("dim,hidden", [(8, 16), (16, 32), (32, 32), (32, 16), (64, 32), (64, 16), (8, 32), (16, 16)])
@@ -444,8 +464,7 @@ def test_made_fast_kernel_shape_grid(dim, hidden):
 @pytest.mark.parametrize("n_h,K", [(8, 8), (16, 5), (32, 8), (8, 5), (24, 8)])
 @pytest.mark.parametrize("n_rows", [3001, 70001])
 def test_dim2_kernel_shape_grid(n_h, K, n_rows):
-    """The register-resident dim-2 kernels exist for a grid of (hidden width, bins), not only the BASELINE shapes: small
-    batches and large ones (shared-memory variant),
+    """The table kernel runs a grid of (hidden width, bins), not only the BASELINE shapes, at small and large batches:
     against the oracle, with an AffineHalfFlow of the same width in the stack."""
     specs = [{"type": "ActNormFlow", "dim": 2, "scale": True, "shift": True},
              {"type": "NSF_CL", "dim": 2, "K": K, "B": 3, "n_h": n_h},
@@ -453,7 +472,7 @@ def test_dim2_kernel_shape_grid(n_h, K, n_rows):
              {"type": "Glow", "dim": 2}, {"type": "NSF_CL", "dim": 2, "K": K, "B": 3, "n_h": n_h}]
     sd = random_flow_sd(specs, seed=n_h + K, scale=0.4)
     prog = load_flow_model(specs, sd)._program()
-    assert prog.plan("cuda", 2) == 1, "shape must take the register-resident kernel"
+    assert prog.plan("cuda", 2) == 1, "shape must take the table kernel"
     x = 1.4 * torch.randn(n_rows, 2, generator=torch.Generator().manual_seed(n_h * K))
     for inverse in (True, False):
         y, ld, _, _ = prog.run(x.cuda(), inverse)

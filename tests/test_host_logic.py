@@ -72,7 +72,7 @@ def test_flow_program_packing_and_plan():
         assert bool(op.flags & _lib.FLAG_PARITY) == bool(k % 2)
         w0 = flows[k].s_net[0].weight.detach().reshape(-1)
         assert torch.equal(prog._blob[op.net_off[0]: op.net_off[0] + 24], w0)
-    assert prog.plan(torch.device("cpu"), 2) == 1  # BASELINE config 1 -> register-resident kernel
+    assert prog.plan(torch.device("cpu"), 2) == 1  # BASELINE config 1 -> table kernel
     key = prog._key
     prog._build(torch.device("cpu"))
     assert prog._key is key  # cached

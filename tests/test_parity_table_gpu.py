@@ -43,7 +43,7 @@ def _fractions(got, ref, floor):
 def _kernels_for(prog, dim):
     ks = [("default", None), ("generic", "generic")]
     if dim == 2 and prog.plan(torch.device("cuda"), 2) == 1:
-        ks += [(f"dim2_variant{v}", v) for v in (2, 6)]  # shared-memory FFMA2, table kernel
+        ks += [(f"dim2_variant{v}", v) for v in (6,)]  # table kernel, tables built in the call
     return ks
 
 

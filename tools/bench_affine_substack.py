@@ -11,7 +11,7 @@ model = load_flow_model(specs, random_flow_sd(specs, seed=0), return_intermediat
 n = 1 << 24
 x = torch.randn(n, 2, device="cuda")
 prog = model._program()
-print("plan (1 = register-resident kernel):", prog.plan(x.device, 2))
+print("plan (1 = dim-2 kernels):", prog.plan(x.device, 2))
 y = torch.empty_like(x); ld = torch.empty(n, device="cuda"); lp = torch.empty(n, device="cuda")
 def t(fn, it=10):
     fn(); torch.cuda.synchronize()

@@ -32,7 +32,7 @@ def main():
         g = torch.Generator(device="cuda").manual_seed(0)
         x = 1.5 * torch.randn(n, 2, device="cuda", generator=g)
         prog = model._program()
-        for kernel in (2, 6, "generic"):
+        for kernel in (6, "generic"):
             xs = x if kernel != "generic" else x[: n // 16].contiguous()
             for inverse in (True, False):
                 best, med = time_prog(prog, xs, inverse, kernel)
@@ -41,7 +41,7 @@ def main():
                 print(key, out[key], flush=True)
     if name == "cfg1_shape":
         x4 = x[:4096].contiguous()
-        for kernel in (2, 6):
+        for kernel in (6,):
             best, med = time_prog(prog, x4, True, kernel, iters=20)
             print("cfg1 B=4096", kernel, "us best", best * 1e3, "med", med * 1e3)
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)

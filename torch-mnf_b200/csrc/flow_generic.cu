@@ -1,8 +1,8 @@
 // flow_generic.cu -- generic flow-stack interpreter: one thread per point, any dim <= 64,
 // any conditioner widths <= 128, any spline bin count <= 32, every flow type of the
 // reference (flows/core.py:17-35 and the modules it iterates over).  This is the
-// correctness-complete path; the BASELINE shapes (dim 2) take the register-resident
-// kernel in flow_fast.cu instead.  Parameters are staged in shared memory when the blob
+// correctness-complete path; the BASELINE shapes (dim 2) take the table kernel in
+// flow_pl.cu instead.  Parameters are staged in shared memory when the blob
 // fits, otherwise read through L1.
 #include "flow_math.cuh"
 

@@ -1,5 +1,5 @@
 // flow_math.cuh -- per-point device math shared by the generic flow interpreter and the
-// register-resident D=2 kernel: LeakyReLU, softplus, and the rational-quadratic spline of
+// D=2 table kernel: LeakyReLU, softplus, and the rational-quadratic spline of
 // NSF_CL / NSF_AR with the reference's exact parameterisation quirks
 // (spline_flow.py:29-179, SURVEY.md section 8a row a10):
 //   * the raw conditioner outputs are softmax'ed and scaled by 2B in NSF_* (:253-256) and
@@ -27,7 +27,7 @@ __device__ __forceinline__ float leaky02(float x) { return fmaxf(x, 0.2f * x); }
 __device__ __forceinline__ float softplus(float x) { return x > 20.f ? x : log1pf(expf(x)); }
 
 // Math flavour.  FAST = false: libdevice expf/logf/log1pf and IEEE division (generic
-// interpreter).  FAST = true (register-resident kernel): MUFU-based forms whose error stays
+// interpreter).  FAST = true (table kernel): MUFU-based forms whose error stays
 // ~1e-6 relative on the ranges that occur here, an order below the 1e-5 parity tolerance:
 //   exp(x)      -> ex2.approx(x*log2e)      x <= 0 after max subtraction, |x| <= 2B where it matters
 //   a / b       -> a * rcp.approx(b)        (__fdividef, 2 ulp)

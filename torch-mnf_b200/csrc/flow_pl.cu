@@ -5,7 +5,7 @@
 // sees a single coordinate c, and an MLP of Linear / LeakyReLU layers (mlp.py:4-12) is piecewise linear in its input:
 // along the real line it has a finite list of breakpoints (the zero crossings of every hidden pre-activation; about one
 // per hidden unit in practice: ~50 for 1-16-16-16-23, ~70 for 1-24-24-24-1) and between two breakpoints EVERY output is
-// A c + B.  So the whole net -- not only its first two layers (flow_fast.cuh, flow_tc.cu) -- is a table:
+// A c + B.  So the whole net -- not only its first two layers, as earlier dim-2 kernels had it -- is a table:
 //
 //   flow_pl_build_kernel   one CTA per conditioner (an AffineHalfFlow's s- and t-net share their input and one table): finds
 //                          the breakpoints layer by layer in fp64 (on every current piece each pre-activation is affine, so
@@ -969,8 +969,7 @@ static Plan make_plan(const mnf_flow_op *ops, int n_ops, int dim) {
             ++n;
         }
     }
-    if (n == 0) return pl;
-    pl.gl.n = n;
+    pl.gl.n = n;  // 0: a stack without conditioner nets, run without tables
     pl.K = K ? K : 8;
     pl.image_floats = off;
     pl.ok = true;
@@ -1008,16 +1007,19 @@ int64_t flow_pl_workspace_floats(int n_ops) {
     return fpl::HDR_FLOATS + (int64_t)2 * n_ops * fpl::region_floats(fpl::nsf_stride4(fpl::K_MAX));
 }
 
-// floats of the table image of this program, 0 if it has no piecewise-linear form
+// floats of the table image of this program, 0 if it has no tables to stage
 int64_t flow_pl_image_floats(const mnf_flow_op *ops, int n_ops, int dim) {
     const fpl::Plan pl = fpl::make_plan(ops, n_ops, dim);
-    return pl.ok ? pl.image_floats : 0;
+    return pl.ok && pl.gl.n > 0 ? pl.image_floats : 0;
 }
+
+// whether launch_flow_pl runs this program (given a workspace when it has conditioner nets)
+bool flow_pl_accepts(const mnf_flow_op *ops, int n_ops, int dim) { return fpl::make_plan(ops, n_ops, dim).ok; }
 
 int flow_pl_build(const mnf_flow_op *ops, int n_ops, const float *params, int dim, float *image, cudaStream_t stream) {
     using namespace fpl;
     const Plan pl = make_plan(ops, n_ops, dim);
-    MNF_REQUIRE(pl.ok, MNF_E_SHAPE, "program has no piecewise-linear form");
+    MNF_REQUIRE(pl.ok && pl.gl.n > 0, MNF_E_SHAPE, "program has no piecewise-linear form");
     MNF_REQUIRE(params && image && ((uintptr_t)image % 16) == 0, MNF_E_ARG, "NULL or misaligned pointer");
     FlowProgram prog;
     prog.n_ops = n_ops;
@@ -1028,7 +1030,7 @@ int flow_pl_build(const mnf_flow_op *ops, int n_ops, const float *params, int di
 
 int fpl::setup_params(const Plan &pl, const mnf_flow_op *ops, int n_ops, const float *params, float *workspace, int64_t n_rows,
                       bool staged, const DeviceProps *dp, cudaStream_t stream, Params &p, size_t &want) {
-    if (!staged) {
+    if (!staged && pl.gl.n > 0) {
         const int rc = flow_pl_build(ops, n_ops, params, 2, workspace, stream);
         if (rc) return rc;
     }
@@ -1045,16 +1047,17 @@ int fpl::setup_params(const Plan &pl, const mnf_flow_op *ops, int n_ops, const f
     return 0;
 }
 
-// returns 1 if the program is not eligible (caller falls back to the other dim-2 kernels).  dir_flags: bit0 inverse,
-// bit1 log-det summed into base_lp, bit2 `workspace` already holds the image of flow_pl_build for these parameters.
+// returns 1 if the program is not eligible (caller falls back to the interpreter).  dir_flags: bit0 inverse, bit1 log-det
+// summed into base_lp, bit2 `workspace` already holds the image of flow_pl_build for these parameters.  A program without
+// conditioner nets has no tables and needs no workspace.
 int launch_flow_pl(const mnf_flow_op *ops, int n_ops, const float *params, const float *x, float *y, float *log_det,
                    float *base_lp, float *inter, int64_t n_rows, int dim, int dir_flags, float *workspace,
-                   const mnf_gather_out *gather, cudaStream_t stream, bool plan_only) {
+                   const mnf_gather_out *gather, cudaStream_t stream) {
     using namespace fpl;
     const Plan pl = make_plan(ops, n_ops, dim);
     if (!pl.ok) return 1;
-    if (plan_only) return 0;
-    if (!workspace) return 1;  // no room for the tables: the shared-memory kernels need none
+    MNF_REQUIRE(workspace || pl.gl.n == 0, MNF_E_ARG,
+                "dim-2 programs with conditioner nets need a workspace of mnf_flow_stack_workspace() floats (or a staged image)");
     const DeviceProps *dp = device_props();
     MNF_REQUIRE(dp != nullptr, MNF_E_DEVICE, "no CUDA device");
     MNF_REQUIRE(((uintptr_t)workspace % 16) == 0, MNF_E_ALIGN, "workspace must be 16-byte aligned");
@@ -1086,7 +1089,7 @@ int launch_flow_pl_sample(const mnf_flow_op *ops, int n_ops, const float *params
                           float *workspace, cudaStream_t stream) {
     using namespace fpl;
     const Plan pl = make_plan(ops, n_ops, dim);
-    if (!pl.ok || !workspace) return 1;
+    if (!pl.ok || pl.gl.n == 0 || !workspace) return 1;
     const DeviceProps *dp = device_props();
     MNF_REQUIRE(dp != nullptr, MNF_E_DEVICE, "no CUDA device");
     MNF_REQUIRE(((uintptr_t)workspace % 16) == 0, MNF_E_ALIGN, "workspace must be 16-byte aligned");

@@ -1,10 +1,11 @@
-// flow_stack.cu -- C-ABI entry points for flow stacks (dispatch: dim-2 register-resident
-// kernel when the program qualifies, generic interpreter otherwise) and the two small
-// parameter-side kernels (Glow assembly, ActNorm data-dependent init).
+// flow_stack.cu -- C-ABI entry points for flow stacks (dispatch: MADE kernels, the dim-2 table kernel or affine
+// stream when the program qualifies, generic interpreter otherwise) and the two small parameter-side kernels (Glow
+// assembly, ActNorm data-dependent init).
 #include <cstdint>
 #include <new>
 
 #include "common.cuh"
+#include "flow_math.cuh"
 #include "mnf_common.cuh"
 
 namespace mnf {
@@ -12,9 +13,10 @@ int validate_program(const mnf_flow_op *ops, int n_ops, int dim, int64_t n_param
 int launch_flow_generic(const mnf_flow_op *ops, int n_ops, const float *params, int64_t n_params, const float *x,
                         float *y, float *log_det, float *base_lp, float *inter, int64_t n_rows, int dim,
                         int inverse, cudaStream_t stream);
-int launch_flow_fast(const mnf_flow_op *ops, int n_ops, const float *params, int64_t n_params, const float *x,
-                     float *y, float *log_det, float *base_lp, float *inter, int64_t n_rows, int dim, int inverse,
-                     int mode, float *workspace, const mnf_gather_out *gather, cudaStream_t stream, bool plan_only);
+bool flow_pl_accepts(const mnf_flow_op *ops, int n_ops, int dim);
+int launch_flow_pl(const mnf_flow_op *ops, int n_ops, const float *params, const float *x, float *y, float *log_det,
+                   float *base_lp, float *inter, int64_t n_rows, int dim, int dir_flags, float *workspace,
+                   const mnf_gather_out *gather, cudaStream_t stream);
 int64_t flow_pl_workspace_floats(int n_ops);
 int64_t flow_pl_image_floats(const mnf_flow_op *ops, int n_ops, int dim);
 int flow_pl_build(const mnf_flow_op *ops, int n_ops, const float *params, int dim, float *image, cudaStream_t stream);
@@ -25,11 +27,118 @@ int launch_flow_pl_sample(const mnf_flow_op *ops, int n_ops, const float *params
                           uint64_t row_offset, float *x, float *log_prob, float *z, int64_t n_rows, int dim, bool staged,
                           float *workspace, cudaStream_t stream);
 
-// MNF_RUN_VARIANT(v) of a call, -1 = library default.  Variant 4 named a kernel the table kernel replaced: its requests run
-// the library default.
-static int requested_variant(int flags) {
-    const int v = ((flags & MNF_RUN_VARIANT_MASK) >> 4) - 1;
-    return v == 4 ? -1 : v;
+// ---------------------------------------------------------------------------------------------------
+// Conditioner-free stacks (AffineConstantFlow / ActNormFlow / Glow only, dim 2): the whole stack is ONE
+// affine map v -> v A + b with a constant log-det.  A one-thread kernel composes it (fp64) from the packed
+// parameters, then a streaming kernel applies it: 8 points per thread in flight, 128-bit accesses, nothing
+// but HBM traffic (8 B in, 8 B out, 4 B log-det per point) -- the one flow kernel that is truly HBM-bound.
+// ---------------------------------------------------------------------------------------------------
+__global__ void affine_compose_kernel(const __grid_constant__ FlowProgram prog, const float *__restrict__ params,
+                                      int inverse, float *__restrict__ comp) {
+    double A[4] = {1, 0, 0, 1}, b[2] = {0, 0}, ld = 0;
+    for (int kk = 0; kk < prog.n_ops; ++kk) {
+        const mnf_flow_op &op = prog.ops[inverse ? prog.n_ops - 1 - kk : kk];
+        double W[4], t[2] = {0, 0};
+        if (op.type == MNF_OP_AFFINE_CONST) {
+            const double s0 = params[op.aux_off], s1 = params[op.aux_off + 1];
+            const double t0 = params[op.aux_off + 2], t1 = params[op.aux_off + 3];
+            if (inverse) {  // (v - t) * exp(-s), affine_constant_flow.py:24
+                W[0] = exp(-s0), W[3] = exp(-s1), W[1] = W[2] = 0;
+                t[0] = -t0 * W[0], t[1] = -t1 * W[3];
+                ld -= s0 + s1;
+            } else {  // v * exp(s) + t, affine_constant_flow.py:19
+                W[0] = exp(s0), W[3] = exp(s1), W[1] = W[2] = 0;
+                t[0] = t0, t[1] = t1;
+                ld += s0 + s1;
+            }
+        } else {  // Glow: v @ W (glow.py:28) or v @ W^-1 (glow.py:36)
+            const float *Wp = params + op.aux_off + (inverse ? 4 : 0);
+            for (int i = 0; i < 4; ++i) W[i] = Wp[i];
+            ld += inverse ? -(double)params[op.aux_off + 8] : (double)params[op.aux_off + 8];
+        }
+        const double n00 = A[0] * W[0] + A[1] * W[2], n01 = A[0] * W[1] + A[1] * W[3];
+        const double n10 = A[2] * W[0] + A[3] * W[2], n11 = A[2] * W[1] + A[3] * W[3];
+        const double nb0 = b[0] * W[0] + b[1] * W[2] + t[0], nb1 = b[0] * W[1] + b[1] * W[3] + t[1];
+        A[0] = n00, A[1] = n01, A[2] = n10, A[3] = n11, b[0] = nb0, b[1] = nb1;
+    }
+    for (int i = 0; i < 4; ++i) comp[i] = (float)A[i];
+    comp[4] = (float)b[0], comp[5] = (float)b[1], comp[6] = (float)ld;
+}
+
+__global__ void __launch_bounds__(256)
+affine_stream_kernel(const float *__restrict__ comp, const float4 *__restrict__ x, float4 *__restrict__ y,
+                     float2 *__restrict__ log_det, float2 *__restrict__ base_lp, long long n_pairs, int sum_lp) {
+    const float a00 = comp[0], a01 = comp[1], a10 = comp[2], a11 = comp[3], b0 = comp[4], b1 = comp[5], ld = comp[6];
+    const float c = -1.8378770664093453f;
+    constexpr int U = 4;
+    const long long stride = (long long)gridDim.x * blockDim.x;
+    for (long long p0 = (long long)blockIdx.x * blockDim.x + threadIdx.x; p0 < n_pairs; p0 += U * stride) {
+        float4 v[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u)
+            if (p0 + u * stride < n_pairs) v[u] = ld_stream4(x + p0 + u * stride);
+#pragma unroll
+        for (int u = 0; u < U; ++u) {
+            const long long p = p0 + u * stride;
+            if (p >= n_pairs) break;
+            const float4 q = v[u];
+            const float4 o = make_float4(fmaf(q.y, a10, fmaf(q.x, a00, b0)), fmaf(q.y, a11, fmaf(q.x, a01, b1)),
+                                         fmaf(q.w, a10, fmaf(q.z, a00, b0)), fmaf(q.w, a11, fmaf(q.z, a01, b1)));
+            if (y) st_stream4(y + p, o);
+            if (log_det) st_stream2(log_det + p, make_float2(ld, ld));
+            if (base_lp) {
+                float2 lp = make_float2(fmaf(-0.5f, fmaf(o.x, o.x, o.y * o.y), c), fmaf(-0.5f, fmaf(o.z, o.z, o.w * o.w), c));
+                if (sum_lp) lp = make_float2(lp.x + ld, lp.y + ld);
+                st_stream2(base_lp + p, lp);
+            }
+        }
+    }
+}
+
+static int launch_affine_stream(const FlowProgram &prog, const float *params, const float *x, float *y, float *log_det,
+                                float *base_lp, int64_t n_rows, int dir_flags, float *workspace, const DeviceProps *dp,
+                                cudaStream_t stream) {
+    affine_compose_kernel<<<1, 1, 0, stream>>>(prog, params, dir_flags & 1, workspace);
+    int rc = launch_status("affine_compose_kernel");
+    if (rc) return rc;
+    const long long n_pairs = n_rows / 2;
+    long long blocks = (n_pairs + 256 * 4 - 1) / (256 * 4);
+    const long long cap = (long long)dp->sm_count * 8;
+    if (blocks > cap) blocks = cap;
+    if (blocks < 1) blocks = 1;
+    affine_stream_kernel<<<(unsigned)blocks, 256, 0, stream>>>(workspace, (const float4 *)x, (float4 *)y, (float2 *)log_det,
+                                                             (float2 *)base_lp, n_pairs, (dir_flags & 2) != 0);
+    return launch_status("affine_stream_kernel");
+}
+
+// Dim-2 dispatch.  Returns 1 if no dim-2 kernel takes the program (the caller runs the interpreter).  dir_flags: bit0
+// inverse, bit1 log-det summed into base_lp, bit2 `workspace` holds the staged tables.
+//   * conditioner-free stacks (AffineConstantFlow / ActNormFlow / Glow only): affine_stream_kernel when the call suits its
+//     128-bit point pairs (even row count, no intermediates, 16-byte aligned points, a workspace for the composed map, not
+//     staged), else the table kernel, which then has no tables to build;
+//   * every other program flow_pl.cu accepts: the table kernel, with the staged tables or tables built into the workspace
+//     (MNF_E_ARG without a workspace).
+// The fused peer-memory gather stores log-probabilities: outside MNF_RUN_LOGPROB mode the caller reports it.
+static int launch_flow_dim2(const mnf_flow_op *ops, int n_ops, const float *params, const float *x, float *y, float *log_det,
+                            float *base_lp, float *inter, int64_t n_rows, int dim, int dir_flags, float *workspace,
+                            const mnf_gather_out *gather, cudaStream_t stream) {
+    if (dim != 2 || n_ops < 1) return 1;
+    const bool want_gather = gather && (gather->n_peers > 0 || gather->multicast_ptr);
+    if (want_gather && !(dir_flags & 2)) return 1;
+    bool affine_only = true;
+    for (int k = 0; k < n_ops; ++k) affine_only &= ops[k].type == MNF_OP_AFFINE_CONST || ops[k].type == MNF_OP_GLOW;
+    const bool pairs_aligned = (uintptr_t)x % 16 == 0 && (uintptr_t)y % 16 == 0 && (uintptr_t)log_det % 8 == 0 &&
+                               (uintptr_t)base_lp % 8 == 0;
+    if (affine_only && !want_gather && !inter && workspace && !(dir_flags & 4) && n_rows % 2 == 0 && n_rows >= 2 &&
+        pairs_aligned) {
+        FlowProgram prog;
+        prog.n_ops = n_ops;
+        for (int k = 0; k < n_ops; ++k) prog.ops[k] = ops[k];
+        const DeviceProps *dp = device_props();
+        MNF_REQUIRE(dp != nullptr, MNF_E_DEVICE, "no CUDA device");
+        return launch_affine_stream(prog, params, x, y, log_det, base_lp, n_rows, dir_flags, workspace, dp, stream);
+    }
+    return launch_flow_pl(ops, n_ops, params, x, y, log_det, base_lp, inter, n_rows, dim, dir_flags, workspace, gather, stream);
 }
 
 // ---- base draws of mnf_flow_stack_sample for the programs the table kernel does not run ----
@@ -150,10 +259,7 @@ int mnf_flow_stack_plan(const mnf_flow_op *ops_host, int n_ops, int dim, int64_t
         if (launch_made_fast(ops_host, n_ops, nullptr, nullptr, &dummy, nullptr, nullptr, nullptr, 0, dim, inverse,
                              nullptr, nullptr, true) == 0)
             return 2;
-    return launch_flow_fast(ops_host, n_ops, nullptr, n_params, nullptr, nullptr, nullptr, nullptr, nullptr, 0,
-                            dim, 0, -1, nullptr, nullptr, nullptr, true) == 0
-               ? 1
-               : 0;
+    return flow_pl_accepts(ops_host, n_ops, dim) ? 1 : 0;
 }
 
 int mnf_flow_stack_run(const mnf_flow_op *ops_host, int n_ops, const float *params, int64_t n_params,
@@ -168,7 +274,6 @@ int mnf_flow_stack_run(const mnf_flow_op *ops_host, int n_ops, const float *para
     // bit1: sum into base_lp; bit2: workspace holds the staged tables of the dim-2 table kernel
     const int inverse = (flags & MNF_RUN_INVERSE) | ((flags & MNF_RUN_LOGPROB) ? 2 : 0) |
                         ((flags & MNF_RUN_STAGED) && workspace && dim == 2 ? 4 : 0);
-    const int variant = requested_variant(flags);
     if (n_rows == 0) return 0;
     MNF_REQUIRE(x != nullptr, MNF_E_ARG, "x is NULL");
     MNF_REQUIRE(y || log_det || base_log_prob, MNF_E_ARG, "no output requested");
@@ -180,12 +285,12 @@ int mnf_flow_stack_run(const mnf_flow_op *ops_host, int n_ops, const float *para
         if (rc != 1) return rc;
     }
     if (!(flags & MNF_RUN_GENERIC)) {
-        rc = launch_flow_fast(ops_host, n_ops, params, n_params, x, y, log_det, base_log_prob, intermediates,
-                              n_rows, dim, inverse, variant, workspace, gather, st, false);
+        rc = launch_flow_dim2(ops_host, n_ops, params, x, y, log_det, base_log_prob, intermediates, n_rows, dim, inverse,
+                              workspace, gather, st);
         if (rc != 1) return rc;
     }
     MNF_REQUIRE(!gather || (gather->n_peers == 0 && !gather->multicast_ptr), MNF_E_SHAPE,
-                "peer-memory gather output needs the piecewise-linear dim-2 kernel (AffineHalfFlow / NSF_CL stack in log-prob mode, with a workspace)");
+                "peer-memory gather output needs the dim-2 table kernel (a program it runs, in log-prob mode)");
     return launch_flow_generic(ops_host, n_ops, params, n_params, x, y, log_det, base_log_prob, intermediates,
                                n_rows, dim, inverse & 3, st);
 }
@@ -203,9 +308,8 @@ int mnf_flow_stack_sample(const mnf_flow_op *ops_host, int n_ops, const float *p
     MNF_REQUIRE(params || n_params == 0, MNF_E_ARG, "params is NULL");
     cudaStream_t st = (cudaStream_t)stream;
     const bool staged = (flags & MNF_RUN_STAGED) && workspace && dim == 2;
-    const int variant = requested_variant(flags);
     // whole call in the table kernel: the draw, the stack and log N(z) - log_det in one pass
-    if (!(flags & MNF_RUN_GENERIC) && (variant < 0 || variant == 6 || staged) && n_ops > 0 && (x || log_prob)) {
+    if (!(flags & MNF_RUN_GENERIC) && n_ops > 0 && (x || log_prob)) {
         rc = launch_flow_pl_sample(ops_host, n_ops, params, seed, noise_stream, row_offset, x, log_prob, z, n_rows, dim, staged,
                                    workspace, st);
         if (rc != 1) return rc;
@@ -226,8 +330,7 @@ int mnf_flow_stack_sample(const mnf_flow_op *ops_host, int n_ops, const float *p
         if (!(flags & MNF_RUN_GENERIC))
             rc = launch_made_fast(ops_host, n_ops, params, zb, x, log_prob, nullptr, nullptr, n_rows, dim, dir, workspace, st, false);
         if (rc == 1 && !(flags & MNF_RUN_GENERIC))
-            rc = launch_flow_fast(ops_host, n_ops, params, n_params, zb, x, log_prob, nullptr, nullptr, n_rows, dim, dir, variant,
-                                  workspace, nullptr, st, false);
+            rc = launch_flow_dim2(ops_host, n_ops, params, zb, x, log_prob, nullptr, nullptr, n_rows, dim, dir, workspace, nullptr, st);
         if (rc == 1)
             rc = launch_flow_generic(ops_host, n_ops, params, n_params, zb, x, log_prob, nullptr, nullptr, n_rows, dim, 0, st);
         if (rc) return rc;
@@ -275,15 +378,15 @@ int mnf_flow_handle_log_prob(const mnf_flow_handle *h, const float *x, float *lo
                               n_rows <= h->workspace_rows ? h->workspace : nullptr, st, false);
         if (rc != 1) return rc;
     } else if (h->staged) {  // the staged conditioner tables: the table kernel, any batch
-        rc = launch_flow_fast(h->ops, h->n_ops, h->params, h->n_params, x, nullptr, nullptr, log_prob, nullptr, n_rows, 2,
-                              base | 4, -1, const_cast<float *>(h->staged), nullptr, st, false);
+        rc = launch_flow_dim2(h->ops, h->n_ops, h->params, x, nullptr, nullptr, log_prob, nullptr, n_rows, 2, base | 4,
+                              const_cast<float *>(h->staged), nullptr, st);
         if (rc != 1) return rc;
     } else {
         MNF_REQUIRE(n_rows <= h->workspace_rows && h->workspace, MNF_E_ARG,
                     "handle was created with a workspace for %lld rows, call has %lld", (long long)h->workspace_rows,
                     (long long)n_rows);
-        rc = launch_flow_fast(h->ops, h->n_ops, h->params, h->n_params, x, nullptr, nullptr, log_prob, nullptr, n_rows, 2,
-                              base, -1, h->workspace, nullptr, st, false);
+        rc = launch_flow_dim2(h->ops, h->n_ops, h->params, x, nullptr, nullptr, log_prob, nullptr, n_rows, 2, base, h->workspace,
+                              nullptr, st);
         if (rc != 1) return rc;
     }
     return launch_flow_generic(h->ops, h->n_ops, h->params, h->n_params, x, nullptr, nullptr, log_prob, nullptr, n_rows,
@@ -309,8 +412,7 @@ int mnf_flow_stack_stage(const mnf_flow_op *ops_host, int n_ops, const float *pa
 
 int64_t mnf_flow_stack_workspace(int n_ops, int64_t n_rows, int dim) {
     if (dim == 64) return n_rows * 64;  // MADE density stack in log-prob mode parks z here between flows
-    // dim 2: the conditioner tables of the piecewise-linear kernel (the constants of affine_stream_kernel fit in less;
-    // every other dim-2 kernel needs none)
+    // dim 2: the conditioner tables of the table kernel (the constants of affine_stream_kernel fit in less)
     (void)n_rows;
     return dim == 2 ? flow_pl_workspace_floats(n_ops) : 0;
 }

@@ -146,6 +146,16 @@ def state_without_caches(module):
     return {k: v for k, v in module.__dict__.items() if k not in CACHE_KEYS}
 
 
+def _kernel_flags(kernel) -> int:
+    """MNF_RUN_* bits of a ``kernel=`` argument: None = library default, "generic" = interpreter, an int v =
+    MNF_RUN_VARIANT(v)."""
+    if kernel is None:
+        return 0
+    if kernel == "generic":
+        return _lib.RUN_GENERIC
+    return ((int(kernel) + 1) << 4) & 0x70
+
+
 def _state_key(flows, device, tensors):
     """Per-call fingerprint of everything the packed blob depends on: in-place updates bump ``_version``;
     re-assigned storage (``.to()``, ``p.data = ...``, ``load_state_dict(assign=True)``) shows in the data pointers of
@@ -298,14 +308,15 @@ class FlowProgram:
         return img if img is not False else None
 
     @staticmethod
-    def _workspace(lib, n_ops, n_rows, dim, dev, have_y=False, kernel=None):
+    def _workspace(lib, n_ops, n_rows, dim, dev, have_y=False):
         if have_y and dim != 2:
             return None  # only log-prob-only runs (no y buffer) of the MADE kernel park points in the workspace
         need = lib.mnf_flow_stack_workspace(n_ops, n_rows, dim)
         return torch.empty(need, device=dev, dtype=torch.float32) if need > 0 else None
 
     def plan(self, device, dim) -> int:
-        """1 if the dim-2 register-resident kernel will run this program, else 0 (generic)."""
+        """mnf_flow_stack_plan: 1 if a dim-2 kernel (the table kernel, or affine_stream_kernel for a stack without
+        conditioner nets) runs this program, 2 if the MADE kernels do, else 0 (generic interpreter)."""
         self._build(device)
         n = min(self._n_ops, _lib.MAX_OPS)
         return _lib.lib().mnf_flow_stack_plan(self._ops, n, dim, self._blob.numel())
@@ -354,16 +365,12 @@ class FlowProgram:
         x = torch.empty(n_rows, dim, device=dev, dtype=torch.float32) if want_x else None
         lp = torch.empty(n_rows, device=dev, dtype=torch.float32) if want_log_prob else None
         z = torch.empty(n_rows, dim, device=dev, dtype=torch.float32) if want_z else None
-        flags = 0
-        if kernel == "generic":
-            flags |= _lib.RUN_GENERIC
-        elif kernel is not None:
-            flags |= ((int(kernel) + 1) << 4) & 0x70
+        flags = _kernel_flags(kernel)
         ws = self._staged_image(lib, n_rows, dim, kernel)
         if ws is not None:
             flags |= _lib.RUN_STAGED
         else:
-            ws = self._workspace(lib, self._n_ops, n_rows, dim, dev, have_y=want_x, kernel=kernel)
+            ws = self._workspace(lib, self._n_ops, n_rows, dim, dev, have_y=want_x)
         with _lib.on_device(dev):
             rc = lib.mnf_flow_stack_sample(self._ops, self._n_ops, self._blob.data_ptr(), self._blob.numel(),
                                            int(seed) & (2**64 - 1), 0, int(row_offset), _lib.ptr(x), _lib.ptr(lp),
@@ -375,8 +382,9 @@ class FlowProgram:
     @torch.no_grad()
     def run(self, x, inverse: bool, want_inter: bool = False, want_base_lp: bool = False, out=None,
             log_det=None, kernel=None, log_prob_only=False, log_prob_out=None, gather=None):
-        """kernel: None = library default, "generic" = interpreter, an int = dim-2 kernel variant (MNF_RUN_VARIANT:
-        2 = shared-memory FFMA2 kernel, 5 = lane-split kernel, 6 = table kernel with the tables built inside the call).
+        """kernel: None = library default, "generic" = interpreter, an int = MNF_RUN_VARIANT(v): every value runs the
+        library default, but without the cached staged image, so a dim-2 program's tables are built inside the call
+        (6 is the conventional value).
         log_prob_only: return (None, None, None, log_det + standard-normal log-density) without
         storing the transformed points (single-chunk programs only).
         gather: optional _lib.GatherOut -- also store the log-probs into peer ranks' buffers (fused gather)."""
@@ -390,16 +398,12 @@ class FlowProgram:
         n = self._n_ops
         if log_prob_only and 0 < n <= _lib.MAX_OPS:
             lp = log_prob_out if log_prob_out is not None else torch.empty(B, device=dev, dtype=torch.float32)
-            flags = (_lib.RUN_INVERSE if inverse else 0) | _lib.RUN_LOGPROB
-            if kernel == "generic":
-                flags |= _lib.RUN_GENERIC
-            elif kernel is not None:
-                flags |= ((int(kernel) + 1) << 4) & 0x70
+            flags = (_lib.RUN_INVERSE if inverse else 0) | _lib.RUN_LOGPROB | _kernel_flags(kernel)
             ws = self._staged_image(lib, B, D, kernel)
             if ws is not None:
                 flags |= _lib.RUN_STAGED
             else:
-                ws = self._workspace(lib, n, B, D, dev, kernel=kernel)
+                ws = self._workspace(lib, n, B, D, dev)
             with _lib.on_device(dev):
                 rc = lib.mnf_flow_stack_run(self._ops, n, self._blob.data_ptr(), self._blob.numel(), x.data_ptr(),
                                             None, None, lp.data_ptr(), None, B, D, flags, _lib.ptr(ws),
@@ -415,12 +419,8 @@ class FlowProgram:
             y.copy_(x)
             ld.zero_()
         stream = _lib.stream_ptr(dev)
-        ws = self._workspace(lib, min(n, _lib.MAX_OPS), B, D, dev, have_y=True, kernel=kernel)
-        flags = _lib.RUN_INVERSE if inverse else 0
-        if kernel == "generic":
-            flags |= _lib.RUN_GENERIC
-        elif kernel is not None:
-            flags |= ((int(kernel) + 1) << 4) & 0x70
+        ws = self._workspace(lib, min(n, _lib.MAX_OPS), B, D, dev, have_y=True)
+        flags = (_lib.RUN_INVERSE if inverse else 0) | _kernel_flags(kernel)
         staged = self._staged_image(lib, B, D, kernel)
         if staged is not None:
             ws, flags = staged, flags | _lib.RUN_STAGED
