@@ -318,6 +318,13 @@ int mnf_linear_forward_tc_affine(const float *x, int64_t x_rows, const float *z,
  * in order give the bits of one call over all samples. */
 int mnf_mc_moments(const float *y, int64_t n_unique, int64_t n_samples, int n_cols, int softmax, double *sums,
                    void *stream);
+/* mnf_mc_moments(..., softmax = 1, sums) plus entropy_sums[b] += sum_s H(softmax(y[s * n_unique + b])), fp64 [n_unique],
+ * caller-owned; same ordering / from-zero / add-once rules as sums.  H = log z - (1/z) sum_c e_c (y_c - m) with m the
+ * row max, e_c = expf(y_c - m), z = sum_c e_c, in fp64; terms with e_c == 0 add nothing (0 log 0 = 0).  The predictive
+ * entropy, expected entropy and mutual information of a classifier follow from sums and entropy_sums
+ * (MNFLeNet / MNFFeedForward.predict_uncertainty).  Either output NULL: MNF_E_ARG. */
+int mnf_mc_class_moments(const float *y, int64_t n_unique, int64_t n_samples, int n_cols, double *sums,
+                         double *entropy_sums, void *stream);
 /* mnf_rnvp_forward on the tensor cores (single-Linear conditioners of width <= 64, dim % 16 == 0).
  * Optionally leaves xz_out = tf32(x[m % x_rows] * z_final), the A operand of mnf_linear_forward_tc's mean
  * GEMM (pass z = NULL there and put xz_out at the start of its workspace).  workspace:

@@ -4,7 +4,8 @@
 // forward_mc lays them out.  Every output element is owned by one thread that walks s in order, in fp64 (the variance is
 // finished as E[y^2] - E[y]^2, which fp32 would lose to cancellation), so the sums do not depend on the launch geometry
 // and need no atomics.  A call forms its sums from zero and adds them to the buffer once: sums split at chunk boundaries
-// then add up to the same bits as one call over all samples.
+// then add up to the same bits as one call over all samples.  With softmax the kernel can also sum each sample row's
+// entropy H(softmax(y)) into entropy_sums[b] (mnf_mc_class_moments), under the same ordering and add-once rules.
 #include <math.h>
 
 #include "common.cuh"
@@ -29,11 +30,15 @@ __global__ void __launch_bounds__(256) mc_moments_kernel(const float *__restrict
 
 // softmax rows: one warp per (unique row b, block of kSoftmaxCols columns).  The row's max and normaliser come from a
 // lane-strided pass over all its columns and a butterfly reduction, which leaves the same bits in every lane; each lane
-// then accumulates its own kSoftmaxCols / 32 columns.
+// then accumulates its own kSoftmaxCols / 32 columns.  entropy_sums (nullable): the warp of column block 0 also forms
+//   H_s = log z - (1 / z) sum_c e_c (y_c - m),   e_c = expf(y_c - m),  z = sum_c e_c
+// in fp64 over all columns (terms with e_c == 0 skipped: 0 log 0 = 0, and a -inf column adds nothing), sums it over the
+// samples in order and adds it to entropy_sums[b] once.  The sums path is the same code with or without it.
 constexpr int kSoftmaxCols = 128;
 
 __global__ void __launch_bounds__(256) mc_moments_softmax_kernel(const float *__restrict__ y, long long n_unique,
-                                                                 long long n_samples, int n_cols, double *__restrict__ sums) {
+                                                                 long long n_samples, int n_cols, double *__restrict__ sums,
+                                                                 double *__restrict__ entropy_sums) {
     constexpr int CPL = kSoftmaxCols / 32;
     const int lane = threadIdx.x & 31;
     const int n_blk = (n_cols + kSoftmaxCols - 1) / kSoftmaxCols;
@@ -41,7 +46,8 @@ __global__ void __launch_bounds__(256) mc_moments_softmax_kernel(const float *__
     for (long long it = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5; it < n_items; it += warps) {
         const long long b = it / n_blk;
         const int c0 = (int)(it % n_blk) * kSoftmaxCols;
-        double s1[CPL], s2[CPL];
+        const bool entropy = entropy_sums != nullptr && c0 == 0;  // warp-uniform
+        double s1[CPL], s2[CPL], h = 0.0;
 #pragma unroll
         for (int k = 0; k < CPL; ++k) s1[k] = 0.0, s2[k] = 0.0;
         for (long long s = 0; s < n_samples; ++s) {
@@ -63,7 +69,18 @@ __global__ void __launch_bounds__(256) mc_moments_softmax_kernel(const float *__
                     s2[k] = fma(p, p, s2[k]);
                 }
             }
+            if (entropy) {
+                double t = 0.0;
+                for (int n = lane; n < n_cols; n += 32) {
+                    const float d = __ldg(row + n) - m, e = expf(d);
+                    if (e != 0.f) t = fma((double)e, (double)d, t);
+                }
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
+                h += log((double)z) - inv * t;
+            }
         }
+        if (entropy && lane == 0) entropy_sums[b] += h;
         const long long plane = n_unique * n_cols;
 #pragma unroll
         for (int k = 0; k < CPL; ++k) {
@@ -80,11 +97,10 @@ __global__ void __launch_bounds__(256) mc_moments_softmax_kernel(const float *__
 
 using namespace mnf;
 
-extern "C" {
+namespace {
 
-int mnf_mc_moments(const float *y, int64_t n_unique, int64_t n_samples, int n_cols, int softmax, double *sums,
-                   void *stream) {
-    MNF_REQUIRE(y && sums, MNF_E_ARG, "NULL pointer");
+int mc_moments(const float *y, int64_t n_unique, int64_t n_samples, int n_cols, int softmax, double *sums,
+               double *entropy_sums, void *stream) {
     MNF_REQUIRE(softmax == 0 || softmax == 1, MNF_E_ARG, "softmax must be 0 or 1 (got %d)", softmax);
     MNF_REQUIRE(n_unique >= 1 && n_samples >= 0 && n_cols >= 1, MNF_E_SHAPE,
                 "bad shape: n_unique=%lld n_samples=%lld n_cols=%d", (long long)n_unique, (long long)n_samples, n_cols);
@@ -98,13 +114,29 @@ int mnf_mc_moments(const float *y, int64_t n_unique, int64_t n_samples, int n_co
         const long long warps = n_unique * ((n_cols + kSoftmaxCols - 1) / kSoftmaxCols);
         long long blocks = (warps + 7) / 8;
         mc_moments_softmax_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, st>>>(y, n_unique, n_samples, n_cols,
-                                                                                             sums);
+                                                                                             sums, entropy_sums);
         return launch_status("mc_moments_softmax_kernel");
     }
     const long long n_elems = n_unique * n_cols;
     long long blocks = (n_elems + 255) / 256;
     mc_moments_kernel<<<(unsigned)(blocks < cap ? blocks : cap), 256, 0, st>>>(y, n_elems, n_samples, sums);
     return launch_status("mc_moments_kernel");
+}
+
+}  // namespace
+
+extern "C" {
+
+int mnf_mc_moments(const float *y, int64_t n_unique, int64_t n_samples, int n_cols, int softmax, double *sums,
+                   void *stream) {
+    MNF_REQUIRE(y && sums, MNF_E_ARG, "NULL pointer");
+    return mc_moments(y, n_unique, n_samples, n_cols, softmax, sums, nullptr, stream);
+}
+
+int mnf_mc_class_moments(const float *y, int64_t n_unique, int64_t n_samples, int n_cols, double *sums,
+                         double *entropy_sums, void *stream) {
+    MNF_REQUIRE(y && sums && entropy_sums, MNF_E_ARG, "NULL pointer");
+    return mc_moments(y, n_unique, n_samples, n_cols, 1, sums, entropy_sums, stream);
 }
 
 }  // extern "C"

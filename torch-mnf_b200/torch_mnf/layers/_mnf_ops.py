@@ -71,6 +71,7 @@ _lib.register({
     "mnf_linear_forward_tc_affine": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int,
                                             _int, _int, _vp, _vp, _vp, _vp]),
     "mnf_mc_moments": (_int, [_vp, _i64, _i64, _int, _int, _vp, _vp]),
+    "mnf_mc_class_moments": (_int, [_vp, _i64, _i64, _int, _vp, _vp, _vp]),
     "mnf_rnvp_tc_workspace": (_i64, [_int, _i64, _int]),
     "mnf_rnvp_forward_tc": (_int, [C.POINTER(RnvpFlow), _int, _vp, _vp, C.POINTER(C.c_void_p), _u64, _u32, _u64, _i64,
                                    _int, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _u32, _int, _vp]),
@@ -340,9 +341,10 @@ def linear_forward(layer, x, z, noise: Noise, x_rows=None, relu=False, precision
     return out
 
 
-def mc_moments(y, n_unique, n_samples, sums, softmax=False):
+def mc_moments(y, n_unique, n_samples, sums, softmax=False, entropy_sums=None):
     """sums [2, n_unique, n_cols] fp64 += (sum_s f(y), sum_s f(y)^2) over the samples of the sample-major y
-    [n_samples * n_unique, n_cols]; f = identity or a per-row softmax (mnf_mc_moments)."""
+    [n_samples * n_unique, n_cols]; f = identity or a per-row softmax (mnf_mc_moments).  entropy_sums [n_unique] fp64
+    (needs softmax): also += sum_s H(softmax(y[s * n_unique + b])), the per-sample entropies (mnf_mc_class_moments)."""
     dev = y.device
     n_cols = y.size(1)
     if y.shape != (n_samples * n_unique, n_cols) or sums.shape != (2, n_unique, n_cols):
@@ -350,11 +352,22 @@ def mc_moments(y, n_unique, n_samples, sums, softmax=False):
                          f"{n_samples} samples of {n_unique} rows")
     if sums.dtype != torch.float64 or not sums.is_contiguous() or sums.device != dev:
         raise ValueError("mc_moments: sums must be a contiguous float64 tensor on the device of y")
+    if entropy_sums is not None:
+        if not softmax:
+            raise ValueError("mc_moments: entropy_sums needs softmax=True (entropies of class probabilities)")
+        if (entropy_sums.shape != (n_unique,) or entropy_sums.dtype != torch.float64
+                or not entropy_sums.is_contiguous() or entropy_sums.device != dev):
+            raise ValueError(f"mc_moments: entropy_sums must be a contiguous float64 [{n_unique}] tensor on the device "
+                             f"of y (got {tuple(entropy_sums.shape)} {entropy_sums.dtype} on {entropy_sums.device})")
     y = _lib.require_cuda_f32(y, "y")
     with _lib.on_device(dev):
-        rc = _lib.lib().mnf_mc_moments(y.data_ptr(), n_unique, n_samples, n_cols, int(softmax), sums.data_ptr(),
-                                       _lib.stream_ptr(dev))
-    _lib.check(rc, "mnf_mc_moments")
+        if entropy_sums is None:
+            rc = _lib.lib().mnf_mc_moments(y.data_ptr(), n_unique, n_samples, n_cols, int(softmax), sums.data_ptr(),
+                                           _lib.stream_ptr(dev))
+        else:
+            rc = _lib.lib().mnf_mc_class_moments(y.data_ptr(), n_unique, n_samples, n_cols, sums.data_ptr(),
+                                                 entropy_sums.data_ptr(), _lib.stream_ptr(dev))
+    _lib.check(rc, "mnf_mc_moments" if entropy_sums is None else "mnf_mc_class_moments")
     _lib.launch_count += 1
     return sums
 

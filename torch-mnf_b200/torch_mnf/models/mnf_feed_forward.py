@@ -1,7 +1,7 @@
 """Feed-forward net of MNFLinear layers (reference: models/mnf_feed_forward.py:14-38)."""
 
 from collections.abc import Sequence
-from typing import Any
+from typing import Any, NamedTuple
 
 import torch
 from torch import nn
@@ -32,6 +32,46 @@ def moments_from_sums(sums: torch.Tensor, n_samples: int) -> tuple[torch.Tensor,
     mean = sums[0] / n_samples
     var = (sums[1] / n_samples - mean * mean).clamp_min_(0.0)
     return mean.float(), var.float()
+
+
+class MCUncertainty(NamedTuple):
+    """Monte-Carlo predictive uncertainty of a classifier over S samples p_s = softmax(model(x)) (natural log units):
+    ``mean``, ``var`` [B, C] fp32: mean and population variance of the class probabilities;
+    ``predictive_entropy`` [B]: H[p_bar], the total uncertainty;
+    ``expected_entropy`` [B]: E_s H[p_s], the aleatoric part;
+    ``mutual_information`` [B]: H[p_bar] - E_s H[p_s] (BALD), the epistemic part."""
+
+    mean: torch.Tensor
+    var: torch.Tensor
+    predictive_entropy: torch.Tensor
+    expected_entropy: torch.Tensor
+    mutual_information: torch.Tensor
+
+
+def check_mc_args(n_samples: int, chunk: int | None, sample_range) -> tuple[int, int]:
+    """(lo, hi) of a Monte-Carlo prediction's samples; ValueError for n_samples < 1, chunk < 1 or a sample_range
+    outside [0, n_samples] -- before any device work."""
+    if n_samples < 1:
+        raise ValueError(f"n_samples must be positive, got {n_samples}")
+    if chunk is not None and chunk < 1:
+        raise ValueError(f"chunk must be positive, got {chunk}")
+    lo, hi = (0, n_samples) if sample_range is None else sample_range
+    if not 0 <= lo <= hi <= n_samples:
+        raise ValueError(f"sample_range {sample_range} outside [0, {n_samples}]")
+    return lo, hi
+
+
+def uncertainty_from_sums(sums: torch.Tensor, entropy_sums: torch.Tensor, n_samples: int) -> MCUncertainty:
+    """MCUncertainty from the fp64 probability sums [2, B, C] and entropy sums [B] of ``predict_uncertainty(...,
+    sample_range=...)`` (all ranks' shares added).  mean / var as moments_from_sums; H[p_bar] = -sum_c p_bar log p_bar in
+    fp64 with 0 log 0 = 0; E_s H[p_s] = entropy_sums / S; the mutual information is clamped at 0 (rounding can leave a
+    tiny negative value where all samples agree)."""
+    mean, var = moments_from_sums(sums, n_samples)
+    p_bar = sums[0] / n_samples
+    predictive = -torch.special.xlogy(p_bar, p_bar).sum(-1)
+    expected = entropy_sums / n_samples
+    mutual = (predictive - expected).clamp_min_(0.0)
+    return MCUncertainty(mean, var, predictive.float(), expected.float(), mutual.float())
 
 
 class MNFFeedForward(nn.Sequential):
@@ -129,6 +169,28 @@ class MNFFeedForward(nn.Sequential):
 
         Needs every BatchNorm1d in eval mode with running statistics: batch statistics of a chunk are not those of the
         whole replicated batch."""
+        sums, _ = self._mc_sums(x, n_samples, chunk, seed, sample_range, softmax, entropy=False)
+        if sample_range is not None:
+            return sums
+        return moments_from_sums(sums, n_samples)
+
+    @torch.no_grad()
+    def predict_uncertainty(self, x, n_samples: int = 500, chunk: int | None = None, seed=None, sample_range=None):
+        """Monte-Carlo predictive uncertainty of the classifier ``softmax(model(x))``: an MCUncertainty with the mean and
+        variance of the class probabilities (the bits of ``predict(..., softmax=True)`` for the same seed and chunk) and
+        the predictive entropy, expected entropy and mutual information per input.  Same chunking, draws and batch-norm
+        requirement as ``predict``; each chunk's per-sample entropies are summed in fp64 on the device in the same pass
+        as the probabilities (mnf_mc_class_moments).  ``sample_range=(lo, hi)``: the raw ``(sums [2, B, C],
+        entropy_sums [B])`` of samples lo..hi-1; all-reduce both and finish with ``uncertainty_from_sums``."""
+        check_mc_args(n_samples, chunk, sample_range)
+        sums, entropy_sums = self._mc_sums(x, n_samples, chunk, seed, sample_range, True, entropy=True)
+        if sample_range is not None:
+            return sums, entropy_sums
+        return uncertainty_from_sums(sums, entropy_sums, n_samples)
+
+    def _mc_sums(self, x, n_samples, chunk, seed, sample_range, softmax, entropy):
+        """The chunk loop of predict / predict_uncertainty: fp64 sums [2, B, n_out] and, with ``entropy``, the entropy
+        sums [B] (else None) of samples lo..hi-1."""
         for m in self:
             if isinstance(m, nn.modules.batchnorm._BatchNorm) and not self._uses_running_stats(m):
                 raise RuntimeError("MNFFeedForward.predict needs every BatchNorm1d in eval mode with running statistics "
@@ -148,10 +210,9 @@ class MNFFeedForward(nn.Sequential):
             seed = int(torch.randint(0, 2**62, (1,)).item())  # follows torch.manual_seed
         n_out = self._blocks()[-1][0].n_out
         sums = torch.zeros((2, B, n_out), device=x.device, dtype=torch.float64)
+        entropy_sums = torch.zeros(B, device=x.device, dtype=torch.float64) if entropy else None
         for c in range(lo, hi, chunk):
             s_here = min(chunk, hi - c)
             y = self.forward_mc(x, s_here, seed=seed, row_offset=c * B)
-            ops.mc_moments(y, B, s_here, sums, softmax=softmax)
-        if sample_range is not None:
-            return sums
-        return moments_from_sums(sums, n_samples)
+            ops.mc_moments(y, B, s_here, sums, softmax=softmax, entropy_sums=entropy_sums)
+        return sums, entropy_sums

@@ -9,6 +9,7 @@ from .. import _lib
 from ..layers import MNFConv2d, MNFLinear
 from ..layers import _mnf_ops as ops
 from ..layers import _train
+from .mnf_feed_forward import check_mc_args, uncertainty_from_sums
 
 
 class MNFLeNet(nn.Sequential):
@@ -68,7 +69,8 @@ class MNFLeNet(nn.Sequential):
         h = self[9].forward(h, nz, precision=prec)
         return torch.log_softmax(h, dim=-1)
 
-    def _forward_per_sample_z(self, x, noise, S, row_offset, seed):
+    def _forward_per_sample_z(self, x, noise, S, row_offset, seed, conv1=None):
+        """conv1: conv_moments(self[0], x, None) when the caller already has them (they do not depend on the sample)."""
         B = x.size(0)
         R = B * S
         if row_offset % B:
@@ -77,7 +79,8 @@ class MNFLeNet(nn.Sequential):
         s0 = row_offset // B  # global index of this shard's first Monte-Carlo sample
         # conv1: moments once per image with unit z (exact fp32), z[s, c] scales the mean in the noise / pool pass
         z1 = ops.conv_sample_z_rows(self[0], S, nz, s0)
-        h = ops.conv_mc_relu_pool(self[0], x, None, nz, R, z_rows=z1, rows_per_z=B)
+        mean1, sd1 = conv1 if conv1 is not None else ops.conv_moments(self[0], x, None)
+        h = ops.conv_noise_relu_pool(mean1, sd1, nz, R, z_rows=z1, rows_per_z=B)
         z2 = ops.conv_sample_z_rows(self[3], S, nz, s0)
         if self.precision != "fp32":
             h = ops.conv_forward_tc(self[3], h, None, nz, z_rows=z2, rows_per_z=B)
@@ -113,11 +116,53 @@ class MNFLeNet(nn.Sequential):
         if seed is None:
             seed = int(torch.randint(0, 2**62, (1,)).item())  # follows torch.manual_seed
         sums = torch.zeros(B, 10, device=x.device, dtype=torch.float32)
+        for s_here, log_probs in self._mc_log_probs(x, chunk, seed, lo, hi):
+            sums += log_probs.exp().view(s_here, B, 10).sum(0)
+        return sums if sample_range is not None else sums / n_samples
+
+    @torch.no_grad()
+    def predict_uncertainty(self, x, n_samples: int = 500, chunk: int = 25, seed=None, sample_range=None,
+                            per_sample_conv_z: bool = False):
+        """Monte-Carlo predictive uncertainty: an MCUncertainty with the mean and variance of the class probabilities
+        ``[B, 10]`` and, per image, the predictive entropy H[p_bar] (total), the expected entropy E_s H[p_s] (aleatoric)
+        and their difference, the mutual information (epistemic; BALD).  The samples and draws are ``predict``'s; each
+        chunk's log-probabilities are reduced on the device into fp64 sums of the probabilities, their squares and the
+        per-sample entropies (mnf_mc_class_moments), so ``mean`` agrees with ``predict`` to fp32 rounding and the result
+        does not depend on ``chunk`` beyond fp64 rounding.  ``sample_range=(lo, hi)``: the raw ``(sums [2, B, 10],
+        entropy_sums [B])`` of samples lo..hi-1; all-reduce both and finish with ``uncertainty_from_sums``.
+
+        ``per_sample_conv_z``: every sample draws its own conv z, as ``forward(..., per_sample_conv_z=True)`` does chunk
+        by chunk (bit for bit).  ``predict``'s single z per conv layer leaves the conv layers' multiplicative posterior
+        out of the spread across samples, so the mutual information undercounts their epistemic part; this mode
+        includes it, at the cost of one z draw per sample."""
+        lo, hi = check_mc_args(n_samples, chunk, sample_range)
+        x = _lib.require_cuda_f32(x, "input")
+        B = x.size(0)
+        if seed is None:
+            seed = int(torch.randint(0, 2**62, (1,)).item())  # follows torch.manual_seed
+        sums = torch.zeros((2, B, 10), device=x.device, dtype=torch.float64)
+        entropy_sums = torch.zeros(B, device=x.device, dtype=torch.float64)
+        for s_here, log_probs in self._mc_log_probs(x, chunk, seed, lo, hi, per_sample_conv_z):
+            ops.mc_moments(log_probs, B, s_here, sums, softmax=True, entropy_sums=entropy_sums)
+        if sample_range is not None:
+            return sums, entropy_sums
+        return uncertainty_from_sums(sums, entropy_sums, n_samples)
+
+    def _mc_log_probs(self, x, chunk, seed, lo, hi, per_sample_conv_z=False):
+        """Yields (s_here, log-probabilities [s_here * B, 10]) chunk by chunk for samples lo..hi-1: the draws of
+        ``forward(x, n_samples=s_here, seed=seed, row_offset=c * B, per_sample_conv_z=...)`` per chunk c."""
+        B = x.size(0)
+        if per_sample_conv_z:  # conv1's unit-z moments do not depend on the sample: once per prediction
+            conv1 = ops.conv_moments(self[0], x, None)
+            for c in range(lo, hi, chunk):
+                s_here = min(chunk, hi - c)
+                yield s_here, self._forward_per_sample_z(x, None, s_here, c * B, seed, conv1=conv1)
+            return
         if self.precision == "fp32" or B * min(chunk, max(hi - lo, 1)) < self.TC_MIN_ROWS:
             for c in range(lo, hi, chunk):  # exact-fp32 pipeline: nothing sample-independent to share across chunks
                 s_here = min(chunk, hi - c)
-                sums += self.forward(x, n_samples=s_here, seed=seed, row_offset=c * B).exp().view(s_here, B, 10).sum(0)
-            return sums if sample_range is not None else sums / n_samples
+                yield s_here, self.forward(x, n_samples=s_here, seed=seed, row_offset=c * B)
+            return
         # the call's two conv z draws (row offset 0 on every rank) and conv1's moments: once
         nz0 = ops.Noise(None, x.device, 0, seed=seed)
         z1, _ = self[0].sample_z(nz0)
@@ -135,8 +180,7 @@ class MNFLeNet(nn.Sequential):
             h = ops.conv_forward_tc(self[3], h, z2, nz)
             h = self[7].forward(h.view(R, -1), nz, relu=True)
             h = self[9].forward(h, nz)
-            sums += torch.log_softmax(h, dim=-1).exp().view(s_here, B, 10).sum(0)
-        return sums if sample_range is not None else sums / n_samples
+            yield s_here, torch.log_softmax(h, dim=-1)
 
     def kl_div(self, noise=None):
         """Sum of the MNF layers' KL estimates (mnf_lenet.py:28-32).  Without an injected tape and outside autograd the
