@@ -396,6 +396,16 @@ int mnf_conv2d_forward(const float *x, int64_t x_imgs, const float *z, const flo
                        const float *W_log_var, const float *b_log_var, const float *eps, uint64_t seed,
                        uint32_t noise_stream, uint64_t row_offset, float *out, int64_t n_imgs, int c_in,
                        int height, int width, int c_out, int ksize, int relu_pool, void *stream);
+/* The same with zero padding pad >= 0 and stride >= 1, as torch.nn.functional.conv2d(..., padding=pad, stride=stride):
+ *   OH = (height + 2 pad - ksize) / stride + 1, OW likewise (both must be >= 1; relu_pool needs them even).
+ * Output pixel (oy, ox) reads the window at (oy*stride - pad, ox*stride - pad); taps in the padding add nothing to the
+ * mean or the variance.  eps is [n_imgs, c_out, OH, OW] with the Philox numbering of mnf_conv2d_forward, which is
+ * this call with pad = 0, stride = 1. */
+int mnf_conv2d_forward_ps(const float *x, int64_t x_imgs, const float *z, const float *W_mean,
+                          const float *W_log_var, const float *b_log_var, const float *eps, uint64_t seed,
+                          uint32_t noise_stream, uint64_t row_offset, float *out, int64_t n_imgs, int c_in,
+                          int height, int width, int c_out, int ksize, int relu_pool, int pad, int stride,
+                          void *stream);
 
 /* Pieces of the MNF-LeNet Monte-Carlo pipeline (models/mnf_lenet.py:13-26 driven as in mnf_mnist.ipynb:316-318).
  * mnf_conv2d_moments: the sample-independent mean and standard deviation of an MNFConv2d (z is shared by the
@@ -409,6 +419,11 @@ int mnf_conv2d_forward(const float *x, int64_t x_imgs, const float *z, const flo
 int mnf_conv2d_moments(const float *x, const float *z, const float *W_mean, const float *W_log_var,
                        const float *b_log_var, float *mean_out, float *sd_out, int64_t n_imgs, int c_in,
                        int height, int width, int c_out, int ksize, void *stream);
+/* mnf_conv2d_moments with zero padding and stride (geometry as for mnf_conv2d_forward_ps; pad = 0, stride = 1 is
+ * mnf_conv2d_moments). */
+int mnf_conv2d_moments_ps(const float *x, const float *z, const float *W_mean, const float *W_log_var,
+                          const float *b_log_var, float *mean_out, float *sd_out, int64_t n_imgs, int c_in,
+                          int height, int width, int c_out, int ksize, int pad, int stride, void *stream);
 int mnf_conv_noise_relu_pool(const float *mean, const float *sd, int64_t n_unique, const float *eps,
                              uint64_t seed, uint32_t noise_stream, uint64_t row_offset, float *out,
                              int64_t n_rows, int channels, int out_h, int out_w, void *stream);
@@ -515,12 +530,20 @@ int mnf_ew(int op, const float *a, const float *b, const float *c, const float *
 /* out[n] = sum_r a[r,n] * (b ? b[r,n] : 1) */
 int mnf_colsum(const float *a, const float *b, int64_t n_rows, int n_cols, float *out, void *stream);
 
-/* MNFConv2d as GEMM (mnf_conv.py:68-79; stride 1, no padding).  cols_t[(ci,kh,kw)][(r,oh,ow)] = x[r,ci,oh+kh,ow+kw], so
- * conv(x, W)[c_out, (r,oh,ow)] = W[c_out, fan] cols_t; mnf_col2im_t is the adjoint (d loss / d x from d loss / d cols_t);
+/* MNFConv2d as GEMM (mnf_conv.py:68-79; these two: stride 1, no padding).  cols_t[(ci,kh,kw)][(r,oh,ow)] =
+ * x[r,ci,oh+kh,ow+kw], so conv(x, W)[c_out, (r,oh,ow)] = W[c_out, fan] cols_t; mnf_col2im_t is the adjoint (d loss / d x from d loss / d cols_t);
  * mnf_swap01 turns [dim0, dim1, inner] into [dim1, dim0, inner] (GEMM layout <-> NCHW); mnf_rowsum: out[r] = sum_c a[r,c]. */
 int mnf_im2col_t(const float *x, float *cols_t, int64_t n_imgs, int c_in, int height, int width, int ksize, void *stream);
 int mnf_col2im_t(const float *grad_cols_t, float *grad_x, int64_t n_imgs, int c_in, int height, int width, int ksize,
                  void *stream);
+/* The same with zero padding pad >= 0 and stride >= 1 (OH = (height + 2 pad - ksize) / stride + 1, OW likewise):
+ * cols_t[(ci,kh,kw)][(r,oh,ow)] = x[r, ci, oh*stride - pad + kh, ow*stride - pad + kw], 0 where that lies in the padding.
+ * mnf_col2im_t_ps is its exact adjoint: entries of overlapping windows (stride < ksize) add up at their input pixel,
+ * entries in the padding are dropped.  pad = 0, stride = 1 is mnf_im2col_t / mnf_col2im_t. */
+int mnf_im2col_t_ps(const float *x, float *cols_t, int64_t n_imgs, int c_in, int height, int width, int ksize, int pad,
+                    int stride, void *stream);
+int mnf_col2im_t_ps(const float *grad_cols_t, float *grad_x, int64_t n_imgs, int c_in, int height, int width, int ksize,
+                    int pad, int stride, void *stream);
 int mnf_swap01(const float *in, float *out, int64_t dim0, int64_t dim1, int64_t inner, void *stream);
 int mnf_rowsum(const float *a, int64_t n_rows, int64_t n_cols, float *out, void *stream);
 

@@ -9,6 +9,8 @@
 
 #include <cuda_fp16.h>
 
+#include <type_traits>
+
 #include "mnf_common.cuh"
 
 namespace mnf {
@@ -176,6 +178,10 @@ struct MnfLinearProb {
 // K = n_in*k*k.  With `pool` the row index is pool-major (4 consecutive rows = one 2x2 window)
 // and the epilogue applies ReLU + max over the window (the nn.ReLU / nn.MaxPool2d(2) that
 // follow every MNFConv2d in MNFLeNet, mnf_lenet.py:16-21).
+// GEOM: zero padding `pad` and stride `stride`.  Output pixel (oy, ox) reads the window whose origin is
+// (oy*stride - pad, ox*stride - pad); a tap outside the image loads 0, so it adds to neither moment.  Without GEOM
+// (pad 0, stride 1) every tap is inside the image and the loads carry no bounds test.
+template <bool GEOM>
 struct MnfConvProb {
     int M, N, K;
     const float *x;  // [R, C, H, W]
@@ -206,19 +212,44 @@ struct MnfConvProb {
     // (the table travels as a kernel parameter); wider filters compute the remaining offsets arithmetically
     static constexpr int kMaxTaps = 1600;
     int koff[kMaxTaps];
+    int pad, stride;                 // GEOM only
+    int kyx[GEOM ? kMaxTaps : 1];    // GEOM: (ky << 16) | kx of tap k, for the bounds test
     __device__ __forceinline__ int tap_offset(int k) const {
         if (k < kMaxTaps) return koff[k];
         const int kx = k % ks, ky = (k / ks) % ks, ci = k / (ks * ks);
         return (ci * H + ky) * W + kx;
     }
-    using RowCtx = size_t;  // offset of the output pixel's receptive-field origin in x
+    // GEOM: offset of the receptive-field origin in x (negative or past a row when it lies in the padding) and
+    // the origin's coordinates; otherwise the offset alone
+    struct GeomRow {
+        long long o;
+        int iy, ix;
+    };
+    using RowCtx = std::conditional_t<GEOM, GeomRow, size_t>;
     __device__ RowCtx row_ctx(int m) const {
         int r, oy, ox;
         decode(m, r, oy, ox);
-        return ((size_t)(r % x_imgs) * C * H + oy) * W + ox;
+        if constexpr (GEOM) {
+            const int iy = oy * stride - pad, ix = ox * stride - pad;
+            return GeomRow{((long long)(r % x_imgs) * C * H + iy) * W + ix, iy, ix};
+        } else {
+            return ((size_t)(r % x_imgs) * C * H + oy) * W + ox;
+        }
     }
     __device__ void load_a(const RowCtx &r, int, int k, float (&a)[2]) const {
-        const float xv = x[r + tap_offset(k)];
+        float xv;
+        if constexpr (GEOM) {
+            int ky, kx;
+            if (k < kMaxTaps) {
+                ky = kyx[k] >> 16, kx = kyx[k] & 0xffff;
+            } else {
+                kx = k % ks, ky = (k / ks) % ks;
+            }
+            const bool in = (unsigned)(r.iy + ky) < (unsigned)H && (unsigned)(r.ix + kx) < (unsigned)W;
+            xv = in ? x[r.o + tap_offset(k)] : 0.f;
+        } else {
+            xv = x[r + tap_offset(k)];
+        }
         a[0] = xv;
         a[1] = xv * xv;
     }
@@ -536,6 +567,22 @@ static int launch_conv_moments_direct(const float *x, const float *z, const floa
     return launch_status("conv_moments_direct_kernel");
 }
 
+// the implicit-GEMM conv of mnf_conv2d_forward_ps / mnf_conv2d_moments_ps: tabulates the tap offsets (and, with
+// GEOM, the tap coordinates) on the host and launches the SIMT GEMM.  sd_out != NULL: moments mode.
+template <bool GEOM>
+static int run_conv_gemm(const float *x, int x_imgs, const float *z, const float *Wm, const float *Wlv, const float *blv,
+                         float *out, float *sd_out, NoiseSrc eps, int pool, long long M, int C, int H, int W, int ks,
+                         int N, int OH, int OW, int pad, int stride, cudaStream_t st, const char *what) {
+    MnfConvProb<GEOM> p{(int)M, N, C * ks * ks, x, x_imgs, C, H, W, ks, OH, OW, Wm, Wlv, blv, z, out, eps, pool, sd_out,
+                        {}, pad, stride, {}};
+    for (int k = 0; k < p.K && k < MnfConvProb<GEOM>::kMaxTaps; ++k) {
+        const int kx = k % ks, ky = (k / ks) % ks, ci = k / (ks * ks);
+        p.koff[k] = (ci * H + ky) * W + kx;
+        if constexpr (GEOM) p.kyx[k] = (ky << 16) | kx;
+    }
+    return launch_simt_gemm<MnfConvProb<GEOM>, 2>(p, st, what);
+}
+
 int conv_pack_weights_f16(const float *z, const float *W_mean, const float *W_log_var, const float *b_log_var, void *Bm,
                           void *Bv, float *bvar_p, int K, int c_out, int Np, int Kp, void *stream) {
     MNF_REQUIRE(W_mean && W_log_var && b_log_var && Bm && Bv && bvar_p, MNF_E_ARG, "NULL pointer");
@@ -555,26 +602,37 @@ extern "C" {
 int mnf_conv2d_moments(const float *x, const float *z, const float *W_mean, const float *W_log_var,
                        const float *b_log_var, float *mean_out, float *sd_out, int64_t n_imgs, int c_in, int height,
                        int width, int c_out, int ksize, void *stream) {
+    return mnf_conv2d_moments_ps(x, z, W_mean, W_log_var, b_log_var, mean_out, sd_out, n_imgs, c_in, height, width, c_out,
+                                 ksize, 0, 1, stream);
+}
+
+// the same with zero padding `pad` and stride `stride` (OH = (H + 2 pad - k) / stride + 1).  Only pad 0 / stride 1
+// takes the direct kernel; every other geometry runs the implicit GEMM with bounds-tested tap loads.
+int mnf_conv2d_moments_ps(const float *x, const float *z, const float *W_mean, const float *W_log_var,
+                          const float *b_log_var, float *mean_out, float *sd_out, int64_t n_imgs, int c_in, int height,
+                          int width, int c_out, int ksize, int pad, int stride, void *stream) {
     MNF_REQUIRE(x && W_mean && W_log_var && b_log_var && mean_out && sd_out, MNF_E_ARG, "NULL pointer");  // z may be NULL (= 1)
-    const int OH = height - ksize + 1, OW = width - ksize + 1;
+    MNF_REQUIRE(pad >= 0 && pad <= 0xffff && stride >= 1, MNF_E_ARG, "bad padding %d or stride %d", pad, stride);
+    const int OH = conv_out_size(height, ksize, pad, stride), OW = conv_out_size(width, ksize, pad, stride);
     MNF_REQUIRE(n_imgs >= 0 && OH >= 1 && OW >= 1, MNF_E_SHAPE, "bad shape");
     const long long M = (long long)n_imgs * OH * OW;
     MNF_REQUIRE(M <= 0x7fffffff - 64, MNF_E_SHAPE, "too many output pixels for one call (%lld)", M);
     if (n_imgs == 0) return 0;
-    if (c_in * ksize * ksize <= 64 && c_out <= 32 && c_in * height * width <= 4096) {  // few taps, few channels: direct form
+    const bool geom = pad != 0 || stride != 1;
+    if (!geom && c_in * ksize * ksize <= 64 && c_out <= 32 && c_in * height * width <= 4096) {  // few taps, few channels: direct form
         if (c_out <= 20)
             return launch_conv_moments_direct<20>(x, z, W_mean, W_log_var, b_log_var, mean_out, sd_out, n_imgs, c_in, height,
                                                   width, ksize, c_out, (cudaStream_t)stream);
         return launch_conv_moments_direct<32>(x, z, W_mean, W_log_var, b_log_var, mean_out, sd_out, n_imgs, c_in, height, width,
                                               ksize, c_out, (cudaStream_t)stream);
     }
-    MnfConvProb p{(int)M, c_out, c_in * ksize * ksize, x, (int)(n_imgs > 0 ? n_imgs : 1), c_in, height, width, ksize,
-                  OH, OW, W_mean, W_log_var, b_log_var, z, mean_out, NoiseSrc{nullptr, 0, 0, 0}, 0, sd_out, {}};
-    for (int k = 0; k < p.K && k < MnfConvProb::kMaxTaps; ++k) {
-        const int kx = k % ksize, ky = (k / ksize) % ksize, ci = k / (ksize * ksize);
-        p.koff[k] = (ci * height + ky) * width + kx;
-    }
-    return launch_simt_gemm<MnfConvProb, 2>(p, (cudaStream_t)stream, "mnf_conv2d_moments");
+    const NoiseSrc none{nullptr, 0, 0, 0};
+    const int x_imgs = (int)(n_imgs > 0 ? n_imgs : 1);
+    if (geom)
+        return run_conv_gemm<true>(x, x_imgs, z, W_mean, W_log_var, b_log_var, mean_out, sd_out, none, 0, M, c_in, height,
+                                   width, ksize, c_out, OH, OW, pad, stride, (cudaStream_t)stream, "mnf_conv2d_moments");
+    return run_conv_gemm<false>(x, x_imgs, z, W_mean, W_log_var, b_log_var, mean_out, sd_out, none, 0, M, c_in, height,
+                                width, ksize, c_out, OH, OW, 0, 1, (cudaStream_t)stream, "mnf_conv2d_moments");
 }
 
 // out[r] = maxpool2(relu(mean[r % n_unique] + sd[r % n_unique] * eps[r])) -- the per-sample tail of an MNFConv2d
@@ -726,22 +784,30 @@ int mnf_conv2d_forward(const float *x, int64_t x_imgs, const float *z, const flo
                        const float *b_log_var, const float *eps, uint64_t seed, uint32_t noise_stream,
                        uint64_t row_offset, float *out, int64_t n_imgs, int c_in, int height, int width, int c_out,
                        int ksize, int relu_pool, void *stream) {
+    return mnf_conv2d_forward_ps(x, x_imgs, z, W_mean, W_log_var, b_log_var, eps, seed, noise_stream, row_offset, out,
+                                 n_imgs, c_in, height, width, c_out, ksize, relu_pool, 0, 1, stream);
+}
+
+int mnf_conv2d_forward_ps(const float *x, int64_t x_imgs, const float *z, const float *W_mean, const float *W_log_var,
+                          const float *b_log_var, const float *eps, uint64_t seed, uint32_t noise_stream,
+                          uint64_t row_offset, float *out, int64_t n_imgs, int c_in, int height, int width, int c_out,
+                          int ksize, int relu_pool, int pad, int stride, void *stream) {
     MNF_REQUIRE(x && z && W_mean && W_log_var && b_log_var && out, MNF_E_ARG, "NULL pointer");
     MNF_REQUIRE(n_imgs >= 0 && c_in >= 1 && c_out >= 1 && ksize >= 1 && x_imgs >= 1, MNF_E_ARG, "bad shape");
-    const int OH = height - ksize + 1, OW = width - ksize + 1;
-    MNF_REQUIRE(OH >= 1 && OW >= 1, MNF_E_SHAPE, "kernel %d larger than input %dx%d", ksize, height, width);
+    MNF_REQUIRE(pad >= 0 && pad <= 0xffff && stride >= 1, MNF_E_ARG, "bad padding %d or stride %d", pad, stride);
+    const int OH = conv_out_size(height, ksize, pad, stride), OW = conv_out_size(width, ksize, pad, stride);
+    MNF_REQUIRE(OH >= 1 && OW >= 1, MNF_E_SHAPE, "kernel %d larger than input %dx%d padded by %d", ksize, height, width, pad);
     MNF_REQUIRE(!relu_pool || (OH % 2 == 0 && OW % 2 == 0), MNF_E_SHAPE,
                 "fused 2x2 max-pool needs even output size, got %dx%d", OH, OW);
     const long long M = (long long)n_imgs * OH * OW;
     MNF_REQUIRE(M <= 0x7fffffff - 64, MNF_E_SHAPE, "too many output pixels for one call (%lld): chunk the batch", M);
-    MnfConvProb p{(int)M, c_out, c_in * ksize * ksize, x, (int)x_imgs, c_in, height, width, ksize, OH, OW,
-                  W_mean, W_log_var, b_log_var, z, out, NoiseSrc{eps, seed, noise_stream, row_offset}, relu_pool,
-                  nullptr, {}};
-    for (int k = 0; k < p.K && k < MnfConvProb::kMaxTaps; ++k) {
-        const int kx = k % ksize, ky = (k / ksize) % ksize, ci = k / (ksize * ksize);
-        p.koff[k] = (ci * height + ky) * width + kx;
-    }
-    return launch_simt_gemm<MnfConvProb, 2>(p, (cudaStream_t)stream, "mnf_conv2d_forward");
+    const NoiseSrc src{eps, seed, noise_stream, row_offset};
+    if (pad != 0 || stride != 1)
+        return run_conv_gemm<true>(x, (int)x_imgs, z, W_mean, W_log_var, b_log_var, out, nullptr, src, relu_pool, M, c_in,
+                                   height, width, ksize, c_out, OH, OW, pad, stride, (cudaStream_t)stream,
+                                   "mnf_conv2d_forward");
+    return run_conv_gemm<false>(x, (int)x_imgs, z, W_mean, W_log_var, b_log_var, out, nullptr, src, relu_pool, M, c_in,
+                                height, width, ksize, c_out, OH, OW, 0, 1, (cudaStream_t)stream, "mnf_conv2d_forward");
 }
 
 }  // extern "C"

@@ -195,37 +195,42 @@ __global__ void kl_rows_bwd_kernel(const float *__restrict__ z, const float *__r
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// convolution as GEMM (stride 1, no padding): transposed im2col  colsT[(ci,kh,kw)][(r,oh,ow)] = x[r,ci,oh+kh,ow+kw],
-// its adjoint (gather form, no atomics), and the [A,B,inner] -> [B,A,inner] layout swap between the GEMM's
-// [c_out, R*OH*OW] and the module's [R, c_out, OH, OW]
+// convolution as GEMM with zero padding `pad` and stride `st`: transposed im2col
+// colsT[(ci,kh,kw)][(r,oh,ow)] = x[r, ci, oh*st - pad + kh, ow*st - pad + kw] (0 in the padding), its adjoint (gather
+// form, no atomics), and the [A,B,inner] -> [B,A,inner] layout swap between the GEMM's [c_out, R*OH*OW] and the
+// module's [R, c_out, OH, OW].  With pad 0 and stride 1 every bounds test passes and the adjoint sums the same terms
+// in the same order as the unpadded form.
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void im2col_t_kernel(const float *__restrict__ x, float *__restrict__ colsT, long long R, int c_in, int H,
-                                int W, int ks) {
-    const int OH = H - ks + 1, OW = W - ks + 1;
+                                int W, int ks, int pad, int st) {
+    const int OH = conv_out_size(H, ks, pad, st), OW = conv_out_size(W, ks, pad, st);
     const long long P = R * OH * OW, total = (long long)c_in * ks * ks * P;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const long long p = i % P;
         const int f = (int)(i / P), kw = f % ks, kh = (f / ks) % ks, ci = f / (ks * ks);
         const int ow = (int)(p % OW), oh = (int)((p / OW) % OH);
         const long long r = p / ((long long)OW * OH);
-        colsT[i] = x[((r * c_in + ci) * H + oh + kh) * W + ow + kw];
+        const int ih = oh * st - pad + kh, iw = ow * st - pad + kw;
+        colsT[i] = ((unsigned)ih < (unsigned)H && (unsigned)iw < (unsigned)W) ? x[((r * c_in + ci) * H + ih) * W + iw] : 0.f;
     }
 }
 
 __global__ void col2im_t_kernel(const float *__restrict__ g_colsT, float *__restrict__ gx, long long R, int c_in, int H,
-                                int W, int ks) {
-    const int OH = H - ks + 1, OW = W - ks + 1;
+                                int W, int ks, int pad, int st) {
+    const int OH = conv_out_size(H, ks, pad, st), OW = conv_out_size(W, ks, pad, st);
     const long long P = R * OH * OW, total = R * c_in * H * W;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const int w = (int)(i % W), h = (int)((i / W) % H), ci = (int)((i / ((long long)W * H)) % c_in);
         const long long r = i / ((long long)W * H * c_in);
         float acc = 0.f;
         for (int kh = 0; kh < ks; ++kh) {
-            const int oh = h - kh;
-            if (oh < 0 || oh >= OH) continue;
+            const int th = h + pad - kh;  // oh * st when input row h is tap row kh of output row oh
+            if (th < 0 || th % st != 0 || th / st >= OH) continue;
+            const int oh = th / st;
             for (int kw = 0; kw < ks; ++kw) {
-                const int ow = w - kw;
-                if (ow < 0 || ow >= OW) continue;
+                const int tw = w + pad - kw;
+                if (tw < 0 || tw % st != 0 || tw / st >= OW) continue;
+                const int ow = tw / st;
                 acc += g_colsT[(long long)((ci * ks + kh) * ks + kw) * P + (r * OH + oh) * OW + ow];
             }
         }
@@ -301,21 +306,38 @@ int mnf_colsum(const float *a, const float *b, int64_t R, int N, float *out, voi
 }
 
 int mnf_im2col_t(const float *x, float *cols_t, int64_t n_imgs, int c_in, int height, int width, int ksize, void *stream) {
+    return mnf_im2col_t_ps(x, cols_t, n_imgs, c_in, height, width, ksize, 0, 1, stream);
+}
+
+int mnf_im2col_t_ps(const float *x, float *cols_t, int64_t n_imgs, int c_in, int height, int width, int ksize, int pad,
+                    int stride, void *stream) {
     MNF_REQUIRE(x && cols_t, MNF_E_ARG, "NULL pointer");
-    MNF_REQUIRE(ksize >= 1 && ksize <= height && ksize <= width, MNF_E_SHAPE, "kernel larger than the image");
-    const long long total = (long long)c_in * ksize * ksize * n_imgs * (height - ksize + 1) * (width - ksize + 1);
+    MNF_REQUIRE(pad >= 0 && stride >= 1, MNF_E_ARG, "bad padding %d or stride %d", pad, stride);
+    MNF_REQUIRE(ksize >= 1 && ksize <= height + 2 * pad && ksize <= width + 2 * pad, MNF_E_SHAPE,
+                "kernel larger than the padded image");
+    const long long total = (long long)c_in * ksize * ksize * n_imgs * conv_out_size(height, ksize, pad, stride) *
+                            conv_out_size(width, ksize, pad, stride);
     if (total == 0) return 0;
-    im2col_t_kernel<<<ew_blocks(total), 256, 0, (cudaStream_t)stream>>>(x, cols_t, n_imgs, c_in, height, width, ksize);
+    im2col_t_kernel<<<ew_blocks(total), 256, 0, (cudaStream_t)stream>>>(x, cols_t, n_imgs, c_in, height, width, ksize, pad,
+                                                                        stride);
     return launch_status("im2col_t_kernel");
 }
 
 int mnf_col2im_t(const float *grad_cols_t, float *grad_x, int64_t n_imgs, int c_in, int height, int width, int ksize,
                  void *stream) {
+    return mnf_col2im_t_ps(grad_cols_t, grad_x, n_imgs, c_in, height, width, ksize, 0, 1, stream);
+}
+
+int mnf_col2im_t_ps(const float *grad_cols_t, float *grad_x, int64_t n_imgs, int c_in, int height, int width, int ksize,
+                    int pad, int stride, void *stream) {
     MNF_REQUIRE(grad_cols_t && grad_x, MNF_E_ARG, "NULL pointer");
-    MNF_REQUIRE(ksize >= 1 && ksize <= height && ksize <= width, MNF_E_SHAPE, "kernel larger than the image");
+    MNF_REQUIRE(pad >= 0 && stride >= 1, MNF_E_ARG, "bad padding %d or stride %d", pad, stride);
+    MNF_REQUIRE(ksize >= 1 && ksize <= height + 2 * pad && ksize <= width + 2 * pad, MNF_E_SHAPE,
+                "kernel larger than the padded image");
     const long long total = n_imgs * c_in * height * width;
     if (total == 0) return 0;
-    col2im_t_kernel<<<ew_blocks(total), 256, 0, (cudaStream_t)stream>>>(grad_cols_t, grad_x, n_imgs, c_in, height, width, ksize);
+    col2im_t_kernel<<<ew_blocks(total), 256, 0, (cudaStream_t)stream>>>(grad_cols_t, grad_x, n_imgs, c_in, height, width,
+                                                                        ksize, pad, stride);
     return launch_status("col2im_t_kernel");
 }
 

@@ -26,6 +26,8 @@ _lib.register({
     "mnf_kl_rows_backward": (_int, [_vp] * 11 + [_int, _int, _vp]),
     "mnf_im2col_t": (_int, [_vp, _vp, _i64, _int, _int, _int, _int, _vp]),
     "mnf_col2im_t": (_int, [_vp, _vp, _i64, _int, _int, _int, _int, _vp]),
+    "mnf_im2col_t_ps": (_int, [_vp, _vp, _i64, _int, _int, _int, _int, _int, _int, _vp]),
+    "mnf_col2im_t_ps": (_int, [_vp, _vp, _i64, _int, _int, _int, _int, _int, _int, _vp]),
     "mnf_swap01": (_int, [_vp, _vp, _i64, _i64, _i64, _vp]),
     "mnf_rowsum": (_int, [_vp, _i64, _i64, _vp, _vp]),
 })
@@ -118,17 +120,23 @@ def _call(name, *args, device):
     _lib.launch_count += 1
 
 
-def im2col_t(x, ks):
+def _conv_out(n, ks, pad, stride):
+    return (n + 2 * pad - ks) // stride + 1
+
+
+def im2col_t(x, ks, pad=0, stride=1):
     R, c_in, H, W = x.shape
-    out = torch.empty((c_in * ks * ks, R * (H - ks + 1) * (W - ks + 1)), device=x.device, dtype=torch.float32)
-    _call("mnf_im2col_t", x.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, device=x.device)
+    P = R * _conv_out(H, ks, pad, stride) * _conv_out(W, ks, pad, stride)
+    out = torch.empty((c_in * ks * ks, P), device=x.device, dtype=torch.float32)
+    _call("mnf_im2col_t_ps", x.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, pad, stride, device=x.device)
     return out
 
 
-def col2im_t(g_cols_t, shape, ks):
+def col2im_t(g_cols_t, shape, ks, pad=0, stride=1):
     R, c_in, H, W = shape
     out = torch.empty(shape, device=g_cols_t.device, dtype=torch.float32)
-    _call("mnf_col2im_t", g_cols_t.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, device=g_cols_t.device)
+    _call("mnf_col2im_t_ps", g_cols_t.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, pad, stride,
+          device=g_cols_t.device)
     return out
 
 
@@ -419,15 +427,16 @@ def linear_kl_div(layer, noise=None):
 # ------------------------------------------------------------------------------------------------------------------
 class MnfConvOutFn(torch.autograd.Function):
     """mean = conv(x, W_mean * z[c]), var = conv(x^2, exp(W_log_var)) + exp(b_log_var), out = mean + sqrt(var) eps
-    (mnf_conv.py:68-79) as im2col GEMMs in the [c_out, R*OH*OW] layout, with a hand-written adjoint."""
+    (mnf_conv.py:68-79) as im2col GEMMs in the [c_out, R*OH*OW] layout, with a hand-written adjoint.  pad / stride:
+    zero padding and stride of the convolution (plain ints, no gradient)."""
 
     @staticmethod
-    def forward(ctx, x, z, W_mean, W_log_var, b_log_var, eps):
+    def forward(ctx, x, z, W_mean, W_log_var, b_log_var, eps, pad=0, stride=1):
         x, z = _c(x), _c(z)
         R, c_in, H, W = x.shape
         c_out, ks = W_mean.shape[0], W_mean.shape[2]
-        S, fan = (H - ks + 1) * (W - ks + 1), c_in * ks * ks
-        cols = im2col_t(x, ks)
+        S, fan = _conv_out(H, ks, pad, stride) * _conv_out(W, ks, pad, stride), c_in * ks * ks
+        cols = im2col_t(x, ks, pad, stride)
         cols2 = ew(EW_SQUARE, cols)
         Wm = _c(W_mean).view(c_out, fan)
         Wz = ew(EW_MUL_COLVEC, Wm, z, ncols=fan)
@@ -437,14 +446,14 @@ class MnfConvOutFn(torch.autograd.Function):
         var_t = ew(EW_ADD_COLVEC, gemm(Wv, cols2), bv, ncols=R * S)
         var = swap01(var_t, c_out, R, S).view(eps.shape)
         ctx.save_for_backward(z, Wm, cols, cols2, Wz, Wv, bv, var, eps)
-        ctx.geom = (tuple(x.shape), ks, W_mean.shape)
+        ctx.geom = (tuple(x.shape), ks, W_mean.shape, pad, stride)
         return ew(EW_NOISE_OUT, mean, var, eps)
 
     @staticmethod
     @torch.autograd.function.once_differentiable
     def backward(ctx, g):
         z, Wm, cols, cols2, Wz, Wv, bv, var, eps = ctx.saved_tensors
-        xshape, ks, wshape = ctx.geom
+        xshape, ks, wshape, pad, stride = ctx.geom
         R, c_out = xshape[0], wshape[0]
         fan, P = cols.shape
         S = P // R
@@ -460,8 +469,8 @@ class MnfConvOutFn(torch.autograd.Function):
         gx = None
         if ctx.needs_input_grad[0]:
             g_cols = ew(EW_ADD_2MUL, gemm(Wz, g_t, trans_a=True), gemm(Wv, gv_t, trans_a=True), cols)
-            gx = col2im_t(g_cols, xshape, ks)
-        return gx, gz, gW_mean, gW_lv, gb_lv, None
+            gx = col2im_t(g_cols, xshape, ks, pad, stride)
+        return gx, gz, gW_mean, gW_lv, gb_lv, None, None, None
 
 
 def conv_forward(layer, x, noise=None, relu_pool=False):
@@ -469,9 +478,9 @@ def conv_forward(layer, x, noise=None, relu_pool=False):
     x = _lib.require_cuda_f32(x, "input")
     tape = _tape(noise, x.device)
     z, _ = sample_z(layer, -1, tape, layer.n_out)
-    ks = layer.kernel_size
-    eps = _draw(tape, "normal", (x.size(0), layer.n_out, x.size(2) - ks + 1, x.size(3) - ks + 1), x.device)
-    out = MnfConvOutFn.apply(x, z[0], layer.W_mean, layer.W_log_var, layer.b_log_var, eps)
+    OH, OW = layer.output_size(x.size(2), x.size(3))
+    eps = _draw(tape, "normal", (x.size(0), layer.n_out, OH, OW), x.device)
+    out = MnfConvOutFn.apply(x, z[0], layer.W_mean, layer.W_log_var, layer.b_log_var, eps, layer.padding, layer.stride)
     return torch.nn.functional.max_pool2d(torch.relu(out), 2) if relu_pool else out
 
 

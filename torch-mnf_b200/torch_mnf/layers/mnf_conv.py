@@ -11,17 +11,28 @@ from . import _mnf_ops as ops
 from . import _train
 
 
+def _check_int(name, value, least):
+    if not isinstance(value, int) or isinstance(value, bool):
+        raise TypeError(f"MNFConv2d: {name} must be an int, got {value!r}")
+    if value < least:
+        raise ValueError(f"MNFConv2d: {name} must be >= {least}, got {value}")
+    return value
+
+
 class MNFConv2d(nn.Module):
-    """Bayesian conv layer (stride 1, no padding).  One z [n_out] per call, shared by the batch,
-    scales the output channels of the mean path; out = conv(x, W_mean*z) + sqrt(conv(x^2,
-    exp(W_log_var)) + exp(b_log_var)) * eps, computed as one implicit-GEMM CUDA kernel.
+    """Bayesian conv layer.  One z [n_out] per call, shared by the batch, scales the output channels
+    of the mean path; out = conv(x, W_mean*z) + sqrt(conv(x^2, exp(W_log_var)) + exp(b_log_var)) * eps,
+    computed as one implicit-GEMM CUDA kernel.  ``padding`` (zeros) and ``stride`` mean what they
+    mean for ``torch.nn.functional.conv2d``; the reference has neither (padding=0, stride=1).
+    They are geometry, not parameters: the state_dict and kl_div do not depend on them.
     ``b_mean`` is a fixed zero tensor and not part of the state_dict, as in the reference."""
 
     __getstate__ = state_without_caches  # copy.deepcopy / pickle drop cached device scratch
 
     def __init__(self, n_in: int, n_out: int, kernel_size: int, n_flows_q: int = 2, n_flows_r: int = 2,
-                 h_sizes: Sequence[int] = (50,)) -> None:
+                 h_sizes: Sequence[int] = (50,), *, padding: int = 0, stride: int = 1) -> None:
         super().__init__()
+        self.padding, self.stride = _check_int("padding", padding, 0), _check_int("stride", stride, 1)
         self.n_in, self.n_out, self.kernel_size = n_in, n_out, kernel_size
         shape = [n_out, n_in, kernel_size, kernel_size]
         self.W_mean = nn.Parameter(0.1 * torch.randn(shape))
@@ -35,6 +46,17 @@ class MNFConv2d(nn.Module):
         self.r0_b2 = nn.Parameter(0.1 * torch.randn(n_out))
         self.flow_q = flows.NormalizingFlow([flows.RNVP(n_out, h_sizes=h_sizes) for _ in range(n_flows_q)])
         self.flow_r = flows.NormalizingFlow([flows.RNVP(n_out, h_sizes=h_sizes) for _ in range(n_flows_r)])
+
+    def extra_repr(self) -> str:
+        return (f"{self.n_in}, {self.n_out}, kernel_size={self.kernel_size}, padding={self.padding}, "
+                f"stride={self.stride}")
+
+    def output_size(self, height: int, width: int) -> tuple[int, int]:
+        """(OH, OW) of this layer on height x width inputs; ValueError when the output would be empty."""
+        k, p, s = self.kernel_size, self.padding, self.stride
+        if height + 2 * p < k or width + 2 * p < k:
+            raise ValueError(f"MNFConv2d: kernel_size {k} is larger than the {height}x{width} input padded by {p}")
+        return (height + 2 * p - k) // s + 1, (width + 2 * p - k) // s + 1
 
     def sample_z(self, noise=None):
         """-> (z [1, n_out], log_det_q)."""
@@ -58,6 +80,8 @@ class MNFConv2d(nn.Module):
     def forward(self, x, noise=None, row_offset=0, relu_pool=False, n_imgs=None):
         """relu_pool=True fuses the ReLU + MaxPool2d(2) that follow this layer in MNFLeNet;
         n_imgs > len(x) replicates the images (image r reads x[r % len(x)])."""
+        if isinstance(x, torch.Tensor) and x.dim() == 4:
+            self.output_size(x.size(2), x.size(3))  # argument errors before any device work
         if _train.needs_grad(self, x):  # training: differentiable exact-fp32 path (layers/_train.py)
             if n_imgs is not None and n_imgs != x.size(0):
                 x = x.repeat(n_imgs // x.size(0), 1, 1, 1)
