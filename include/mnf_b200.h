@@ -406,6 +406,22 @@ int mnf_conv2d_forward_ps(const float *x, int64_t x_imgs, const float *z, const 
                           uint32_t noise_stream, uint64_t row_offset, float *out, int64_t n_imgs, int c_in,
                           int height, int width, int c_out, int ksize, int relu_pool, int pad, int stride,
                           void *stream);
+/* The same with dilation >= 1 and channel groups >= 1 as well, as torch.nn.functional.conv2d(..., padding=pad,
+ * stride=stride, dilation=dilation, groups=groups):
+ *   OH = (height + 2 pad - dilation (ksize - 1) - 1) / stride + 1, OW likewise;
+ *   W_mean, W_log_var: [c_out, c_in / groups, ksize, ksize]; groups must divide c_in and c_out (at most 65535 groups,
+ *   dilation (ksize - 1) <= 32767).
+ * Output channel c reads the c_in / groups input channels of its group c / (c_out / groups); tap (ky, kx) of output
+ * pixel (oy, ox) reads (oy*stride - pad + ky*dilation, ox*stride - pad + kx*dilation).  eps and its Philox numbering
+ * are those of mnf_conv2d_forward_ps over [n_imgs, c_out, OH, OW], which is this call with dilation = groups = 1.
+ * Kernels: the default geometry runs the unpadded implicit GEMM; groups > 1 with at most 8 output channels per group
+ * and at most 4096 taps per group (c_in / groups * ksize^2) run a direct kernel (one thread per output pixel and
+ * channel); every other geometry runs the bounds-tested implicit GEMM with one problem per group. */
+int mnf_conv2d_forward_geom(const float *x, int64_t x_imgs, const float *z, const float *W_mean,
+                            const float *W_log_var, const float *b_log_var, const float *eps, uint64_t seed,
+                            uint32_t noise_stream, uint64_t row_offset, float *out, int64_t n_imgs, int c_in,
+                            int height, int width, int c_out, int ksize, int relu_pool, int pad, int stride,
+                            int dilation, int groups, void *stream);
 
 /* Pieces of the MNF-LeNet Monte-Carlo pipeline (models/mnf_lenet.py:13-26 driven as in mnf_mnist.ipynb:316-318).
  * mnf_conv2d_moments: the sample-independent mean and standard deviation of an MNFConv2d (z is shared by the
@@ -424,6 +440,12 @@ int mnf_conv2d_moments(const float *x, const float *z, const float *W_mean, cons
 int mnf_conv2d_moments_ps(const float *x, const float *z, const float *W_mean, const float *W_log_var,
                           const float *b_log_var, float *mean_out, float *sd_out, int64_t n_imgs, int c_in,
                           int height, int width, int c_out, int ksize, int pad, int stride, void *stream);
+/* mnf_conv2d_moments with padding, stride, dilation and groups (geometry and kernel choice as for
+ * mnf_conv2d_forward_geom; dilation = groups = 1 is mnf_conv2d_moments_ps). */
+int mnf_conv2d_moments_geom(const float *x, const float *z, const float *W_mean, const float *W_log_var,
+                            const float *b_log_var, float *mean_out, float *sd_out, int64_t n_imgs, int c_in,
+                            int height, int width, int c_out, int ksize, int pad, int stride, int dilation, int groups,
+                            void *stream);
 int mnf_conv_noise_relu_pool(const float *mean, const float *sd, int64_t n_unique, const float *eps,
                              uint64_t seed, uint32_t noise_stream, uint64_t row_offset, float *out,
                              int64_t n_rows, int channels, int out_h, int out_w, void *stream);
@@ -505,6 +527,11 @@ int mnf_kl_div_fused_multi(const mnf_kl_fused_args *const *layers_host, int n_la
  * dimension lda, else [M,K]; trans_b: B is stored [N,K] (torch's Linear.weight), else [K,N]. */
 int mnf_gemm_f32(int trans_a, int trans_b, int64_t M, int N, int K, const float *A, int64_t lda, const float *B,
                  int64_t ldb, const float *bias, float beta, float *C, int64_t ldc, void *stream);
+/* batch (<= 65535) such products in one launch: product i reads A + i stride_a, B + i stride_b and writes
+ * C + i stride_c (strides in floats; bias is shared).  The grouped convolution's per-group GEMMs. */
+int mnf_gemm_f32_batched(int trans_a, int trans_b, int batch, int64_t M, int N, int K, const float *A, int64_t lda,
+                         int64_t stride_a, const float *B, int64_t ldb, int64_t stride_b, const float *bias, float beta,
+                         float *C, int64_t ldc, int64_t stride_c, void *stream);
 
 enum mnf_ew_op {
     MNF_EW_MUL = 1,        /* out = a b                                                                    */
@@ -544,6 +571,15 @@ int mnf_im2col_t_ps(const float *x, float *cols_t, int64_t n_imgs, int c_in, int
                     int stride, void *stream);
 int mnf_col2im_t_ps(const float *grad_cols_t, float *grad_x, int64_t n_imgs, int c_in, int height, int width, int ksize,
                     int pad, int stride, void *stream);
+/* The same with dilation >= 1 (OH = (height + 2 pad - dilation (ksize - 1) - 1) / stride + 1):
+ * cols_t[(ci,kh,kw)][(r,oh,ow)] = x[r, ci, oh*stride - pad + kh*dilation, ow*stride - pad + kw*dilation].
+ * mnf_col2im_t_geom stays the exact gather-form adjoint: an input pixel sums every dilated window tap that lands on it.
+ * A grouped convolution needs no other layout: group g's rows are the contiguous block of its input channels.
+ * dilation = 1 is mnf_im2col_t_ps / mnf_col2im_t_ps. */
+int mnf_im2col_t_geom(const float *x, float *cols_t, int64_t n_imgs, int c_in, int height, int width, int ksize,
+                      int pad, int stride, int dilation, void *stream);
+int mnf_col2im_t_geom(const float *grad_cols_t, float *grad_x, int64_t n_imgs, int c_in, int height, int width,
+                      int ksize, int pad, int stride, int dilation, void *stream);
 int mnf_swap01(const float *in, float *out, int64_t dim0, int64_t dim1, int64_t inner, void *stream);
 int mnf_rowsum(const float *a, int64_t n_rows, int64_t n_cols, float *out, void *stream);
 

@@ -48,9 +48,11 @@ struct DeviceProps {
 // cached per device, thread-safe (function-local statics); returns nullptr on error
 const DeviceProps *device_props();
 
-// output size of a zero-padded, strided convolution along one axis; 0 when the padded input is narrower than the filter
-__host__ __device__ inline int conv_out_size(int in, int ks, int pad, int stride) {
-    return in + 2 * pad >= ks ? (in + 2 * pad - ks) / stride + 1 : 0;
+// output size of a zero-padded, strided, dilated convolution along one axis; 0 when the padded input is narrower than
+// the dilated filter, whose extent is dil * (ks - 1) + 1
+__host__ __device__ inline int conv_out_size(int in, int ks, int pad, int stride, int dil = 1) {
+    const int ext = dil * (ks - 1) + 1;
+    return in + 2 * pad >= ext ? (in + 2 * pad - ext) / stride + 1 : 0;
 }
 
 __device__ __forceinline__ float warp_sum(float v) {

@@ -246,14 +246,16 @@ __global__ void __launch_bounds__(128) simt_gemv_kernel(const Prob p) {
     }
 }
 
+// batches > 1: that many independent problems of the same shape on grid dimension z; the functor tells them apart by
+// blockIdx.z (the groups of a grouped convolution)
 template <class Prob, int NACC>
-int launch_simt_gemm(const Prob &p, cudaStream_t stream, const char *what) {
+int launch_simt_gemm(const Prob &p, cudaStream_t stream, const char *what, int batches = 1) {
     if (p.M <= 0 || p.N <= 0) return 0;
     if (p.M <= 4 && p.K >= 256) {
-        simt_gemv_kernel<Prob, NACC><<<(unsigned)p.N, 128, 0, stream>>>(p);
+        simt_gemv_kernel<Prob, NACC><<<dim3((unsigned)p.N, 1, (unsigned)batches), 128, 0, stream>>>(p);
         return launch_status(what);
     }
-    dim3 grid((unsigned)((p.M + GBM - 1) / GBM), (unsigned)((p.N + GBN - 1) / GBN));
+    dim3 grid((unsigned)((p.M + GBM - 1) / GBM), (unsigned)((p.N + GBN - 1) / GBN), (unsigned)batches);
     if (grid.y > 65535) return fail(MNF_E_SHAPE, "%s: too many column tiles (%u)", what, grid.y);
     simt_gemm_kernel<Prob, NACC><<<grid, GTHREADS, 0, stream>>>(p);
     return launch_status(what);

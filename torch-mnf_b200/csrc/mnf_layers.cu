@@ -178,16 +178,19 @@ struct MnfLinearProb {
 // K = n_in*k*k.  With `pool` the row index is pool-major (4 consecutive rows = one 2x2 window)
 // and the epilogue applies ReLU + max over the window (the nn.ReLU / nn.MaxPool2d(2) that
 // follow every MNFConv2d in MNFLeNet, mnf_lenet.py:16-21).
-// GEOM: zero padding `pad` and stride `stride`.  Output pixel (oy, ox) reads the window whose origin is
-// (oy*stride - pad, ox*stride - pad); a tap outside the image loads 0, so it adds to neither moment.  Without GEOM
-// (pad 0, stride 1) every tap is inside the image and the loads carry no bounds test.
+// GEOM: zero padding `pad`, stride `stride`, dilation `dil` and channel groups.  Output pixel (oy, ox) reads the window
+// whose origin is (oy*stride - pad, ox*stride - pad), tap (ky, kx) at (ky*dil, kx*dil) from it; a tap outside the
+// image loads 0, so it adds to neither moment.  With groups, the launch carries one problem per group on grid
+// dimension z: N and K are the group's (n_out / groups columns, cg * ks * ks taps), group g reads input channels
+// g*cg .. g*cg + cg - 1 and writes output channels g*N .. g*N + N - 1.  Without GEOM (pad 0, stride 1, dilation 1,
+// one group) every tap is inside the image and the loads carry no bounds test.
 template <bool GEOM>
 struct MnfConvProb {
     int M, N, K;
     const float *x;  // [R, C, H, W]
     int x_imgs;      // image r reads x[r % x_imgs]
     int C, H, W, ks, OH, OW;
-    const float *Wm, *Wlv, *blv;  // [N, C, ks, ks], [N]
+    const float *Wm, *Wlv, *blv;  // [N, C, ks, ks], [N] (GEOM: [N * groups, cg, ks, ks], [N * groups])
     const float *z;               // [N] multiplicative noise, shared by the batch (mnf_conv.py:72)
     float *out;                   // [R, N, OH, OW] or pooled [R, N, OH/2, OW/2]
     NoiseSrc eps;                 // indexed like the un-pooled output [R, N, OH, OW]
@@ -213,11 +216,26 @@ struct MnfConvProb {
     static constexpr int kMaxTaps = 1600;
     int koff[kMaxTaps];
     int pad, stride;                 // GEOM only
-    int kyx[GEOM ? kMaxTaps : 1];    // GEOM: (ky << 16) | kx of tap k, for the bounds test
+    int kyx[GEOM ? kMaxTaps : 1];    // GEOM: (ky*dil << 16) | kx*dil of tap k, for the bounds test
+    int dil, cg;                     // GEOM only: dilation, input channels per group
     __device__ __forceinline__ int tap_offset(int k) const {
         if (k < kMaxTaps) return koff[k];
-        const int kx = k % ks, ky = (k / ks) % ks, ci = k / (ks * ks);
-        return (ci * H + ky) * W + kx;
+        if constexpr (GEOM) {
+            const int kx = (k % ks) * dil, ky = ((k / ks) % ks) * dil, ci = k / (ks * ks);
+            return (ci * H + ky) * W + kx;
+        } else {
+            const int kx = k % ks, ky = (k / ks) % ks, ci = k / (ks * ks);
+            return (ci * H + ky) * W + kx;
+        }
+    }
+    // GEOM: global output channel of the group's column n, and the layer's channel count
+    __device__ __forceinline__ int gcol(int n) const {
+        if constexpr (GEOM) return (int)blockIdx.z * N + n;
+        else return n;
+    }
+    __device__ __forceinline__ int n_total() const {
+        if constexpr (GEOM) return N * (int)gridDim.z;
+        else return N;
     }
     // GEOM: offset of the receptive-field origin in x (negative or past a row when it lies in the padding) and
     // the origin's coordinates; otherwise the offset alone
@@ -231,7 +249,7 @@ struct MnfConvProb {
         decode(m, r, oy, ox);
         if constexpr (GEOM) {
             const int iy = oy * stride - pad, ix = ox * stride - pad;
-            return GeomRow{((long long)(r % x_imgs) * C * H + iy) * W + ix, iy, ix};
+            return GeomRow{(((long long)(r % x_imgs) * C + (long long)blockIdx.z * cg) * H + iy) * W + ix, iy, ix};
         } else {
             return ((size_t)(r % x_imgs) * C * H + oy) * W + ox;
         }
@@ -243,7 +261,7 @@ struct MnfConvProb {
             if (k < kMaxTaps) {
                 ky = kyx[k] >> 16, kx = kyx[k] & 0xffff;
             } else {
-                kx = k % ks, ky = (k / ks) % ks;
+                kx = (k % ks) * dil, ky = ((k / ks) % ks) * dil;
             }
             const bool in = (unsigned)(r.iy + ky) < (unsigned)H && (unsigned)(r.ix + kx) < (unsigned)W;
             xv = in ? x[r.o + tap_offset(k)] : 0.f;
@@ -253,11 +271,13 @@ struct MnfConvProb {
         a[0] = xv;
         a[1] = xv * xv;
     }
-    __device__ void load_b(int n, int k, float (&v)[2]) const {
+    __device__ void load_b(int gn, int k, float (&v)[2]) const {
+        const int n = gcol(gn);
         v[0] = Wm[(size_t)n * K + k] * (z ? z[n] : 1.f);  // z == NULL: unit scale (per-sample z applied later)
         v[1] = expf(Wlv[(size_t)n * K + k]);
     }
-    __device__ void epilogue4(int m0, int n, const float (&acc)[2][4], float (&)[4]) const {
+    __device__ void epilogue4(int m0, int gn, const float (&acc)[2][4], float (&)[4]) const {
+        const int n = gcol(gn), NT = n_total();
         const float bvar = expf(blv[n]);
         float best = 0.f;  // ReLU floor
 #pragma unroll
@@ -266,8 +286,8 @@ struct MnfConvProb {
             if (m >= M) continue;
             int r, oy, ox;
             decode(m, r, oy, ox);
-            const long long e = (((long long)r * N + n) * OH + oy) * OW + ox;
-            const long long ge = ((((long long)r + (long long)eps.row_offset) * N + n) * OH + oy) * OW + ox;
+            const long long e = (((long long)r * NT + n) * OH + oy) * OW + ox;
+            const long long ge = ((((long long)r + (long long)eps.row_offset) * NT + n) * OH + oy) * OW + ox;
             if (sd_out) {
                 out[e] = acc[0][i];
                 sd_out[e] = sqrtf(acc[1][i] + bvar);
@@ -282,7 +302,7 @@ struct MnfConvProb {
         if (pool && m0 < M) {
             int r, oy, ox;
             decode(m0, r, oy, ox);
-            out[(((size_t)r * N + n) * (OH >> 1) + (oy >> 1)) * (OW >> 1) + (ox >> 1)] = best;
+            out[(((size_t)r * NT + n) * (OH >> 1) + (oy >> 1)) * (OW >> 1) + (ox >> 1)] = best;
         }
     }
     __device__ void row_out(int, float) const {}
@@ -567,20 +587,115 @@ static int launch_conv_moments_direct(const float *x, const float *z, const floa
     return launch_status("conv_moments_direct_kernel");
 }
 
-// the implicit-GEMM conv of mnf_conv2d_forward_ps / mnf_conv2d_moments_ps: tabulates the tap offsets (and, with
-// GEOM, the tap coordinates) on the host and launches the SIMT GEMM.  sd_out != NULL: moments mode.
+// Direct form of a grouped conv with few output channels per group (depthwise and its small channel multipliers):
+// as a grouped GEMM a group is a tile of 64 columns with 1..8 useful ones.  A CTA owns one output channel c (grid
+// dimension y) and a tile of output pixels (grid dimension x; with `pool`, of 2x2 windows) and walks the images
+// r = blockIdx.z, blockIdx.z + gridDim.z, ...; it stages c's folded weights [cg * ks * ks] (W_mean * z, exp(W_log_var))
+// in shared memory, and a thread walks the taps of its pixel over the cg input channels of c's group.  The sums run
+// over the taps in the order of the implicit GEMM's K loop with the same operands, and the noise, moments and
+// ReLU + pool epilogues are the GEMM's: the two kernels give the same bits for the same problem whenever the GEMM
+// runs its tiled form (launch_simt_gemm's GEMV form for M <= 4, K >= 256 sums in another order).
+struct ConvDirectArgs {
+    const float *x;
+    int x_imgs;  // image r reads x[r % x_imgs]
+    int C, H, W, ks, OH, OW, pad, stride, dil, cg, ng, N;  // N = n_out, ng = n_out / groups, cg = c_in / groups
+    const float *Wm, *Wlv, *blv, *z;  // z may be NULL (unit scale)
+    float *out;
+    float *sd_out;  // moments mode: out <- mean, sd_out <- sqrt(var), no noise
+    NoiseSrc eps;   // indexed like the un-pooled output [R, N, OH, OW]
+    int pool;
+    long long R;
+};
+
+__global__ void __launch_bounds__(256) conv_grouped_direct_kernel(const ConvDirectArgs p) {
+    extern __shared__ float sm_gd[];
+    const int c = blockIdx.y, taps = p.cg * p.ks * p.ks;
+    float *wm = sm_gd, *wv = sm_gd + taps;
+    const float zc = p.z ? p.z[c] : 1.f;
+    for (int t = threadIdx.x; t < taps; t += blockDim.x) {
+        wm[t] = p.Wm[(size_t)c * taps + t] * zc;
+        wv[t] = expf(p.Wlv[(size_t)c * taps + t]);
+    }
+    __syncthreads();
+    const int H = p.H, W = p.W, ks = p.ks, dil = p.dil, OH = p.OH, OW = p.OW, N = p.N;
+    const int PW = p.pool ? OW >> 1 : OW, PH = p.pool ? OH >> 1 : OH, sub = p.pool ? 4 : 1;
+    const int pix = blockIdx.x * blockDim.x + threadIdx.x;
+    if (pix >= PH * PW) return;
+    const int px = pix % PW, py = pix / PW;
+    const float bvar = expf(p.blv[c]);
+    const size_t in_ch0 = (size_t)(c / p.ng) * p.cg;  // first input channel of c's group
+    for (long long r = blockIdx.z; r < p.R; r += gridDim.z) {
+        const float *xr = p.x + ((size_t)(r % p.x_imgs) * p.C + in_ch0) * H * W;
+        float best = 0.f;  // ReLU floor
+        for (int q = 0; q < sub; ++q) {
+            const int oy = p.pool ? 2 * py + (q >> 1) : py, ox = p.pool ? 2 * px + (q & 1) : px;
+            const int iy = oy * p.stride - p.pad, ix = ox * p.stride - p.pad;
+            float am = 0.f, av = 0.f;
+            const float *xc = xr;
+            int t = 0;
+            for (int ci = 0; ci < p.cg; ++ci, xc += (size_t)H * W) {
+                for (int ky = 0; ky < ks; ++ky) {
+                    const int y = iy + ky * dil;
+                    const bool in_y = (unsigned)y < (unsigned)H;
+                    for (int kx = 0; kx < ks; ++kx, ++t) {
+                        const int xx = ix + kx * dil;
+                        const float xv = in_y && (unsigned)xx < (unsigned)W ? xc[y * W + xx] : 0.f;
+                        am = fmaf(xv, wm[t], am);
+                        av = fmaf(xv * xv, wv[t], av);
+                    }
+                }
+            }
+            const long long e = ((r * N + c) * OH + oy) * OW + ox;
+            if (p.sd_out) {
+                p.out[e] = am;
+                p.sd_out[e] = sqrtf(av + bvar);
+                continue;
+            }
+            const long long ge = (((r + (long long)p.eps.row_offset) * N + c) * OH + oy) * OW + ox;
+            const float v = am + sqrtf(av + bvar) * noise_normal(p.eps, e, ge);  // b_mean == 0
+            if (p.pool)
+                best = fmaxf(best, v);
+            else
+                p.out[e] = v;
+        }
+        if (p.pool) p.out[((r * N + c) * PH + py) * PW + px] = best;
+    }
+}
+
+// the grouped direct kernel serves groups of at most this many output channels and this many taps (its weights stay
+// in 32 KB of shared memory); wider groups run the grouped implicit GEMM.  On a B200, 64 -> 64 channels 3x3 on
+// 256 x 32 x 32 images with 8 channels a group: 3.67 ms on the grouped GEMM, 1.43 ms on the direct kernel; with 16 a
+// group the GEMM took 2.85 ms, about what the direct kernel's cost per channel predicts (profiles/r10_mnf_conv_groups.md).
+constexpr int kDirectMaxNg = 8, kDirectMaxTaps = 4096;
+
+// the conv of mnf_conv2d_forward_geom / mnf_conv2d_moments_geom: the implicit GEMM (tap offsets and, with GEOM, the
+// dilated tap coordinates tabulated on the host), or for groups > 1 with few channels per group the direct kernel.
+// sd_out != NULL: moments mode.
 template <bool GEOM>
 static int run_conv_gemm(const float *x, int x_imgs, const float *z, const float *Wm, const float *Wlv, const float *blv,
                          float *out, float *sd_out, NoiseSrc eps, int pool, long long M, int C, int H, int W, int ks,
-                         int N, int OH, int OW, int pad, int stride, cudaStream_t st, const char *what) {
-    MnfConvProb<GEOM> p{(int)M, N, C * ks * ks, x, x_imgs, C, H, W, ks, OH, OW, Wm, Wlv, blv, z, out, eps, pool, sd_out,
-                        {}, pad, stride, {}};
+                         int N, int OH, int OW, int pad, int stride, int dil, int groups, cudaStream_t st,
+                         const char *what) {
+    const int cg = C / groups, ng = N / groups, taps = cg * ks * ks;
+    if (GEOM && groups > 1 && ng <= kDirectMaxNg && taps <= kDirectMaxTaps && N <= 65535) {
+        const long long R = M / ((long long)OH * OW);
+        if (R == 0) return 0;
+        const int P = pool ? (OH / 2) * (OW / 2) : OH * OW;  // work items of one image and channel
+        const int threads = P < 256 ? (P + 31) & ~31 : 256;
+        const dim3 grid((unsigned)((P + threads - 1) / threads), (unsigned)N, (unsigned)(R < 65535 ? R : 65535));
+        const ConvDirectArgs a{x, x_imgs, C, H, W, ks, OH, OW, pad, stride, dil, cg, ng, N, Wm, Wlv, blv, z, out, sd_out,
+                               eps, pool, R};
+        conv_grouped_direct_kernel<<<grid, threads, 2 * sizeof(float) * taps, st>>>(a);
+        return launch_status("conv_grouped_direct_kernel");
+    }
+    MnfConvProb<GEOM> p{(int)M, ng, taps, x, x_imgs, C, H, W, ks, OH, OW, Wm, Wlv, blv, z, out, eps, pool, sd_out,
+                        {}, pad, stride, {}, dil, cg};
     for (int k = 0; k < p.K && k < MnfConvProb<GEOM>::kMaxTaps; ++k) {
-        const int kx = k % ks, ky = (k / ks) % ks, ci = k / (ks * ks);
+        const int kx = (k % ks) * dil, ky = ((k / ks) % ks) * dil, ci = k / (ks * ks);
         p.koff[k] = (ci * H + ky) * W + kx;
         if constexpr (GEOM) p.kyx[k] = (ky << 16) | kx;
     }
-    return launch_simt_gemm<MnfConvProb<GEOM>, 2>(p, st, what);
+    return launch_simt_gemm<MnfConvProb<GEOM>, 2>(p, st, what, groups);
 }
 
 int conv_pack_weights_f16(const float *z, const float *W_mean, const float *W_log_var, const float *b_log_var, void *Bm,
@@ -606,19 +721,35 @@ int mnf_conv2d_moments(const float *x, const float *z, const float *W_mean, cons
                                  ksize, 0, 1, stream);
 }
 
-// the same with zero padding `pad` and stride `stride` (OH = (H + 2 pad - k) / stride + 1).  Only pad 0 / stride 1
-// takes the direct kernel; every other geometry runs the implicit GEMM with bounds-tested tap loads.
 int mnf_conv2d_moments_ps(const float *x, const float *z, const float *W_mean, const float *W_log_var,
                           const float *b_log_var, float *mean_out, float *sd_out, int64_t n_imgs, int c_in, int height,
                           int width, int c_out, int ksize, int pad, int stride, void *stream) {
+    return mnf_conv2d_moments_geom(x, z, W_mean, W_log_var, b_log_var, mean_out, sd_out, n_imgs, c_in, height, width,
+                                   c_out, ksize, pad, stride, 1, 1, stream);
+}
+
+// checks shared by the _geom entry points: dilation, groups and the size of the tap table entries
+#define MNF_CHECK_DIL_GROUPS(c_in, c_out, ksize, dilation, groups)                                                        \
+    MNF_REQUIRE(dilation >= 1 && (long long)dilation * ((ksize) - 1) <= 0x7fff, MNF_E_ARG, "bad dilation %d", dilation); \
+    MNF_REQUIRE(groups >= 1 && groups <= 65535 && (c_in) % groups == 0 && (c_out) % groups == 0, MNF_E_ARG,             \
+                "groups %d must divide c_in %d and c_out %d", groups, c_in, c_out)
+
+// the same with zero padding `pad`, stride `stride`, dilation and channel groups (OH = (H + 2 pad - dil (k-1) - 1) /
+// stride + 1).  Only the default geometry takes the direct moments kernel; groups > 1 with few channels per group take
+// the grouped direct kernel, every other geometry runs the implicit GEMM with bounds-tested tap loads.
+int mnf_conv2d_moments_geom(const float *x, const float *z, const float *W_mean, const float *W_log_var,
+                            const float *b_log_var, float *mean_out, float *sd_out, int64_t n_imgs, int c_in, int height,
+                            int width, int c_out, int ksize, int pad, int stride, int dilation, int groups,
+                            void *stream) {
     MNF_REQUIRE(x && W_mean && W_log_var && b_log_var && mean_out && sd_out, MNF_E_ARG, "NULL pointer");  // z may be NULL (= 1)
     MNF_REQUIRE(pad >= 0 && pad <= 0xffff && stride >= 1, MNF_E_ARG, "bad padding %d or stride %d", pad, stride);
-    const int OH = conv_out_size(height, ksize, pad, stride), OW = conv_out_size(width, ksize, pad, stride);
+    MNF_CHECK_DIL_GROUPS(c_in, c_out, ksize, dilation, groups);
+    const int OH = conv_out_size(height, ksize, pad, stride, dilation), OW = conv_out_size(width, ksize, pad, stride, dilation);
     MNF_REQUIRE(n_imgs >= 0 && OH >= 1 && OW >= 1, MNF_E_SHAPE, "bad shape");
     const long long M = (long long)n_imgs * OH * OW;
     MNF_REQUIRE(M <= 0x7fffffff - 64, MNF_E_SHAPE, "too many output pixels for one call (%lld)", M);
     if (n_imgs == 0) return 0;
-    const bool geom = pad != 0 || stride != 1;
+    const bool geom = pad != 0 || stride != 1 || dilation != 1 || groups != 1;
     if (!geom && c_in * ksize * ksize <= 64 && c_out <= 32 && c_in * height * width <= 4096) {  // few taps, few channels: direct form
         if (c_out <= 20)
             return launch_conv_moments_direct<20>(x, z, W_mean, W_log_var, b_log_var, mean_out, sd_out, n_imgs, c_in, height,
@@ -630,9 +761,10 @@ int mnf_conv2d_moments_ps(const float *x, const float *z, const float *W_mean, c
     const int x_imgs = (int)(n_imgs > 0 ? n_imgs : 1);
     if (geom)
         return run_conv_gemm<true>(x, x_imgs, z, W_mean, W_log_var, b_log_var, mean_out, sd_out, none, 0, M, c_in, height,
-                                   width, ksize, c_out, OH, OW, pad, stride, (cudaStream_t)stream, "mnf_conv2d_moments");
+                                   width, ksize, c_out, OH, OW, pad, stride, dilation, groups, (cudaStream_t)stream,
+                                   "mnf_conv2d_moments");
     return run_conv_gemm<false>(x, x_imgs, z, W_mean, W_log_var, b_log_var, mean_out, sd_out, none, 0, M, c_in, height,
-                                width, ksize, c_out, OH, OW, 0, 1, (cudaStream_t)stream, "mnf_conv2d_moments");
+                                width, ksize, c_out, OH, OW, 0, 1, 1, 1, (cudaStream_t)stream, "mnf_conv2d_moments");
 }
 
 // out[r] = maxpool2(relu(mean[r % n_unique] + sd[r % n_unique] * eps[r])) -- the per-sample tail of an MNFConv2d
@@ -792,22 +924,34 @@ int mnf_conv2d_forward_ps(const float *x, int64_t x_imgs, const float *z, const 
                           const float *b_log_var, const float *eps, uint64_t seed, uint32_t noise_stream,
                           uint64_t row_offset, float *out, int64_t n_imgs, int c_in, int height, int width, int c_out,
                           int ksize, int relu_pool, int pad, int stride, void *stream) {
+    return mnf_conv2d_forward_geom(x, x_imgs, z, W_mean, W_log_var, b_log_var, eps, seed, noise_stream, row_offset, out,
+                                   n_imgs, c_in, height, width, c_out, ksize, relu_pool, pad, stride, 1, 1, stream);
+}
+
+int mnf_conv2d_forward_geom(const float *x, int64_t x_imgs, const float *z, const float *W_mean,
+                            const float *W_log_var, const float *b_log_var, const float *eps, uint64_t seed,
+                            uint32_t noise_stream, uint64_t row_offset, float *out, int64_t n_imgs, int c_in, int height,
+                            int width, int c_out, int ksize, int relu_pool, int pad, int stride, int dilation, int groups,
+                            void *stream) {
     MNF_REQUIRE(x && z && W_mean && W_log_var && b_log_var && out, MNF_E_ARG, "NULL pointer");
     MNF_REQUIRE(n_imgs >= 0 && c_in >= 1 && c_out >= 1 && ksize >= 1 && x_imgs >= 1, MNF_E_ARG, "bad shape");
     MNF_REQUIRE(pad >= 0 && pad <= 0xffff && stride >= 1, MNF_E_ARG, "bad padding %d or stride %d", pad, stride);
-    const int OH = conv_out_size(height, ksize, pad, stride), OW = conv_out_size(width, ksize, pad, stride);
-    MNF_REQUIRE(OH >= 1 && OW >= 1, MNF_E_SHAPE, "kernel %d larger than input %dx%d padded by %d", ksize, height, width, pad);
+    MNF_CHECK_DIL_GROUPS(c_in, c_out, ksize, dilation, groups);
+    const int OH = conv_out_size(height, ksize, pad, stride, dilation), OW = conv_out_size(width, ksize, pad, stride, dilation);
+    MNF_REQUIRE(OH >= 1 && OW >= 1, MNF_E_SHAPE, "kernel %d at dilation %d larger than input %dx%d padded by %d", ksize,
+                dilation, height, width, pad);
     MNF_REQUIRE(!relu_pool || (OH % 2 == 0 && OW % 2 == 0), MNF_E_SHAPE,
                 "fused 2x2 max-pool needs even output size, got %dx%d", OH, OW);
     const long long M = (long long)n_imgs * OH * OW;
     MNF_REQUIRE(M <= 0x7fffffff - 64, MNF_E_SHAPE, "too many output pixels for one call (%lld): chunk the batch", M);
     const NoiseSrc src{eps, seed, noise_stream, row_offset};
-    if (pad != 0 || stride != 1)
+    if (pad != 0 || stride != 1 || dilation != 1 || groups != 1)
         return run_conv_gemm<true>(x, (int)x_imgs, z, W_mean, W_log_var, b_log_var, out, nullptr, src, relu_pool, M, c_in,
-                                   height, width, ksize, c_out, OH, OW, pad, stride, (cudaStream_t)stream,
+                                   height, width, ksize, c_out, OH, OW, pad, stride, dilation, groups, (cudaStream_t)stream,
                                    "mnf_conv2d_forward");
     return run_conv_gemm<false>(x, (int)x_imgs, z, W_mean, W_log_var, b_log_var, out, nullptr, src, relu_pool, M, c_in,
-                                height, width, ksize, c_out, OH, OW, 0, 1, (cudaStream_t)stream, "mnf_conv2d_forward");
+                                height, width, ksize, c_out, OH, OW, 0, 1, 1, 1, (cudaStream_t)stream,
+                                "mnf_conv2d_forward");
 }
 
 }  // extern "C"

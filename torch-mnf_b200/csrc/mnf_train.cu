@@ -2,7 +2,8 @@
 // MNFLinear / kl_div through torch autograd, tests/test_mnf_mnist.py:28-43; these are the forward-with-saved-state and
 // backward kernels the drop-in modules' autograd Functions call).  Exact fp32 throughout -- training batches are
 // small (32 rows in the reference's test) and gradients should not carry TF32 rounding:
-//   mnf_gemm_f32            C = op(A) op(B) + bias + beta C, any transposition / leading dimensions (dgrad, wgrad)
+//   mnf_gemm_f32            C = op(A) op(B) + bias + beta C, any transposition / leading dimensions (dgrad, wgrad);
+//                           mnf_gemm_f32_batched: a batch of such products at fixed strides in one launch
 //   mnf_ew                  fused elementwise stages of the layer forward / backward
 //   mnf_colsum              bias-style reductions over rows
 //   mnf_rnvp_gate_*         the RNVP update z' = (1-m) z gate + (1-gate) shift + m z and its adjoint (rnvp.py:26-40)
@@ -12,13 +13,16 @@
 namespace mnf {
 
 // ---------------------------------------------------------------------------------------------------------------
-// generic fp32 GEMM: 64 x 64 tile, 16-deep slices, 256 threads x (4 x 4) accumulators
+// generic fp32 GEMM: 64 x 64 tile, 16-deep slices, 256 threads x (4 x 4) accumulators.  Grid dimension z walks a
+// batch of products whose operands lie sA / sB / sC floats apart (the groups of a grouped convolution).
 // ---------------------------------------------------------------------------------------------------------------
 template <bool TA, bool TB>
 __global__ void __launch_bounds__(256)
 gemm_f32_kernel(long long M, int N, int K, const float *__restrict__ A, long long lda, const float *__restrict__ B,
-                long long ldb, const float *__restrict__ bias, float beta, float *__restrict__ C, long long ldc) {
+                long long ldb, const float *__restrict__ bias, float beta, float *__restrict__ C, long long ldc,
+                long long sA, long long sB, long long sC) {
     __shared__ float As[16][64 + 4], Bs[16][64 + 4];
+    A += blockIdx.z * sA, B += blockIdx.z * sB, C += blockIdx.z * sC;
     const int tid = threadIdx.x, tx = tid % 16, ty = tid / 16;
     const long long m0 = (long long)blockIdx.y * 64;
     const int n0 = blockIdx.x * 64;
@@ -195,40 +199,41 @@ __global__ void kl_rows_bwd_kernel(const float *__restrict__ z, const float *__r
 }
 
 // ---------------------------------------------------------------------------------------------------------------
-// convolution as GEMM with zero padding `pad` and stride `st`: transposed im2col
-// colsT[(ci,kh,kw)][(r,oh,ow)] = x[r, ci, oh*st - pad + kh, ow*st - pad + kw] (0 in the padding), its adjoint (gather
-// form, no atomics), and the [A,B,inner] -> [B,A,inner] layout swap between the GEMM's [c_out, R*OH*OW] and the
-// module's [R, c_out, OH, OW].  With pad 0 and stride 1 every bounds test passes and the adjoint sums the same terms
-// in the same order as the unpadded form.
+// convolution as GEMM with zero padding `pad`, stride `st` and dilation `dl`: transposed im2col
+// colsT[(ci,kh,kw)][(r,oh,ow)] = x[r, ci, oh*st - pad + kh*dl, ow*st - pad + kw*dl] (0 in the padding), its adjoint
+// (gather form, no atomics), and the [A,B,inner] -> [B,A,inner] layout swap between the GEMM's [c_out, R*OH*OW] and
+// the module's [R, c_out, OH, OW].  With pad 0, stride 1 and dilation 1 every bounds test passes and the adjoint sums
+// the same terms in the same order as the unpadded form.  Channel groups need nothing here: group g's rows of colsT
+// are the contiguous block of its input channels.
 // ---------------------------------------------------------------------------------------------------------------
 __global__ void im2col_t_kernel(const float *__restrict__ x, float *__restrict__ colsT, long long R, int c_in, int H,
-                                int W, int ks, int pad, int st) {
-    const int OH = conv_out_size(H, ks, pad, st), OW = conv_out_size(W, ks, pad, st);
+                                int W, int ks, int pad, int st, int dl) {
+    const int OH = conv_out_size(H, ks, pad, st, dl), OW = conv_out_size(W, ks, pad, st, dl);
     const long long P = R * OH * OW, total = (long long)c_in * ks * ks * P;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const long long p = i % P;
         const int f = (int)(i / P), kw = f % ks, kh = (f / ks) % ks, ci = f / (ks * ks);
         const int ow = (int)(p % OW), oh = (int)((p / OW) % OH);
         const long long r = p / ((long long)OW * OH);
-        const int ih = oh * st - pad + kh, iw = ow * st - pad + kw;
+        const int ih = oh * st - pad + kh * dl, iw = ow * st - pad + kw * dl;
         colsT[i] = ((unsigned)ih < (unsigned)H && (unsigned)iw < (unsigned)W) ? x[((r * c_in + ci) * H + ih) * W + iw] : 0.f;
     }
 }
 
 __global__ void col2im_t_kernel(const float *__restrict__ g_colsT, float *__restrict__ gx, long long R, int c_in, int H,
-                                int W, int ks, int pad, int st) {
-    const int OH = conv_out_size(H, ks, pad, st), OW = conv_out_size(W, ks, pad, st);
+                                int W, int ks, int pad, int st, int dl) {
+    const int OH = conv_out_size(H, ks, pad, st, dl), OW = conv_out_size(W, ks, pad, st, dl);
     const long long P = R * OH * OW, total = R * c_in * H * W;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const int w = (int)(i % W), h = (int)((i / W) % H), ci = (int)((i / ((long long)W * H)) % c_in);
         const long long r = i / ((long long)W * H * c_in);
         float acc = 0.f;
         for (int kh = 0; kh < ks; ++kh) {
-            const int th = h + pad - kh;  // oh * st when input row h is tap row kh of output row oh
+            const int th = h + pad - kh * dl;  // oh * st when input row h is tap row kh of output row oh
             if (th < 0 || th % st != 0 || th / st >= OH) continue;
             const int oh = th / st;
             for (int kw = 0; kw < ks; ++kw) {
-                const int tw = w + pad - kw;
+                const int tw = w + pad - kw * dl;
                 if (tw < 0 || tw % st != 0 || tw / st >= OW) continue;
                 const int ow = tw / st;
                 acc += g_colsT[(long long)((ci * ks + kh) * ks + kw) * P + (r * OH + oh) * OW + ow];
@@ -271,17 +276,29 @@ extern "C" {
 
 int mnf_gemm_f32(int trans_a, int trans_b, int64_t M, int N, int K, const float *A, int64_t lda, const float *B,
                  int64_t ldb, const float *bias, float beta, float *C, int64_t ldc, void *stream) {
+    return mnf_gemm_f32_batched(trans_a, trans_b, 1, M, N, K, A, lda, 0, B, ldb, 0, bias, beta, C, ldc, 0, stream);
+}
+
+int mnf_gemm_f32_batched(int trans_a, int trans_b, int batch, int64_t M, int N, int K, const float *A, int64_t lda,
+                         int64_t stride_a, const float *B, int64_t ldb, int64_t stride_b, const float *bias, float beta,
+                         float *C, int64_t ldc, int64_t stride_c, void *stream) {
     MNF_REQUIRE(A && B && C, MNF_E_ARG, "NULL pointer");
     MNF_REQUIRE(M >= 0 && N >= 0 && K >= 0, MNF_E_ARG, "negative size");
-    if (M == 0 || N == 0) return 0;
+    MNF_REQUIRE(batch >= 0 && batch <= 65535, MNF_E_ARG, "bad batch count %d", batch);
+    if (M == 0 || N == 0 || batch == 0) return 0;
     const long long gy = (M + 63) / 64;
     MNF_REQUIRE(gy <= 65535, MNF_E_SHAPE, "M=%lld too large for one launch", (long long)M);
-    dim3 grid((N + 63) / 64, (unsigned)gy);
+    dim3 grid((N + 63) / 64, (unsigned)gy, (unsigned)batch);
     cudaStream_t st = (cudaStream_t)stream;
-    if (trans_a && trans_b) gemm_f32_kernel<true, true><<<grid, 256, 0, st>>>(M, N, K, A, lda, B, ldb, bias, beta, C, ldc);
-    else if (trans_a) gemm_f32_kernel<true, false><<<grid, 256, 0, st>>>(M, N, K, A, lda, B, ldb, bias, beta, C, ldc);
-    else if (trans_b) gemm_f32_kernel<false, true><<<grid, 256, 0, st>>>(M, N, K, A, lda, B, ldb, bias, beta, C, ldc);
-    else gemm_f32_kernel<false, false><<<grid, 256, 0, st>>>(M, N, K, A, lda, B, ldb, bias, beta, C, ldc);
+    const long long sa = stride_a, sb = stride_b, sc = stride_c;
+    if (trans_a && trans_b)
+        gemm_f32_kernel<true, true><<<grid, 256, 0, st>>>(M, N, K, A, lda, B, ldb, bias, beta, C, ldc, sa, sb, sc);
+    else if (trans_a)
+        gemm_f32_kernel<true, false><<<grid, 256, 0, st>>>(M, N, K, A, lda, B, ldb, bias, beta, C, ldc, sa, sb, sc);
+    else if (trans_b)
+        gemm_f32_kernel<false, true><<<grid, 256, 0, st>>>(M, N, K, A, lda, B, ldb, bias, beta, C, ldc, sa, sb, sc);
+    else
+        gemm_f32_kernel<false, false><<<grid, 256, 0, st>>>(M, N, K, A, lda, B, ldb, bias, beta, C, ldc, sa, sb, sc);
     return launch_status("gemm_f32_kernel");
 }
 
@@ -311,15 +328,29 @@ int mnf_im2col_t(const float *x, float *cols_t, int64_t n_imgs, int c_in, int he
 
 int mnf_im2col_t_ps(const float *x, float *cols_t, int64_t n_imgs, int c_in, int height, int width, int ksize, int pad,
                     int stride, void *stream) {
-    MNF_REQUIRE(x && cols_t, MNF_E_ARG, "NULL pointer");
+    return mnf_im2col_t_geom(x, cols_t, n_imgs, c_in, height, width, ksize, pad, stride, 1, stream);
+}
+
+// argument checks shared by the _geom im2col / col2im
+static int check_unfold_geom(int height, int width, int ksize, int pad, int stride, int dilation) {
     MNF_REQUIRE(pad >= 0 && stride >= 1, MNF_E_ARG, "bad padding %d or stride %d", pad, stride);
-    MNF_REQUIRE(ksize >= 1 && ksize <= height + 2 * pad && ksize <= width + 2 * pad, MNF_E_SHAPE,
-                "kernel larger than the padded image");
-    const long long total = (long long)c_in * ksize * ksize * n_imgs * conv_out_size(height, ksize, pad, stride) *
-                            conv_out_size(width, ksize, pad, stride);
+    MNF_REQUIRE(dilation >= 1 && (ksize < 1 || (long long)dilation * (ksize - 1) <= 0x7fff), MNF_E_ARG,
+                "bad dilation %d", dilation);
+    MNF_REQUIRE(ksize >= 1 && conv_out_size(height, ksize, pad, stride, dilation) >= 1 &&
+                    conv_out_size(width, ksize, pad, stride, dilation) >= 1,
+                MNF_E_SHAPE, "kernel larger than the padded image");
+    return 0;
+}
+
+int mnf_im2col_t_geom(const float *x, float *cols_t, int64_t n_imgs, int c_in, int height, int width, int ksize,
+                      int pad, int stride, int dilation, void *stream) {
+    MNF_REQUIRE(x && cols_t, MNF_E_ARG, "NULL pointer");
+    if (const int rc = check_unfold_geom(height, width, ksize, pad, stride, dilation)) return rc;
+    const long long total = (long long)c_in * ksize * ksize * n_imgs * conv_out_size(height, ksize, pad, stride, dilation) *
+                            conv_out_size(width, ksize, pad, stride, dilation);
     if (total == 0) return 0;
     im2col_t_kernel<<<ew_blocks(total), 256, 0, (cudaStream_t)stream>>>(x, cols_t, n_imgs, c_in, height, width, ksize, pad,
-                                                                        stride);
+                                                                        stride, dilation);
     return launch_status("im2col_t_kernel");
 }
 
@@ -330,14 +361,17 @@ int mnf_col2im_t(const float *grad_cols_t, float *grad_x, int64_t n_imgs, int c_
 
 int mnf_col2im_t_ps(const float *grad_cols_t, float *grad_x, int64_t n_imgs, int c_in, int height, int width, int ksize,
                     int pad, int stride, void *stream) {
+    return mnf_col2im_t_geom(grad_cols_t, grad_x, n_imgs, c_in, height, width, ksize, pad, stride, 1, stream);
+}
+
+int mnf_col2im_t_geom(const float *grad_cols_t, float *grad_x, int64_t n_imgs, int c_in, int height, int width,
+                      int ksize, int pad, int stride, int dilation, void *stream) {
     MNF_REQUIRE(grad_cols_t && grad_x, MNF_E_ARG, "NULL pointer");
-    MNF_REQUIRE(pad >= 0 && stride >= 1, MNF_E_ARG, "bad padding %d or stride %d", pad, stride);
-    MNF_REQUIRE(ksize >= 1 && ksize <= height + 2 * pad && ksize <= width + 2 * pad, MNF_E_SHAPE,
-                "kernel larger than the padded image");
+    if (const int rc = check_unfold_geom(height, width, ksize, pad, stride, dilation)) return rc;
     const long long total = n_imgs * c_in * height * width;
     if (total == 0) return 0;
     col2im_t_kernel<<<ew_blocks(total), 256, 0, (cudaStream_t)stream>>>(grad_cols_t, grad_x, n_imgs, c_in, height, width,
-                                                                        ksize, pad, stride);
+                                                                        ksize, pad, stride, dilation);
     return launch_status("col2im_t_kernel");
 }
 

@@ -66,6 +66,8 @@ _lib.register({
                                   _int, _int, _int, _int, _vp]),
     "mnf_conv2d_forward_ps": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int, _int,
                                      _int, _int, _int, _int, _int, _int, _vp]),
+    "mnf_conv2d_forward_geom": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int, _int,
+                                       _int, _int, _int, _int, _int, _int, _int, _int, _vp]),
     "mnf_kl_div": (_int, [C.POINTER(KlArgs), _vp]),
     "mnf_linear_tc_workspace": (_i64, [_i64, _i64, _int, _int]),
     "mnf_linear_forward_tc": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int,
@@ -80,6 +82,8 @@ _lib.register({
     "mnf_conv2d_moments": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _int, _int, _int, _vp]),
     "mnf_conv2d_moments_ps": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _int, _int, _int, _int, _int,
                                      _vp]),
+    "mnf_conv2d_moments_geom": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _int, _int, _int, _int, _int,
+                                       _int, _int, _int, _vp]),
     "mnf_conv_noise_relu_pool": (_int, [_vp, _vp, _i64, _vp, _u64, _u32, _u64, _vp, _i64, _int, _int, _int, _vp]),
     "mnf_conv_noise_relu_pool_z": (_int, [_vp, _vp, _i64, _vp, _u64, _u32, _u64, _vp, _i64, _int, _int, _int, _vp, _i64,
                                           _vp]),
@@ -391,10 +395,11 @@ def conv_forward(layer, x, z, noise: Noise, n_imgs=None, relu_pool=False, drawn=
     args = [_param(t, dev, n) for t, n in ((layer.W_mean, "W_mean"), (layer.W_log_var, "W_log_var"),
                                            (layer.b_log_var, "b_log_var"))]
     with torch.cuda.device(dev):
-        rc = _lib.lib().mnf_conv2d_forward_ps(x.data_ptr(), x_imgs, z.data_ptr(), *(a.data_ptr() for a in args),
-                                              _p(eps), noise.seed, sid, row_offset, out.data_ptr(), R, c_in, H, W, c_out,
-                                              ks, int(relu_pool), layer.padding, layer.stride, _lib.stream_ptr(dev))
-    _lib.check(rc, "mnf_conv2d_forward_ps")
+        rc = _lib.lib().mnf_conv2d_forward_geom(x.data_ptr(), x_imgs, z.data_ptr(), *(a.data_ptr() for a in args),
+                                                _p(eps), noise.seed, sid, row_offset, out.data_ptr(), R, c_in, H, W,
+                                                c_out, ks, int(relu_pool), layer.padding, layer.stride, layer.dilation,
+                                                layer.groups, _lib.stream_ptr(dev))
+    _lib.check(rc, "mnf_conv2d_forward_geom")
     _lib.launch_count += 1
     return out
 
@@ -430,10 +435,10 @@ def conv_moments(layer, x, z):
     sd = torch.empty_like(mean)
     args = _conv_args(layer, dev)
     with torch.cuda.device(dev):
-        rc = _lib.lib().mnf_conv2d_moments_ps(x.data_ptr(), _p(z), *(a.data_ptr() for a in args), mean.data_ptr(),
-                                              sd.data_ptr(), B, c_in, H, W, c_out, ks, layer.padding, layer.stride,
-                                              _lib.stream_ptr(dev))
-    _lib.check(rc, "mnf_conv2d_moments_ps")
+        rc = _lib.lib().mnf_conv2d_moments_geom(x.data_ptr(), _p(z), *(a.data_ptr() for a in args), mean.data_ptr(),
+                                                sd.data_ptr(), B, c_in, H, W, c_out, ks, layer.padding, layer.stride,
+                                                layer.dilation, layer.groups, _lib.stream_ptr(dev))
+    _lib.check(rc, "mnf_conv2d_moments_geom")
     _lib.launch_count += 1
     return mean, sd
 
@@ -465,10 +470,13 @@ def conv_mc_relu_pool(layer, x, z, noise: Noise, n_rows, z_rows=None, rows_per_z
 def conv_forward_tc(layer, x, z, noise: Noise, z_rows=None, rows_per_z=1):
     """maxpool2(relu(MNFConv2d(x))) on the TF32 tensor cores (implicit GEMM, or im2col + GEMMs for other geometries).
     z_rows [n_z, c_out] (with z = None): per-sample z, image r scaled by z_rows[r // rows_per_z].
-    Padding and stride are not supported here: the tensor-core conv serves MNFLeNet's unpadded layers."""
+    Padding, stride, dilation and groups are not supported here: the tensor-core conv serves MNFLeNet's plain layers."""
     if layer.padding != 0 or layer.stride != 1:
         raise ValueError(f"the tensor-core conv supports padding=0, stride=1 only (got padding={layer.padding}, "
                          f"stride={layer.stride})")
+    if layer.dilation != 1 or layer.groups != 1:
+        raise ValueError(f"the tensor-core conv supports dilation=1, groups=1 only (got dilation={layer.dilation}, "
+                         f"groups={layer.groups})")
     dev = x.device
     R, c_in, H, W = x.shape
     c_out, ks = layer.W_mean.shape[0], layer.W_mean.shape[2]

@@ -18,6 +18,8 @@ from .. import _lib
 _vp, _i64, _int, _f = C.c_void_p, C.c_int64, C.c_int, C.c_float
 _lib.register({
     "mnf_gemm_f32": (_int, [_int, _int, _i64, _int, _int, _vp, _i64, _vp, _i64, _vp, _f, _vp, _i64, _vp]),
+    "mnf_gemm_f32_batched": (_int, [_int, _int, _int, _i64, _int, _int, _vp, _i64, _i64, _vp, _i64, _i64, _vp, _f, _vp,
+                                    _i64, _i64, _vp]),
     "mnf_ew": (_int, [_int, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _vp]),
     "mnf_colsum": (_int, [_vp, _vp, _i64, _int, _vp, _vp]),
     "mnf_rnvp_gate_forward": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _i64, _int, _vp]),
@@ -28,6 +30,8 @@ _lib.register({
     "mnf_col2im_t": (_int, [_vp, _vp, _i64, _int, _int, _int, _int, _vp]),
     "mnf_im2col_t_ps": (_int, [_vp, _vp, _i64, _int, _int, _int, _int, _int, _int, _vp]),
     "mnf_col2im_t_ps": (_int, [_vp, _vp, _i64, _int, _int, _int, _int, _int, _int, _vp]),
+    "mnf_im2col_t_geom": (_int, [_vp, _vp, _i64, _int, _int, _int, _int, _int, _int, _int, _vp]),
+    "mnf_col2im_t_geom": (_int, [_vp, _vp, _i64, _int, _int, _int, _int, _int, _int, _int, _vp]),
     "mnf_swap01": (_int, [_vp, _vp, _i64, _i64, _i64, _vp]),
     "mnf_rowsum": (_int, [_vp, _i64, _i64, _vp, _vp]),
 })
@@ -92,6 +96,25 @@ def gemm(A, B, trans_a=False, trans_b=False, bias=None, out=None, beta=0.0):
     return out
 
 
+def gemm_grouped(A, B, groups, trans_a=False, trans_b=False):
+    """The block-diagonal product of a grouped convolution: A and B are split along their rows into `groups` equal
+    blocks and out[block g] = op(A_g) @ op(B_g), all blocks in one launch (mnf_gemm_f32_batched).  groups = 1 is
+    gemm(A, B, trans_a, trans_b)."""
+    if groups == 1:
+        return gemm(A, B, trans_a=trans_a, trans_b=trans_b)
+    ra, rb = A.shape[0] // groups, B.shape[0] // groups  # rows of one block of A and of B as stored
+    M, K = (A.shape[1], ra) if trans_a else (ra, A.shape[1])
+    N = rb if trans_b else B.shape[1]
+    out = torch.empty((groups * M, N), device=A.device, dtype=torch.float32)
+    with torch.cuda.device(A.device):
+        rc = _lib.lib().mnf_gemm_f32_batched(int(trans_a), int(trans_b), groups, M, N, K, A.data_ptr(), A.stride(0),
+                                             ra * A.stride(0), B.data_ptr(), B.stride(0), rb * B.stride(0), None, 0.0,
+                                             out.data_ptr(), out.stride(0), M * out.stride(0), _lib.stream_ptr(A.device))
+    _lib.check(rc, "mnf_gemm_f32_batched")
+    _lib.launch_count += 1
+    return out
+
+
 def ew(op, a, b=None, c=None, d=None, ncols=1, two=False):
     out = torch.empty_like(a)
     out2 = torch.empty_like(a) if two else None
@@ -120,23 +143,31 @@ def _call(name, *args, device):
     _lib.launch_count += 1
 
 
-def _conv_out(n, ks, pad, stride):
-    return (n + 2 * pad - ks) // stride + 1
+def _conv_out(n, ks, pad, stride, dilation=1):
+    return (n + 2 * pad - dilation * (ks - 1) - 1) // stride + 1
 
 
-def im2col_t(x, ks, pad=0, stride=1):
+def im2col_t(x, ks, pad=0, stride=1, dilation=1):
     R, c_in, H, W = x.shape
-    P = R * _conv_out(H, ks, pad, stride) * _conv_out(W, ks, pad, stride)
+    P = R * _conv_out(H, ks, pad, stride, dilation) * _conv_out(W, ks, pad, stride, dilation)
     out = torch.empty((c_in * ks * ks, P), device=x.device, dtype=torch.float32)
-    _call("mnf_im2col_t_ps", x.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, pad, stride, device=x.device)
+    if dilation == 1:
+        _call("mnf_im2col_t_ps", x.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, pad, stride, device=x.device)
+    else:
+        _call("mnf_im2col_t_geom", x.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, pad, stride, dilation,
+              device=x.device)
     return out
 
 
-def col2im_t(g_cols_t, shape, ks, pad=0, stride=1):
+def col2im_t(g_cols_t, shape, ks, pad=0, stride=1, dilation=1):
     R, c_in, H, W = shape
     out = torch.empty(shape, device=g_cols_t.device, dtype=torch.float32)
-    _call("mnf_col2im_t_ps", g_cols_t.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, pad, stride,
-          device=g_cols_t.device)
+    if dilation == 1:
+        _call("mnf_col2im_t_ps", g_cols_t.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, pad, stride,
+              device=g_cols_t.device)
+    else:
+        _call("mnf_col2im_t_geom", g_cols_t.data_ptr(), out.data_ptr(), R, c_in, H, W, ks, pad, stride, dilation,
+              device=g_cols_t.device)
     return out
 
 
@@ -427,50 +458,53 @@ def linear_kl_div(layer, noise=None):
 # ------------------------------------------------------------------------------------------------------------------
 class MnfConvOutFn(torch.autograd.Function):
     """mean = conv(x, W_mean * z[c]), var = conv(x^2, exp(W_log_var)) + exp(b_log_var), out = mean + sqrt(var) eps
-    (mnf_conv.py:68-79) as im2col GEMMs in the [c_out, R*OH*OW] layout, with a hand-written adjoint.  pad / stride:
-    zero padding and stride of the convolution (plain ints, no gradient)."""
+    (mnf_conv.py:68-79) as im2col GEMMs in the [c_out, R*OH*OW] layout, with a hand-written adjoint.  pad / stride /
+    dilation / groups: geometry of the convolution (plain ints, no gradient).  With groups, the rows of the im2col
+    matrix and of the weights split into per-group blocks and every product is a batched, block-diagonal GEMM."""
 
     @staticmethod
-    def forward(ctx, x, z, W_mean, W_log_var, b_log_var, eps, pad=0, stride=1):
+    def forward(ctx, x, z, W_mean, W_log_var, b_log_var, eps, pad=0, stride=1, dilation=1, groups=1):
         x, z = _c(x), _c(z)
         R, c_in, H, W = x.shape
         c_out, ks = W_mean.shape[0], W_mean.shape[2]
-        S, fan = _conv_out(H, ks, pad, stride) * _conv_out(W, ks, pad, stride), c_in * ks * ks
-        cols = im2col_t(x, ks, pad, stride)
+        S = _conv_out(H, ks, pad, stride, dilation) * _conv_out(W, ks, pad, stride, dilation)
+        fan = (c_in // groups) * ks * ks
+        cols = im2col_t(x, ks, pad, stride, dilation)
         cols2 = ew(EW_SQUARE, cols)
         Wm = _c(W_mean).view(c_out, fan)
         Wz = ew(EW_MUL_COLVEC, Wm, z, ncols=fan)
         Wv = ew(EW_EXP, _c(W_log_var).view(c_out, fan))
         bv = ew(EW_EXP, _c(b_log_var))
-        mean = swap01(gemm(Wz, cols), c_out, R, S).view(eps.shape)
-        var_t = ew(EW_ADD_COLVEC, gemm(Wv, cols2), bv, ncols=R * S)
+        mean = swap01(gemm_grouped(Wz, cols, groups), c_out, R, S).view(eps.shape)
+        var_t = ew(EW_ADD_COLVEC, gemm_grouped(Wv, cols2, groups), bv, ncols=R * S)
         var = swap01(var_t, c_out, R, S).view(eps.shape)
         ctx.save_for_backward(z, Wm, cols, cols2, Wz, Wv, bv, var, eps)
-        ctx.geom = (tuple(x.shape), ks, W_mean.shape, pad, stride)
+        ctx.geom = (tuple(x.shape), ks, W_mean.shape, pad, stride, dilation, groups)
         return ew(EW_NOISE_OUT, mean, var, eps)
 
     @staticmethod
     @torch.autograd.function.once_differentiable
     def backward(ctx, g):
         z, Wm, cols, cols2, Wz, Wv, bv, var, eps = ctx.saved_tensors
-        xshape, ks, wshape, pad, stride = ctx.geom
+        xshape, ks, wshape, pad, stride, dilation, groups = ctx.geom
         R, c_out = xshape[0], wshape[0]
-        fan, P = cols.shape
+        P = cols.shape[1]
         S = P // R
         g = _c(g)
         g_var = ew(EW_GVAR, g, var, eps)
         g_t = swap01(g, R, c_out, S).view(c_out, P)
         gv_t = swap01(g_var, R, c_out, S).view(c_out, P)
-        gWz = gemm(g_t, cols, trans_b=True)
-        gW_mean = ew(EW_MUL_COLVEC, gWz, z, ncols=fan).view(wshape)
+        gWz = gemm_grouped(g_t, cols, groups, trans_b=True)
+        gW_mean = ew(EW_MUL_COLVEC, gWz, z, ncols=Wm.shape[1]).view(wshape)
         gz = rowsum(ew(EW_MUL, gWz, Wm))
-        gW_lv = ew(EW_MUL, gemm(gv_t, cols2, trans_b=True), Wv).view(wshape)
+        gW_lv = ew(EW_MUL, gemm_grouped(gv_t, cols2, groups, trans_b=True), Wv).view(wshape)
         gb_lv = ew(EW_MUL, rowsum(gv_t), bv)
         gx = None
         if ctx.needs_input_grad[0]:
-            g_cols = ew(EW_ADD_2MUL, gemm(Wz, g_t, trans_a=True), gemm(Wv, gv_t, trans_a=True), cols)
-            gx = col2im_t(g_cols, xshape, ks, pad, stride)
-        return gx, gz, gW_mean, gW_lv, gb_lv, None, None, None
+            g_cols = ew(EW_ADD_2MUL, gemm_grouped(Wz, g_t, groups, trans_a=True),
+                        gemm_grouped(Wv, gv_t, groups, trans_a=True), cols)
+            gx = col2im_t(g_cols, xshape, ks, pad, stride, dilation)
+        return gx, gz, gW_mean, gW_lv, gb_lv, None, None, None, None, None
 
 
 def conv_forward(layer, x, noise=None, relu_pool=False):
@@ -480,7 +514,8 @@ def conv_forward(layer, x, noise=None, relu_pool=False):
     z, _ = sample_z(layer, -1, tape, layer.n_out)
     OH, OW = layer.output_size(x.size(2), x.size(3))
     eps = _draw(tape, "normal", (x.size(0), layer.n_out, OH, OW), x.device)
-    out = MnfConvOutFn.apply(x, z[0], layer.W_mean, layer.W_log_var, layer.b_log_var, eps, layer.padding, layer.stride)
+    out = MnfConvOutFn.apply(x, z[0], layer.W_mean, layer.W_log_var, layer.b_log_var, eps, layer.padding, layer.stride,
+                             layer.dilation, layer.groups)
     return torch.nn.functional.max_pool2d(torch.relu(out), 2) if relu_pool else out
 
 

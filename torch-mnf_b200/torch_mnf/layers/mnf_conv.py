@@ -22,19 +22,25 @@ def _check_int(name, value, least):
 class MNFConv2d(nn.Module):
     """Bayesian conv layer.  One z [n_out] per call, shared by the batch, scales the output channels
     of the mean path; out = conv(x, W_mean*z) + sqrt(conv(x^2, exp(W_log_var)) + exp(b_log_var)) * eps,
-    computed as one implicit-GEMM CUDA kernel.  ``padding`` (zeros) and ``stride`` mean what they
-    mean for ``torch.nn.functional.conv2d``; the reference has neither (padding=0, stride=1).
-    They are geometry, not parameters: the state_dict and kl_div do not depend on them.
+    computed as one implicit-GEMM CUDA kernel.  ``padding`` (zeros), ``stride``, ``dilation`` and
+    ``groups`` mean what they mean for ``torch.nn.functional.conv2d``; the reference has none of them
+    (padding=0, stride=1, dilation=1, groups=1).  Padding, stride and dilation are geometry, not
+    parameters: the state_dict and kl_div do not depend on them.  ``groups`` splits the channels
+    into groups that do not mix: W_mean / W_log_var are [n_out, n_in // groups, k, k].
     ``b_mean`` is a fixed zero tensor and not part of the state_dict, as in the reference."""
 
     __getstate__ = state_without_caches  # copy.deepcopy / pickle drop cached device scratch
 
     def __init__(self, n_in: int, n_out: int, kernel_size: int, n_flows_q: int = 2, n_flows_r: int = 2,
-                 h_sizes: Sequence[int] = (50,), *, padding: int = 0, stride: int = 1) -> None:
+                 h_sizes: Sequence[int] = (50,), *, padding: int = 0, stride: int = 1, dilation: int = 1,
+                 groups: int = 1) -> None:
         super().__init__()
         self.padding, self.stride = _check_int("padding", padding, 0), _check_int("stride", stride, 1)
+        self.dilation, self.groups = _check_int("dilation", dilation, 1), _check_int("groups", groups, 1)
+        if n_in % groups or n_out % groups:
+            raise ValueError(f"MNFConv2d: groups={groups} must divide n_in={n_in} and n_out={n_out}")
         self.n_in, self.n_out, self.kernel_size = n_in, n_out, kernel_size
-        shape = [n_out, n_in, kernel_size, kernel_size]
+        shape = [n_out, n_in // groups, kernel_size, kernel_size]
         self.W_mean = nn.Parameter(0.1 * torch.randn(shape))
         self.W_log_var = nn.Parameter(-9 + 0.1 * torch.randn(shape))
         self.register_buffer("b_mean", torch.zeros(n_out), persistent=False)
@@ -48,14 +54,20 @@ class MNFConv2d(nn.Module):
         self.flow_r = flows.NormalizingFlow([flows.RNVP(n_out, h_sizes=h_sizes) for _ in range(n_flows_r)])
 
     def extra_repr(self) -> str:
-        return (f"{self.n_in}, {self.n_out}, kernel_size={self.kernel_size}, padding={self.padding}, "
-                f"stride={self.stride}")
+        s = f"{self.n_in}, {self.n_out}, kernel_size={self.kernel_size}, padding={self.padding}, stride={self.stride}"
+        if self.dilation != 1:
+            s += f", dilation={self.dilation}"
+        if self.groups != 1:
+            s += f", groups={self.groups}"
+        return s
 
     def output_size(self, height: int, width: int) -> tuple[int, int]:
         """(OH, OW) of this layer on height x width inputs; ValueError when the output would be empty."""
-        k, p, s = self.kernel_size, self.padding, self.stride
+        p, s = self.padding, self.stride
+        k = self.dilation * (self.kernel_size - 1) + 1  # extent of the dilated filter
         if height + 2 * p < k or width + 2 * p < k:
-            raise ValueError(f"MNFConv2d: kernel_size {k} is larger than the {height}x{width} input padded by {p}")
+            raise ValueError(f"MNFConv2d: kernel_size {self.kernel_size} (extent {k} at dilation {self.dilation}) "
+                             f"is larger than the {height}x{width} input padded by {p}")
         return (height + 2 * p - k) // s + 1, (width + 2 * p - k) // s + 1
 
     def sample_z(self, noise=None):
