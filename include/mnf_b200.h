@@ -595,7 +595,9 @@ int mnf_rnvp_gate_backward(const float *z, const float *mask, const float *shift
 /* Weight-sized part of MNFLinear.kl_div (mnf_linear.py:67-79) with injected eps_w [n_out, n_in]:
  *   pre[j] = sum_i (W_mean[j,i] z_i + exp(W_log_var[j,i]/2) eps_w[j,i]) r0_c[i]   (the tanh argument, :77)
  *   kl_rows[j] = 0.5 sum_i (-W_log_var + exp(W_log_var) + (W_mean z)^2 - 1)       (kl_div_W = sum_j, :72)
- * and the adjoint (grad_W_* overwritten, grad_z / grad_r0_c overwritten). */
+ * and the adjoint (grad_W_* overwritten, grad_z / grad_r0_c overwritten).  Negative sizes: MNF_E_ARG; an empty
+ * problem returns 0 (with n_out = 0 the adjoint zeroes grad_z / grad_r0_c, with n_in = 0 the forward zeroes pre and
+ * kl_rows). */
 int mnf_kl_rows_forward(const float *z, const float *W_mean, const float *W_log_var, const float *r0_c, const float *eps_w,
                         float *pre, float *kl_rows, int n_out, int n_in, void *stream);
 int mnf_kl_rows_backward(const float *z, const float *W_mean, const float *W_log_var, const float *r0_c,

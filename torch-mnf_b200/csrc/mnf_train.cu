@@ -415,6 +415,8 @@ int mnf_rnvp_gate_backward(const float *z, const float *mask, const float *shift
 int mnf_kl_rows_forward(const float *z, const float *W_mean, const float *W_log_var, const float *r0_c, const float *eps_w,
                         float *pre, float *kl_rows, int n_out, int n_in, void *stream) {
     MNF_REQUIRE(z && W_mean && W_log_var && r0_c && eps_w && pre && kl_rows, MNF_E_ARG, "NULL pointer");
+    MNF_REQUIRE(n_out >= 0 && n_in >= 0, MNF_E_ARG, "negative size n_out=%d n_in=%d", n_out, n_in);
+    if (n_out == 0) return 0;  // n_in == 0 still writes the empty sums: pre = kl_rows = 0
     const long long threads = (long long)n_out * 32;
     kl_rows_fwd_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(z, W_mean, W_log_var, r0_c, eps_w,
                                                                                           pre, kl_rows, n_out, n_in);
@@ -427,9 +429,12 @@ int mnf_kl_rows_backward(const float *z, const float *W_mean, const float *W_log
     MNF_REQUIRE(z && W_mean && W_log_var && r0_c && eps_w && grad_pre && grad_kl_rows && grad_W_mean && grad_W_log_var &&
                     grad_z && grad_r0_c,
                 MNF_E_ARG, "NULL pointer");
+    MNF_REQUIRE(n_out >= 0 && n_in >= 0, MNF_E_ARG, "negative size n_out=%d n_in=%d", n_out, n_in);
+    if (n_in == 0) return 0;
     cudaStream_t st = (cudaStream_t)stream;
     MNF_CUDA(cudaMemsetAsync(grad_z, 0, sizeof(float) * n_in, st));
     MNF_CUDA(cudaMemsetAsync(grad_r0_c, 0, sizeof(float) * n_in, st));
+    if (n_out == 0) return 0;  // grad_z = grad_r0_c = 0, no weights
     int gy = (n_out + 31) / 32;
     if (gy > 64) gy = 64;
     kl_rows_bwd_kernel<<<dim3((n_in + 127) / 128, gy), 128, 0, st>>>(z, W_mean, W_log_var, r0_c, eps_w, grad_pre,
