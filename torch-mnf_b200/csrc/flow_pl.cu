@@ -485,9 +485,21 @@ __device__ __forceinline__ const float4 *piece_row(const float *tb, bool fast, f
     return reinterpret_cast<const float4 *>(tb + BP_FLOATS) + find_piece<SM>(tb, c) * stride4;
 }
 
+// MNF_FPL_ABLATE selects a timing ablation of the spline conditioner (tools/bench_flow_pl_pipes.py; its outputs are
+// wrong by construction): 1 every ex2 becomes a multiply (no XU work for the exponentials), 2 the bin selection is
+// short-circuited to a fixed bin, 3 the knot derivatives are constant.  0, the only value the library is built with,
+// leaves the kernel as it is.
+#ifndef MNF_FPL_ABLATE
+#define MNF_FPL_ABLATE 0
+#endif
+
 __device__ __forceinline__ float ex2_approx(float x) {
     float r;
+#if MNF_FPL_ABLATE == 1
+    asm("mul.f32 %0, %1, 0f3F7FFFFE;" : "=f"(r) : "f"(x));
+#else
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(x));
+#endif
     return r;
 }
 __device__ __forceinline__ float sqrt_approx(float x) {
@@ -514,8 +526,9 @@ __device__ __forceinline__ float knot_const(float k) { return fmaf(2.f * kMinBin
 // sum lies in [1, K 2^FAST_T] and, with the second softmax's arguments centred on 0, every second-softmax sum in
 // [e^-B, K e^B], so each pair of sums is inverted by one reciprocal of its product.  Otherwise (natural units) the
 // largest output of each axis is subtracted first.
+// X[k]: the second softmax's (width, height) terms, S[k] = X[0] + .. + X[k] summed in that order.
 template <int K, bool FAST>
-__device__ __forceinline__ void unit_knots(const float *raw, float twoB, float2 *S, float2 &c1) {
+__device__ __forceinline__ void unit_knots(const float *raw, float twoB, float2 *X, float2 *S, float2 &c1) {
     constexpr float span = 1.f - kMinBin * (float)K;
     float2 e[K], sc, off;
     if constexpr (FAST) {
@@ -545,8 +558,8 @@ __device__ __forceinline__ void unit_knots(const float *raw, float twoB, float2 
 #pragma unroll
     for (int k = 0; k < K; ++k) {
         const float2 a = f2_fma(e[k], sc, off);
-        const float2 x = make_float2(ex2_approx(a.x), ex2_approx(a.y));
-        p = k ? f2_add(p, x) : x;
+        X[k] = make_float2(ex2_approx(a.x), ex2_approx(a.y));
+        p = k ? f2_add(p, X[k]) : X[k];
         if (k + 1 < K) S[k] = p;
     }
     if constexpr (FAST) {
@@ -557,9 +570,10 @@ __device__ __forceinline__ void unit_knots(const float *raw, float twoB, float2 
     }
 }
 
-// flow_math.cuh::knot_derivative (FAST flavour) of a raw output given in log2 units
+// flow_math.cuh::knot_derivative (FAST flavour) of a raw output given in log2 units, without a branch: lg2(2 + 2^r) is r to
+// fp32 precision above 20 log2(e), where the clamp keeps ex2 finite and the max returns r itself.
 __device__ __forceinline__ float knot_derivative_log2(float r) {
-    return fmaf(LN2, r > 20.f * LOG2E ? r : lg2_approx(2.f + ex2_approx(r)), kMinDeriv);
+    return fmaf(LN2, fmaxf(r, lg2_approx(2.f + ex2_approx(fminf(r, 20.f * LOG2E)))), kMinDeriv);
 }
 
 // Log-det of the spline conditioners of a point as a running product P in [1, 2) times 2^E: one lg2 per point at the end
@@ -587,38 +601,49 @@ __device__ __forceinline__ void ld_flush(float &ld, float &P, int &E) {
 template <int K, bool FAST, bool INV, class DerivFn>
 __device__ __forceinline__ void rq_spline_lazy(const float *raw, float B, float inv_B, float edge_deriv, float &v, float &P, int &E,
                                                DerivFn deriv) {
-    float2 S[K - 1], c1;
-    unit_knots<K, FAST>(raw, 2.f * B, S, c1);
+    float2 X[K], S[K - 1], c1;
+    unit_knots<K, FAST>(raw, 2.f * B, X, S, c1);
     const float u = v * inv_B;
     // bin = number of interior knots <= u (spline_flow.py:22-24,115-118; u lies inside [t_0, t_K], so the count needs no
-    // clamp).  Only the searched axis's knots are formed; the prefix sums at both ends of the bin are picked for both axes
-    // with the same predicates, and the knots made from them afterwards.
-    int idx = 0;
-    float2 lo = f2_splat(0.f), hi = S[0];
+    // clamp).  Only the searched axis's knots are formed.  Each compare gives a mask m_k in {0, 1}, non-increasing in k, so
+    // the prefix sums at both ends of the bin are masked sums of the terms X in the order S was summed: lo = S[idx - 1]
+    // (0 for idx = 0) and hi = S[idx] bit for bit, one FFMA2 per knot and end for both axes.  The knots are made from them
+    // afterwards.
+    float fidx = 0.f;
+    float2 lo = f2_splat(0.f), hi = X[0];
+#if MNF_FPL_ABLATE == 2
+    fidx = (float)(K / 2), lo = S[K / 2 - 1], hi = S[K / 2];
+#else
 #pragma unroll
     for (int k = 1; k < K; ++k) {
-        const bool ge = u >= fmaf(INV ? S[k - 1].y : S[k - 1].x, INV ? c1.y : c1.x, knot_const((float)k));
-        idx += ge ? 1 : 0;
-        lo = ge ? S[k - 1] : lo;
-        if (k + 1 < K) hi = ge ? S[k] : hi;  // (the last bin's upper knots are pinned)
+        const float m = u >= fmaf(INV ? S[k - 1].y : S[k - 1].x, INV ? c1.y : c1.x, knot_const((float)k)) ? 1.f : 0.f;
+        fidx += m;
+        lo = f2_fma(f2_splat(m), X[k - 1], lo);
+        if (k + 1 < K) hi = f2_fma(f2_splat(m), X[k], hi);  // (the last bin's upper knots are pinned)
     }
-    const float fidx = __int_as_float(0x4b000000 | idx) - 8388608.f;  // (float)idx without the XU pipe
+#endif
+    const int idx = __float_as_int(fidx + 8388608.f) - 0x4b000000;  // (int)fidx without the XU pipe
     const float k0 = knot_const(fidx), k1 = knot_const(fidx + 1.f);
-    const float xk = fmaf(lo.x, c1.x, k0), yk = fmaf(lo.y, c1.y, k0);
+    const float2 lk = f2_fma(lo, c1, f2_splat(k0)), hk2 = f2_fma(hi, c1, f2_splat(k1));
+    const float xk = lk.x, yk = lk.y;
     const bool last = idx == K - 1;
-    const float xk1 = last ? 1.f : fmaf(hi.x, c1.x, k1), yk1 = last ? 1.f : fmaf(hi.y, c1.y, k1);
+    const float xk1 = last ? 1.f : hk2.x, yk1 = last ? 1.f : hk2.y;
     const float wk = xk1 - xk, hk = yk1 - yk;  // spline_flow.py:102,113
     // interior knot derivatives (spline_flow.py:256,104), the padded constant at the two ends (:46-49); the loads are
     // unconditional on a clamped index so that lanes in different bins do not diverge
     const float r0 = deriv(max(idx - 1, 0)), r1 = deriv(min(idx, K - 2));
     float dk, dk1;
-    if constexpr (FAST) {
-        dk = (idx > 0) ? knot_derivative_log2(r0) : edge_deriv;
-        dk1 = (idx < K - 1) ? knot_derivative_log2(r1) : edge_deriv;
+    if constexpr (FAST) {  // both formed, then selected: no branch around the MUFU work
+        const float d0 = knot_derivative_log2(r0), d1 = knot_derivative_log2(r1);
+        dk = idx > 0 ? d0 : edge_deriv;
+        dk1 = idx < K - 1 ? d1 : edge_deriv;
     } else {
         dk = (idx > 0) ? knot_derivative<true>(r0) : edge_deriv;
         dk1 = (idx < K - 1) ? knot_derivative<true>(r1) : edge_deriv;
     }
+#if MNF_FPL_ABLATE == 3
+    dk = dk1 = edge_deriv;
+#endif
     // Reciprocals are rcp.approx.ftz, which differs from __fdividef only where the operand is not a normal number; every
     // operand below is a product or sum of bin widths and heights (>= 2 min_bin), knot derivatives (>= min_deriv) and
     // terms in [0, 1], so it is not below the normal range.  (-b - sqrt(disc) is -2 hk dk wk at dy = 0 and grows in
