@@ -292,6 +292,32 @@ int mnf_linear_forward_affine(const float *x, int64_t x_rows, const float *z, co
                               float *out, int64_t n_rows, int n_in, int n_out, int relu,
                               const float *col_scale, const float *col_shift, void *stream);
 
+/* Posterior function samples of MNFLinear: one weight draw per sample, shared by every input row.
+ *   W_out[s] = W_mean * z[s][None, :] + exp(0.5 * W_log_var) * E[s]      [n_samples, n_out, n_in]
+ *   b_out[s] = b_mean + exp(0.5 * b_log_var) * e[s]                      [n_samples, n_out]
+ * z: [n_samples, n_in], row s of MNFLinear.sample_z(n_samples) drawn with row_offset = sample_offset.  eps_w
+ * [n_samples, n_out, n_in] and eps_b [n_samples, n_out] may each be NULL: Philox keyed by `seed`, stream
+ * w_noise_stream / b_noise_stream, with the 64-bit GLOBAL element indices
+ *   E: ((sample_offset + s) * n_out + o) * n_in + i,      e: (sample_offset + s) * n_out + o
+ * (the unit of the offset is the sample), so a sample depends only on (seed, sample_offset + s), and calls over
+ * consecutive sample blocks reproduce one call bit for bit.  The normals are philox_normal's: one Philox block serves
+ * four consecutive elements.  n_samples = 0 is a no-op; an element index past 2^63 is MNF_E_SHAPE. */
+int mnf_linear_sample_weights(const float *W_mean, const float *W_log_var, const float *b_mean,
+                              const float *b_log_var, const float *z, const float *eps_w, const float *eps_b,
+                              uint64_t seed, uint32_t w_noise_stream, uint32_t b_noise_stream,
+                              uint64_t sample_offset, float *W_out, float *b_out, int64_t n_samples, int n_in,
+                              int n_out, void *stream);
+/* The function GEMM over the weight image of mnf_linear_sample_weights, exact fp32:
+ *   out[s, m, :] = x_s[m] @ W[s]^T + b[s], then relu (1 = nn.ReLU), then the optional per-column affine map of
+ *   mnf_linear_forward_affine (col_scale / col_shift both [n_out] or both NULL)
+ * x_per_sample = 0: x [batch, n_in] is shared by every sample (x_s = x); 1: x [n_samples, batch, n_in], one block per
+ * sample (x_s = x[s]).  W [n_samples, n_out, n_in], b [n_samples, n_out], out [n_samples, batch, n_out].  Every batch
+ * size runs the same tiled kernel, so a row's output does not depend on the other rows of the call.  At most 65535
+ * samples per call (they run on grid dimension z; MNF_E_SHAPE beyond). */
+int mnf_linear_function_forward(const float *x, int x_per_sample, const float *W, const float *b, float *out,
+                                int64_t n_samples, int64_t batch, int n_in, int n_out, int relu,
+                                const float *col_scale, const float *col_shift, void *stream);
+
 /* Tensor-core (tcgen05, TF32 inputs, fp32 accumulation in TMEM, TMA-fed) variant of mnf_linear_forward
  * for n_in % 4 == 0 and 16-byte aligned operands; results agree with the fp32 path to the 2e-3 relative
  * tolerance BASELINE.json states for tensor-core GEMM outputs.  workspace: mnf_linear_tc_workspace()

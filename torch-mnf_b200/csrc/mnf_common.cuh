@@ -247,11 +247,12 @@ __global__ void __launch_bounds__(128) simt_gemv_kernel(const Prob p) {
 }
 
 // batches > 1: that many independent problems of the same shape on grid dimension z; the functor tells them apart by
-// blockIdx.z (the groups of a grouped convolution)
+// blockIdx.z (the groups of a grouped convolution).  gemv_ok = false keeps the tiled form for every M, so that a row's
+// sum runs in the same order whatever the number of rows in the call.
 template <class Prob, int NACC>
-int launch_simt_gemm(const Prob &p, cudaStream_t stream, const char *what, int batches = 1) {
+int launch_simt_gemm(const Prob &p, cudaStream_t stream, const char *what, int batches = 1, bool gemv_ok = true) {
     if (p.M <= 0 || p.N <= 0) return 0;
-    if (p.M <= 4 && p.K >= 256) {
+    if (gemv_ok && p.M <= 4 && p.K >= 256) {
         simt_gemv_kernel<Prob, NACC><<<dim3((unsigned)p.N, 1, (unsigned)batches), 128, 0, stream>>>(p);
         return launch_status(what);
     }

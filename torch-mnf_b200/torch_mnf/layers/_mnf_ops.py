@@ -62,6 +62,9 @@ _lib.register({
                                   _int, _int, _vp]),
     "mnf_linear_forward_affine": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int,
                                          _int, _int, _vp, _vp, _vp]),
+    "mnf_linear_sample_weights": (_int, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u32, _u64, _vp, _vp, _i64, _int,
+                                         _int, _vp]),
+    "mnf_linear_function_forward": (_int, [_vp, _int, _vp, _vp, _vp, _i64, _i64, _int, _int, _int, _vp, _vp, _vp]),
     "mnf_conv2d_forward": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int, _int,
                                   _int, _int, _int, _int, _vp]),
     "mnf_conv2d_forward_ps": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, _u64, _u32, _u64, _vp, _i64, _int, _int,
@@ -345,6 +348,98 @@ def linear_forward(layer, x, z, noise: Noise, x_rows=None, relu=False, precision
                                                   out.data_ptr(), R, n_in, n_out, int(relu), _p(scale), _p(shift),
                                                   _lib.stream_ptr(dev))
     _lib.check(rc, "mnf_linear_forward")
+    _lib.launch_count += 1
+    return out
+
+
+#: bytes of one chunk's weight image [S_c, n_out, n_in] when function samples run without a tape: small enough to stay
+#: in the B200's 126 MB L2 between the weight draw that writes it and the function GEMM that reads it
+FUNCTION_IMAGE_BYTES = 64 << 20
+
+
+def function_chunk(weights_per_sample: int) -> int:
+    """Samples per chunk of a function-sample call: FUNCTION_IMAGE_BYTES of weights, at least one sample, at most the
+    65535 of one function GEMM launch."""
+    return max(1, min(65535, FUNCTION_IMAGE_BYTES // (4 * weights_per_sample)))
+
+
+def check_function_args(n_samples, sample_offset, chunk=None):
+    """ValueError for n_samples < 1, chunk < 1 or a negative sample_offset -- before any device work."""
+    if int(n_samples) < 1:
+        raise ValueError(f"n_samples must be positive, got {n_samples}")
+    if chunk is not None and int(chunk) < 1:
+        raise ValueError(f"chunk must be positive, got {chunk}")
+    if int(sample_offset) < 0:
+        raise ValueError(f"sample_offset must be non-negative, got {sample_offset}")
+
+
+def function_input(x, n_in, n_samples):
+    """x [B, n_in] (shared by the samples) or [n_samples, B, n_in] (one block per sample), CUDA fp32, contiguous."""
+    if not isinstance(x, torch.Tensor):
+        raise TypeError("input must be a torch.Tensor")
+    if x.dim() == 2:
+        ok = x.size(1) == n_in
+    elif x.dim() == 3:
+        ok = x.size(0) == n_samples and x.size(2) == n_in
+    else:
+        ok = False
+    if not ok:
+        raise ValueError(f"input of shape {tuple(x.shape)}: expected [B, {n_in}] or [{n_samples}, B, {n_in}]")
+    return _lib.require_cuda_f32(x, "input")
+
+
+#: rows of the z draw of a function-sample call at the least: mnf_rnvp_forward runs one row on its cluster kernel and at
+#: most 4 rows of a wide layer on the GEMV form, both summing in another order than the tiled GEMM, so fewer rows would
+#: make a sample's z depend on how many samples the call draws
+Z_MIN_ROWS = 5
+
+
+@torch.no_grad()
+def linear_function_z(layer, n_samples, noise: Noise, sample_offset=0):
+    """z [S, n_in] of S posterior function samples: rows sample_offset .. sample_offset + S - 1 of MNFLinear.sample_z
+    (normal[S, n_in], one Bernoulli[S, n_in] per q-flow).  Without a tape at least Z_MIN_ROWS rows are drawn (the extra
+    rows are the next samples' z and are dropped), so a sample's z does not depend on S."""
+    rows = n_samples if noise.tape is not None else max(n_samples, Z_MIN_ROWS)
+    return conv_sample_z_rows(layer, rows, noise, sample_offset)[:n_samples]
+
+
+@torch.no_grad()
+def linear_sample_weights(layer, z, noise: Noise, sample_offset=0):
+    """Posterior weight draws of an MNFLinear for the S rows of z (linear_function_z): (W [S, n_out, n_in], b [S, n_out])
+    from the next two draws of noise, normal[S, n_out, n_in] (E) and normal[S, n_out] (e); Philox elements are keyed by
+    the global sample index sample_offset + s."""
+    dev = noise.device
+    n_out, n_in = layer.W_mean.shape
+    n_samples = z.size(0)
+    eps_w, sid_w = noise.normal((n_samples, n_out, n_in))
+    eps_b, sid_b = noise.normal((n_samples, n_out))
+    W = torch.empty((n_samples, n_out, n_in), device=dev, dtype=torch.float32)
+    b = torch.empty((n_samples, n_out), device=dev, dtype=torch.float32)
+    args = [_param(getattr(layer, n), dev, n) for n in ("W_mean", "W_log_var", "b_mean", "b_log_var")]
+    with _lib.on_device(dev):
+        rc = _lib.lib().mnf_linear_sample_weights(*(a.data_ptr() for a in args), z.data_ptr(), _p(eps_w), _p(eps_b),
+                                                  noise.seed, sid_w, sid_b, int(sample_offset), W.data_ptr(),
+                                                  b.data_ptr(), n_samples, n_in, n_out, _lib.stream_ptr(dev))
+    _lib.check(rc, "mnf_linear_sample_weights")
+    _lib.launch_count += 1
+    return W, b
+
+
+@torch.no_grad()
+def linear_function_forward(x, W, b, relu=False, affine=None, out=None):
+    """out [S, B, n_out] = x_s @ W[s]^T + b[s] (then ReLU, then the folded batch norm ``affine`` = (col_scale,
+    col_shift)); x [B, n_in] shared by the samples or [S, B, n_in]."""
+    dev = x.device
+    S, n_out, n_in = W.shape
+    B = x.size(-2)
+    scale, shift = affine if affine is not None else (None, None)
+    if out is None:
+        out = torch.empty((S, B, n_out), device=dev, dtype=torch.float32)
+    with _lib.on_device(dev):
+        rc = _lib.lib().mnf_linear_function_forward(x.data_ptr(), int(x.dim() == 3), W.data_ptr(), b.data_ptr(),
+                                                    out.data_ptr(), S, B, n_in, n_out, int(relu), _p(scale), _p(shift),
+                                                    _lib.stream_ptr(dev))
+    _lib.check(rc, "mnf_linear_function_forward")
     _lib.launch_count += 1
     return out
 

@@ -89,6 +89,57 @@ class MNFLinear(nn.Module):
         x = _lib.require_cuda_f32(x, "input")
         return self._forward_rows(x, x.size(0) * n_samples, self._noise(noise, x.device, row_offset), relu)
 
+    def _function_noise(self, noise, seed, device):
+        """Noise of a function-sample call: ``noise`` (a tape or an ops.Noise) as given, else Philox keyed by ``seed``
+        (drawn from torch's generator when None; a device tape under CUDA-graph capture, as ops.Noise does)."""
+        return noise if isinstance(noise, ops.Noise) else ops.Noise(noise, device, seed=seed)
+
+    @torch.no_grad()
+    def sample_weights(self, n_samples, seed=None, sample_offset=0, noise=None):
+        """``n_samples`` draws of the layer's weights from the posterior: (W [S, n_out, n_in], b [S, n_out]) with
+        W_s = W_mean * z_s[None, :] + exp(0.5 W_log_var) * E_s and b_s = b_mean + exp(0.5 b_log_var) * e_s, z_s row s
+        of sample_z(S).  Draws, in order: normal[S, n_in] and one Bernoulli[S, n_in] per q-flow (sample_z with
+        row_offset = sample_offset), normal[S, n_out, n_in] (E), normal[S, n_out] (e).  Philox elements are keyed by
+        ``(seed, sample_offset + s)``, so a sample does not depend on how the samples are split between calls."""
+        ops.check_function_args(n_samples, sample_offset)
+        dev = self.W_mean.device
+        if dev.type != "cuda":
+            raise RuntimeError("torch_mnf (B200) runs only on CUDA parameters (no CPU fallback)")
+        noise = self._function_noise(noise, seed, dev)
+        z = ops.linear_function_z(self, int(n_samples), noise, int(sample_offset))
+        return ops.linear_sample_weights(self, z, noise, int(sample_offset))
+
+    @torch.no_grad()
+    def forward_functions(self, x, n_samples, seed=None, sample_offset=0, noise=None, relu=False):
+        """The layer under ``n_samples`` posterior weight draws (those of ``sample_weights``): [S, B, n_out] with
+        out[s] = x_s @ W_s^T + b_s, every input row of sample s through the same W_s, b_s.  x: [B, n_in], shared by the
+        samples, or [S, B, n_in], one block per sample.  ``relu`` applies a ReLU in the GEMM's epilogue.  Exact fp32
+        whatever ``precision`` says.  Row s * B + b of ``out.view(S * B, n_out)`` is sample s of input b, the layout of
+        forward_mc."""
+        ops.check_function_args(n_samples, sample_offset)
+        x = ops.function_input(x, self.n_in, int(n_samples))
+        return self._functions(x, int(n_samples), self._function_noise(noise, seed, x.device), int(sample_offset),
+                               relu)
+
+    def _functions(self, x, n_samples, noise, sample_offset, relu=False, affine=None, chunk=None):
+        """forward_functions on a Noise: z of all samples in one draw, then chunk by chunk the weight image
+        (mnf_linear_sample_weights) and the function GEMM.  Without a tape every chunk takes the same two stream ids
+        for E and e, its Philox elements keyed by its global samples; a tape is consumed in one chunk.  affine: the
+        folded batch norm of the GEMM's epilogue."""
+        if noise.tape is not None:
+            chunk = n_samples
+        elif chunk is None:
+            chunk = ops.function_chunk(self.n_out * (self.n_in + 1))
+        z = ops.linear_function_z(self, n_samples, noise, sample_offset)
+        out = torch.empty((n_samples, x.size(-2), self.n_out), device=x.device, dtype=torch.float32)
+        weight_stream = noise.streams
+        for c in range(0, n_samples, chunk):
+            k = min(chunk, n_samples - c)
+            noise.streams = weight_stream
+            W, b = ops.linear_sample_weights(self, z[c:c + k], noise, sample_offset + c)
+            ops.linear_function_forward(x[c:c + k] if x.dim() == 3 else x, W, b, relu, affine, out=out[c:c + k])
+        return out
+
     def kl_div(self, noise=None):
         if _train.needs_grad(self):
             return _train.linear_kl_div(self, noise)

@@ -188,14 +188,47 @@ class MNFFeedForward(nn.Sequential):
             return sums, entropy_sums
         return uncertainty_from_sums(sums, entropy_sums, n_samples)
 
-    def _mc_sums(self, x, n_samples, chunk, seed, sample_range, softmax, entropy):
-        """The chunk loop of predict / predict_uncertainty: fp64 sums [2, B, n_out] and, with ``entropy``, the entropy
-        sums [B] (else None) of samples lo..hi-1."""
+    def _require_running_stats(self):
         for m in self:
             if isinstance(m, nn.modules.batchnorm._BatchNorm) and not self._uses_running_stats(m):
                 raise RuntimeError("MNFFeedForward.predict needs every BatchNorm1d in eval mode with running statistics "
                                    "(call model.eval()): batch statistics of a chunk of samples are not those of the "
                                    "whole replicated batch")
+
+    @torch.no_grad()
+    def forward_functions(self, x, n_samples: int, seed=None, sample_offset: int = 0, chunk: int | None = None,
+                          noise=None):
+        """The network under ``n_samples`` posterior function draws: [S, B, n_out_last], out[s] = f_s(x) with every layer
+        evaluated on its weights of sample s (MNFLinear.sample_weights), shared by all rows of x [B, n_in] (or of its
+        block x[s] when x is [S, B, n_in]).
+
+        One noise source is shared by the layers, which draw in layer order as ``MNFLinear.forward_functions`` does
+        (1 + n_flows_q + 2 draws each), from the tape ``noise`` or from Philox keyed by ``(seed, sample_offset + s)``:
+        the result does not depend on x, the batch size, ``chunk`` or a split of the samples between calls.  The layers
+        run one after the other over all samples; in each, the weight images are drawn and applied ``chunk`` samples at
+        a time (default: about ops.FUNCTION_IMAGE_BYTES of weights; a tape runs as one chunk).  Blocks with ``nn.ReLU``
+        and an eval-mode BatchNorm1d run both in the function GEMM's epilogue, other activations are applied by their
+        modules.  Needs every BatchNorm1d in eval mode with running statistics, as ``predict`` does: batch statistics
+        would mix the samples."""
+        ops.check_function_args(n_samples, sample_offset, chunk)
+        self._require_running_stats()
+        blocks = self._blocks()
+        n_samples, sample_offset = int(n_samples), int(sample_offset)
+        x = ops.function_input(x, blocks[0][0].n_in, n_samples)
+        nz = noise if isinstance(noise, ops.Noise) else ops.Noise(noise, x.device, seed=seed)
+        h = x
+        for i, (lin, act, bn) in enumerate(blocks):
+            relu = type(act) is nn.ReLU
+            affine = self._folded(i, bn, x.device) if relu else None
+            h = lin._functions(h, n_samples, nz, sample_offset, relu=relu, affine=affine, chunk=chunk)
+            if act is not None and affine is None:
+                h = bn(act(h.view(-1, h.size(-1)))).view(h.shape)
+        return h
+
+    def _mc_sums(self, x, n_samples, chunk, seed, sample_range, softmax, entropy):
+        """The chunk loop of predict / predict_uncertainty: fp64 sums [2, B, n_out] and, with ``entropy``, the entropy
+        sums [B] (else None) of samples lo..hi-1."""
+        self._require_running_stats()
         x = _lib.require_cuda_f32(x, "input")
         B = x.size(0)
         lo, hi = (0, n_samples) if sample_range is None else sample_range
