@@ -105,3 +105,40 @@ def load_flow_model_unloaded(specs):
 
     dim = specs[0]["dim"]
     return nf.NormalizingFlowModel(MultivariateNormal(torch.zeros(dim), torch.eye(dim)), [build_flow(s) for s in specs])
+
+
+# ---------------------------------------------------------------------------
+# oracle flow stacks that torch autograd can differentiate
+# ---------------------------------------------------------------------------
+def nsf_ar_forward_functional(p, spec, v):
+    """oracle.flows_cpu.nsf_ar(inverse=False) without the in-place column writes: the reference's NSF_AR.forward
+    (spline_flow.py:199-216) assigns x[:, i] in place after x[:, :i] fed the conditioner, which torch autograd rejects, so
+    the reference itself cannot differentiate this direction; the CUDA backward can, and is checked against this."""
+    from oracle import flows_cpu
+
+    d, K, B = spec["dim"], spec["K"], spec["B"]
+    cols, ld = [], torch.zeros(v.shape[0], dtype=v.dtype)
+    for i in range(d):
+        raw = (p["init_param"].expand(v.shape[0], 3 * K - 1) if i == 0
+               else flows_cpu.mlp(flows_cpu.sub(p, f"layers.{i - 1}."), torch.stack(cols, 1)))
+        W, H, D = flows_cpu._spline_params(raw, K, B)
+        col, l = flows_cpu.unconstrained_rqs(v[:, i], W, H, D, True, B)
+        cols.append(col)
+        ld = ld + l
+    return torch.stack(cols, 1), ld
+
+
+def oracle_stack(sd, specs, v, inverse):
+    """oracle.flows_cpu.stack, with NSF_AR.forward replaced by its autograd-friendly form."""
+    from oracle import flows_cpu
+
+    if inverse or not any(s["type"] == "NSF_AR" for s in specs):
+        return flows_cpu.stack(sd, specs, v, inverse)
+    ld, outs = torch.zeros(v.size(0), dtype=v.dtype), [v]
+    for i, spec in enumerate(specs):
+        p = flows_cpu.sub(sd, f"flows.{i}.")
+        v, l = (nsf_ar_forward_functional(p, spec, v) if spec["type"] == "NSF_AR"
+                else flows_cpu.apply_flow(p, spec, v, False))
+        ld = ld + l
+        outs.append(v)
+    return outs, ld

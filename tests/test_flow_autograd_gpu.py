@@ -5,8 +5,7 @@ through torch autograd (tests/test_flows.py:14-31) -- so the oracle + autograd I
 import pytest
 import torch
 
-from oracle import flows_cpu
-from tests.helpers import golden_sd, golden_spec, load_flow_model, load_golden, t
+from tests.helpers import golden_sd, golden_spec, load_flow_model, load_golden, oracle_stack, t
 
 pytestmark = pytest.mark.gpu
 
@@ -19,35 +18,6 @@ CASES = [  # (fixture, directions)
     ("maf_iaf_d2", ("inv", "fwd")),
     ("affine_misc_d4", ("inv", "fwd")),
 ]
-
-
-def _nsf_ar_forward_functional(p, spec, v):
-    """oracle.flows_cpu.nsf_ar(inverse=False) without the in-place column writes: the reference's NSF_AR.forward
-    (spline_flow.py:199-216) assigns x[:, i] in place after x[:, :i] fed the conditioner, which torch autograd rejects, so
-    the reference itself cannot differentiate this direction; the CUDA backward can, and is checked against this."""
-    d, K, B = spec["dim"], spec["K"], spec["B"]
-    cols, ld = [], torch.zeros(v.shape[0], dtype=v.dtype)
-    for i in range(d):
-        raw = (p["init_param"].expand(v.shape[0], 3 * K - 1) if i == 0
-               else flows_cpu.mlp(flows_cpu.sub(p, f"layers.{i - 1}."), torch.stack(cols, 1)))
-        W, H, D = flows_cpu._spline_params(raw, K, B)
-        col, l = flows_cpu.unconstrained_rqs(v[:, i], W, H, D, True, B)
-        cols.append(col)
-        ld = ld + l
-    return torch.stack(cols, 1), ld
-
-
-def _oracle_stack(sd, specs, v, inverse):
-    if inverse or not any(s["type"] == "NSF_AR" for s in specs):
-        return flows_cpu.stack(sd, specs, v, inverse)
-    ld, outs = torch.zeros(v.size(0), dtype=v.dtype), [v]
-    for i, spec in enumerate(specs):
-        p = flows_cpu.sub(sd, f"flows.{i}.")
-        v, l = (_nsf_ar_forward_functional(p, spec, v) if spec["type"] == "NSF_AR"
-                else flows_cpu.apply_flow(p, spec, v, False))
-        ld = ld + l
-        outs.append(v)
-    return outs, ld
 
 
 def _loss(outs, ld, weights):
@@ -76,7 +46,7 @@ def test_gradients_match_oracle_autograd(name, direction, use_intermediates):
     sd64 = {k: (v.double().requires_grad_() if v.is_floating_point() and not k.endswith((".P", ".mask")) else v.double()
                 if v.is_floating_point() else v) for k, v in sd.items()}
     x64 = x.double().requires_grad_()
-    outs, ld = _oracle_stack(sd64, specs, x64, inverse)
+    outs, ld = oracle_stack(sd64, specs, x64, inverse)
     _loss(outs, ld, (w_ld, w_out)).backward()
 
     model = load_flow_model(specs, sd, return_intermediates=use_intermediates)

@@ -8,7 +8,7 @@ import pytest
 import torch
 
 from tests.helpers import golden_sd, golden_spec, load_flow_model, load_golden, random_flow_sd
-from tests.test_flow_autograd_gpu import _oracle_stack
+from tests.helpers import oracle_stack
 from tests.test_flows_gpu import close_vs_oracle
 
 pytestmark = pytest.mark.gpu
@@ -197,7 +197,7 @@ def test_gradients_match_oracle_autograd(name):
     sd64 = {k: (v.double().requires_grad_() if v.is_floating_point() and not k.endswith((".P", ".mask")) else v.double()
                 if v.is_floating_point() else v) for k, v in sd.items()}
     z64 = z.double().cpu()
-    outs, ld = _oracle_stack(sd64, specs, z64, False)
+    outs, ld = oracle_stack(sd64, specs, z64, False)
     lp64 = _log_normal64(z64) - ld
     ((outs[-1] * w_x).sum() + (lp64 * w_lp).sum()).backward()
     torch.testing.assert_close(x.detach().double().cpu(), outs[-1].detach(), rtol=1e-4, atol=1e-4)
